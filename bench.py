@@ -14,7 +14,10 @@ step (--shards distinct batches per rank); per-shard step times are reported.
           solve + D2H of every solution vector inside the timed region)
 Rank layout: one process per GPU, scenario sharding, no data-path collective ("weak").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (solution vectors and per-plan solve results of rank 0) as
+.npy files, so that two builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -120,6 +123,32 @@ def algorithmic_flops(stats: dict, N: int) -> float:
     iteration 1000 flops per stage for the Riccati factorisation and sweeps, 60 flops per
     active inequality row for residuals, Hessian update, two gradients and two step lengths."""
     return 1000.0 * N * stats["qp_iters"] + 60.0 * stats["rows_visited"]
+
+
+DUMP_BYTES = 64_000_000
+DUMP_FIELDS = ("status", "proven", "objective", "best_bound", "gap", "max_violation")
+
+
+def dump_outputs(out_dir: str, solver, seeds):
+    """Writes the results the solver holds (its last batch run) as float64 .npy files: x.npy [plans, columns] (the solution
+    vectors), plan_seed.npy (scenario seed of every row) and one array per solve-result field.  Search statistics (nodes,
+    iterations, seconds) are left out: they say how the search went, not what it computed.  When the whole batch exceeds
+    DUMP_BYTES, a fixed seeded sample of its plans is written."""
+    xs, infos = solver.fetch()
+    ncols = max(len(x) for x in xs)
+    per_plan = 8 * (ncols + 1 + len(DUMP_FIELDS))
+    keep = min(len(xs), (DUMP_BYTES - (1 << 16)) // per_plan)        # (1 << 16): room for the .npy headers
+    idx = np.arange(len(xs))
+    if keep < len(xs):
+        idx = np.sort(np.random.default_rng(0).choice(len(xs), keep, replace=False))
+    x = np.full((keep, ncols), np.nan)
+    for row, k in enumerate(idx):
+        x[row, :len(xs[k])] = xs[k]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), x)
+    np.save(os.path.join(out_dir, "plan_seed.npy"), np.asarray(seeds, dtype=np.float64)[idx])
+    for f in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f + ".npy"), np.array([float(getattr(infos[k], f)) for k in idx]))
 
 
 def cpu_oracle_rate(plans, threads: int):
@@ -477,7 +506,13 @@ def main():
     ap.add_argument("--first-shard", type=int, default=0, help="offset of the scenario shards (knobs are tuned on held-out shards >= 100, the reported runs use 0)")
     ap.add_argument("--skip-extras", action="store_true", help="only the throughput legs (no latency, replanning, assembly, CPU baseline): for A/B runs")
     ap.add_argument("--in-flight", type=int, default=3, help="batches in flight on one GPU (solver instances / streams); 1 = one at a time")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the solution vectors and solve results of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "config2"):
+        ap.error("--dump-outputs covers the device path of the default workload (config2)")
     args.batch_given = any(a == "--batch" or a.startswith("--batch=") for a in sys.argv[1:])
     if args.impl == "reference":
         return run_reference(args)
@@ -616,6 +651,16 @@ def main():
     value = value_pipe if use_pipe else value_seq
     if use_pipe:
         total_ms = pipe_ms
+    if args.dump_outputs and rank == 0:
+        # results of the leg that gave `value`, as its last timed step left them: the sequential solver ran shard
+        # shard_ids[(steps - 1) mod S] last; pipelined step (steps - 1) ran on instance (steps - 1) mod depth, which holds
+        # shard_ids[instance mod S] (upload_resident above)
+        if use_pipe:
+            w = (args.steps - 1) % len(pipe.solvers)
+            last_solver, last_sid = pipe.solvers[w], shard_ids[w % S]
+        else:
+            last_solver, last_sid = solver, shard_ids[(args.steps - 1) % S]
+        dump_outputs(args.dump_outputs, last_solver, [last_sid * B + k for k in range(B)])
 
     # ---- end to end through the C ABI with host buffers ------------------------------------
     # the caller holds the batch as MiqpB200Problem structs over host arrays and receives every

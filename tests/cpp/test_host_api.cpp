@@ -1,6 +1,7 @@
 // C++ API test of the host side (planner-miqp_b200/host): the class-level behaviour the reference's gtest
 // suites check on MiqpPlanner / CplexWrapper (test/miqp_planner_test.cc, test/cplex_wrapper_test.cc) that needs
-// no BARK.  `test_host_api cpu` runs the device-free part, `test_host_api gpu` adds the solves.
+// no BARK.  `test_host_api cpu|gpu <repository root> <scratch directory>`: `cpu` runs the device-free part, `gpu` adds
+// the solves.
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -13,6 +14,7 @@ using namespace miqp::planner;
 using miqp::planner::cplex::CplexWrapper;
 
 static int failures = 0;
+static std::string g_tmp;    // directory the test writes its files to (argv[3]; one per run, so runs of other users cannot collide)
 #define CHECK(c) do { if (!(c)) { std::printf("FAIL %s:%d  %s\n", __FILE__, __LINE__, #c); ++failures; } } while (0)
 
 static PolyLine Line(std::initializer_list<double> pts, double inc = 0.2) {
@@ -111,7 +113,7 @@ static void cpu_part() {
   CHECK((int)names.size() == l.ncols && names[0] == "u_x(1)(1)" && names[2 * 2 * 20 + 20 + 3] == "pos_x(2)(4)");
   CHECK(names[l.base_ar + (1 * 20 + 2) * 16 + 5] == "active_region(2)(3)(6)" && names[l.base_rcna + 4 * 2 * 20] == "region_change_not_allowed_combined(1)(1)");
   CHECK(names[l.base_c2c + 17] == "car2car_collision(1)(1)(2)(2)" && names[l.ncols - 1] == "slackvars(1)(1)(20)(4)");
-  const std::string mst = "/tmp/miqp_b200_test_roundtrip.mst";
+  const std::string mst = g_tmp + "/miqp_b200_test_roundtrip.mst";
   CHECK(miqp::planner::cplex::WriteMst(mst, l, x));
   std::vector<double> xr;
   CHECK(miqp::planner::cplex::ReadMst(mst, l.ncols, xr) && xr == x);
@@ -119,11 +121,11 @@ static void cpu_part() {
   {   // a wrapper bound to the same parameters takes the file as its "last solution" MIP start and writes it back unchanged
     CplexWrapper w2(12);
     w2.resetParameters(p);
-    CHECK(!w2.writeMIPStarts("/tmp/miqp_b200_test_none.mst"));      // nothing solved or read yet
+    CHECK(!w2.writeMIPStarts(g_tmp + "/miqp_b200_test_none.mst"));      // nothing solved or read yet
     CHECK(w2.readMIPStarts(mst) && w2.getSolutionVector() == x);
-    CHECK(w2.writeMIPStarts("/tmp/miqp_b200_test_roundtrip2.mst") && miqp::planner::cplex::ReadMst("/tmp/miqp_b200_test_roundtrip2.mst", l.ncols, xr) && xr == x);
-    w2.setTmpWarmstartFile("/tmp/miqp_b200_test_tmpws.mst");
-    CHECK(w2.getTmpWarmstartFile() == "/tmp/miqp_b200_test_tmpws.mst");
+    CHECK(w2.writeMIPStarts(g_tmp + "/miqp_b200_test_roundtrip2.mst") && miqp::planner::cplex::ReadMst(g_tmp + "/miqp_b200_test_roundtrip2.mst", l.ncols, xr) && xr == x);
+    w2.setTmpWarmstartFile(g_tmp + "/miqp_b200_test_tmpws.mst");
+    CHECK(w2.getTmpWarmstartFile() == g_tmp + "/miqp_b200_test_tmpws.mst");
     // overrideSolverSettingsDataSource copies the solver options only (src/model_input_data_source.cpp:282-296)
     auto o = std::make_shared<ModelParameters>();
     o->max_solution_time = 3.5f; o->relative_mip_gap_tolerance = 0.02f; o->mipemphasis = 1; o->parallelmode = -1; o->NumSteps = 7;
@@ -147,7 +149,7 @@ static void dat_part() {
   CHECK(m.fraction_parameters.rows() == 32 && m.poly_curvature_params.POLY_KAPPA_AX_MAX.rows() == 32 && m.obstacle_is_soft[0] == 0);
   cplex::FlatProblem f1, f2;
   cplex::Flatten(m, 0, f1);
-  const std::string tmp = "/tmp/miqp_b200_test_roundtrip.dat";
+  const std::string tmp = g_tmp + "/miqp_b200_test_roundtrip.dat";
   CHECK(cplex::WriteParametersDat(f1.p, m, tmp));
   ModelParameters m2;
   datio::ReadParametersDat(tmp, m2);
@@ -215,7 +217,7 @@ static void gpu_part() {
     MiqpPlanner src(sc, map);
     src.AddCar(st, ref, 5, 1);
     src.AddObstacle({{20.0, 1.0, 0.0}}, 2.0, 1.0, false, true);
-    src.ActivateDebugFileWrite("/tmp", "miqp_b200_hostapi_");
+    src.ActivateDebugFileWrite(g_tmp, "miqp_b200_hostapi_");
     CHECK(src.Plan(7.0));
     const std::string dump = src.GetCplexWrapper().getDebugOutputParameterFilePath();
     CHECK(!dump.empty());
@@ -236,17 +238,17 @@ static void gpu_part() {
     CplexWrapper fx("", "cplexmodel.mod", CplexWrapper::DATFILE, 12);
     fx.setParameterDatFileAbsolute((g_root + "/tests/golden/cplexmodel_testcase.dat").c_str());
     fx.setLastSolutionWarmstart(LAST_SOLUTION_WARMSTART);
-    fx.setTmpWarmstartFile("/tmp/miqp_b200_hostapi_ws.mst");
+    fx.setTmpWarmstartFile(g_tmp + "/miqp_b200_hostapi_ws.mst");
     fx.deleteLastSolutionWarmstartFile();
     CHECK(fx.callCplex(0.0) == SUCCESS);
-    CHECK(fx.exportModel("/tmp/miqp_b200_hostapi_testcase.lp"));
+    CHECK(fx.exportModel(g_tmp + "/miqp_b200_hostapi_testcase.lp"));
     // LAST_SOLUTION_WARMSTART wrote the solution to the warm-start file; a fresh wrapper starts from it
     std::vector<double> xr;
-    CHECK(miqp::planner::cplex::ReadMst("/tmp/miqp_b200_hostapi_ws.mst", (int)fx.getSolutionVector().size(), xr) && xr == fx.getSolutionVector());
+    CHECK(miqp::planner::cplex::ReadMst(g_tmp + "/miqp_b200_hostapi_ws.mst", (int)fx.getSolutionVector().size(), xr) && xr == fx.getSolutionVector());
     CplexWrapper fy("", "cplexmodel.mod", CplexWrapper::DATFILE, 12);
     fy.setParameterDatFileAbsolute((g_root + "/tests/golden/cplexmodel_testcase.dat").c_str());
     fy.setLastSolutionWarmstart(LAST_SOLUTION_WARMSTART);
-    fy.setTmpWarmstartFile("/tmp/miqp_b200_hostapi_ws.mst");
+    fy.setTmpWarmstartFile(g_tmp + "/miqp_b200_hostapi_ws.mst");
     CHECK(fy.callCplex(1.0) == SUCCESS);
     CHECK(std::fabs(fy.getSolutionProperties().objective - fx.getSolutionProperties().objective) <= 0.1 * 9.57603);
     CHECK(fy.getSolutionProperties().NrNodes <= fx.getSolutionProperties().NrNodes);   // the MIP start is an incumbent from the first round on
@@ -261,6 +263,7 @@ static void gpu_part() {
 
 int main(int argc, char **argv) {
   g_root = (argc > 2) ? argv[2] : ".";
+  g_tmp = (argc > 3) ? argv[3] : "/tmp";
   cpu_part();
   dat_part();
   if (argc > 1 && std::strcmp(argv[1], "gpu") == 0) gpu_part();

@@ -12,7 +12,6 @@ import pytest
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
-LP = "/tmp/miqp_b200_hostapi_testcase.lp"
 
 
 def parse_lp(path):
@@ -30,12 +29,12 @@ def parse_lp(path):
     return rows, binaries, free, boxed, txt
 
 
-def test_lp_export_matches_the_pinned_statistics_and_the_oracle_rows(testcase_problem):
+def test_lp_export_matches_the_pinned_statistics_and_the_oracle_rows(testcase_problem, tmp_path):
     from test_host_api_cpp import _build, EXE, ROOT   # the C++ test writes the file
     _build()
-    r = subprocess.run([EXE, "gpu", os.path.abspath(ROOT)], capture_output=True, text=True)
+    r = subprocess.run([EXE, "gpu", os.path.abspath(ROOT), str(tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
-    rows, binaries, free, boxed, txt = parse_lp(LP)
+    rows, binaries, free, boxed, txt = parse_lp(str(tmp_path / "miqp_b200_hostapi_testcase.lp"))
     p = testcase_problem
     # reference pins: 12361 rows, 29834 non-zeros, 1240 binaries, 340 continuous
     assert len(rows) == 12361

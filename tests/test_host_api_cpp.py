@@ -23,14 +23,14 @@ def _build():
                     "-lmiqp_b200", "-Wl,-rpath," + PKG], check=True)
 
 
-def test_host_api_cpu():
+def test_host_api_cpu(tmp_path):
     _build()
-    r = subprocess.run([EXE, "cpu", os.path.abspath(ROOT)], capture_output=True, text=True)
+    r = subprocess.run([EXE, "cpu", os.path.abspath(ROOT), str(tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
 
 
 @pytest.mark.gpu
-def test_host_api_gpu():
+def test_host_api_gpu(tmp_path):
     _build()
-    r = subprocess.run([EXE, "gpu", os.path.abspath(ROOT)], capture_output=True, text=True)
+    r = subprocess.run([EXE, "gpu", os.path.abspath(ROOT), str(tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr

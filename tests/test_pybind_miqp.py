@@ -100,14 +100,15 @@ def test_cplex_wrapper_surface_without_device(miqp):
 
 
 @pytest.mark.gpu
-def test_cplex_wrapper_solves_the_reference_fixture(miqp):
+def test_cplex_wrapper_solves_the_reference_fixture(miqp, tmp_path):
     w = miqp.CplexWrapper("cplexmodel.mod", 12)
     w.setParameterDatFileAbsolute(os.path.join(ROOT, "tests", "golden", "cplexmodel_testcase.dat"))
     assert w.callCplex(0.0) == miqp.OptimizationStatus.SUCCESS
     sp = w.getSolutionProperties()
     assert abs(sp.objective - 9.57603) <= 0.1 * 9.57603 and sp.gap <= 0.1 and sp.time > 0    # the file asks for a 10 % gap
-    assert w.writeMIPStarts("/tmp/miqp_b200_pybind.mst") and w.readMIPStarts("/tmp/miqp_b200_pybind.mst")
-    assert w.exportModel("/tmp/miqp_b200_pybind.lp") and os.path.getsize("/tmp/miqp_b200_pybind.lp") > 100000
+    mst, lp = str(tmp_path / "miqp_b200_pybind.mst"), str(tmp_path / "miqp_b200_pybind.lp")
+    assert w.writeMIPStarts(mst) and w.readMIPStarts(mst)
+    assert w.exportModel(lp) and os.path.getsize(lp) > 100000
 
 
 # ---- BehaviorMiqpAgent (host/behavior_miqp_agent.hpp: the planning cycle of src/behavior_miqp_agent.cpp:137-335 without BARK) ----
