@@ -24,6 +24,11 @@
  *                                  collectSolutionStatus, src/cplex_wrapper.cpp:158-249,
  *                                  :311-448, :672-678; MIP start :494-639
  * miqp_b200_batch_* (resident)     the same solve with the batch already in HBM
+ * miqp_b200_set_solution_pool      the solution pool of cplex.solve(); its size is
+ *                                  SolutionProperties.NrSolutionPool, collectCplexStatistics,
+ *                                  src/cplex_wrapper.cpp:680-690
+ * miqp_b200_pool_sizes / _fetch    the pool's members (IloCplex::getSolnPoolNsolns /
+ *                                  getValues(sol, i)), best first
  */
 #ifndef MIQP_B200_H
 #define MIQP_B200_H
@@ -190,6 +195,27 @@ int miqp_b200_frontier_ub_device(MiqpB200Solver *s, void **ub, int *count);
 int miqp_b200_frontier_get_ub(MiqpB200Solver *s, double *ub /* [count] */);
 int miqp_b200_frontier_tighten(MiqpB200Solver *s, const double *ub /* [count] */);
 int miqp_b200_frontier_finish(MiqpB200Solver *s, float *device_ms);
+
+/* Solution pool (CPLEX's pool, counted by SolutionProperties.NrSolutionPool): up to `capacity` distinct integer-feasible
+ * completions per plan that the search solved, best first.  0 = off (default); 1..64; takes effect at the next upload.
+ * The pool records leaves the search solves anyway (those that do not beat the incumbent too); it does not change the search or
+ * its results.  Policy: the `capacity` best leaves by the incumbent's key (search value, node uid) with pairwise different
+ * decisions, so the pool is as deterministic as the search.  The pool of the last run stays on the device until the next upload. */
+int miqp_b200_set_solution_pool(MiqpB200Solver *s, int capacity);
+typedef struct MiqpB200PoolEntry {
+  double objective, max_violation; /* of the expanded full vector, device-evaluated, like MiqpB200SolveInfo */
+  double search_value;             /* value the search stored (order key with uid) */
+  int converged;                   /* 1: the leaf QP was solved to optimality */
+  int round;                       /* round of the search that solved the leaf */
+  unsigned long long uid;          /* node uid */
+} MiqpB200PoolEntry;
+/* entries per plan, [count]; ERR_ARG with the pool off or before a run */
+int miqp_b200_pool_sizes(MiqpB200Solver *s, int *sizes /* [count] */);
+/* the first min(size, max_entries) entries of plan k in (search_value, uid) order -- entry 0 is the incumbent --, their full column
+ * vectors (x_out, RawResults order like fetch_vector) and trajectories (traj_out, the compact layout of batch_fetch_compact) */
+int miqp_b200_pool_fetch(MiqpB200Solver *s, int k, int max_entries, MiqpB200PoolEntry *entries,
+                         double *x_out /* [max_entries][ncols(k)] or NULL */,
+                         double *traj_out /* [max_entries][C][N][8] or NULL */, int *n_out);
 
 /* counters of the last run: kernel launches, node relaxations, IPM iterations, seconds
  * spent in the node kernel (CUDA events on the solver stream) */

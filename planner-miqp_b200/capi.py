@@ -26,6 +26,7 @@ DECLARED_SYMBOLS = [
     "miqp_b200_frontier_start", "miqp_b200_frontier_rounds", "miqp_b200_frontier_split", "miqp_b200_frontier_get_ub",
     "miqp_b200_frontier_tighten", "miqp_b200_frontier_finish", "miqp_b200_frontier_fingerprint", "miqp_b200_frontier_ub_device", "miqp_b200_batch_upload_replan", "miqp_b200_mark", "miqp_b200_elapsed", "miqp_b200_batch_fetch_compact", "miqp_b200_fetch_vector",
     "miqp_b200_solve_batch_compact",
+    "miqp_b200_set_solution_pool", "miqp_b200_pool_sizes", "miqp_b200_pool_fetch",
 ]
 
 
@@ -77,6 +78,11 @@ class COptions(C.Structure):
                 ("max_rounds", C.c_int), ("verbose", C.c_int)]
 
 
+class CPoolEntry(C.Structure):
+    _fields_ = [("objective", C.c_double), ("max_violation", C.c_double), ("search_value", C.c_double),
+                ("converged", C.c_int), ("round", C.c_int), ("uid", C.c_ulonglong)]
+
+
 class CRunStats(C.Structure):
     _fields_ = [("launches", C.c_long), ("node_kernel_launches", C.c_long), ("nodes", C.c_long),
                 ("qp_iters", C.c_long), ("rounds", C.c_long), ("node_kernel_ms", C.c_double),
@@ -98,6 +104,20 @@ class SolveInfo:
     rounds: int
     uncertified: int = 0
     pool_exhausted: int = 0
+
+
+@dataclass
+class PoolEntry:
+    """One member of a plan's solution pool (miqp_b200_pool_fetch): objective and max violation of its full column
+    vector `x` (device-evaluated), the value the search stored for the leaf, and its trajectory `traj` [C][N][8]."""
+    objective: float
+    max_violation: float
+    search_value: float
+    converged: bool
+    round: int
+    uid: int
+    x: np.ndarray | None = None
+    traj: np.ndarray | None = None
 
 
 def library_path() -> str:
@@ -136,6 +156,9 @@ def load_library():
     lib.miqp_b200_measure_fp64_peak.argtypes = [C.c_void_p, _dp]
     lib.miqp_b200_debug_profile.argtypes = [C.c_void_p, C.POINTER(C.c_ulonglong)]
     lib.miqp_b200_debug_traces.argtypes = [C.c_void_p, _dp]
+    lib.miqp_b200_set_solution_pool.argtypes = [C.c_void_p, C.c_int]
+    lib.miqp_b200_pool_sizes.argtypes = [C.c_void_p, _ip]
+    lib.miqp_b200_pool_fetch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CPoolEntry), _dp, _dp, _ip]
     _lib = lib
     return lib
 
@@ -231,7 +254,9 @@ class Solver:
     """Owns one MiqpB200Solver handle (one CUDA device, one stream)."""
 
     def __init__(self, device: int = 0, nodes_per_round: int = 0, pool_capacity: int = 0,
-                 max_rounds: int = 0, verbose: int = 0):
+                 max_rounds: int = 0, verbose: int = 0, solution_pool: int = 0):
+        """pool_capacity: open-node slots per plan (0 = auto).  solution_pool: up to this many distinct feasible plans
+        per problem are kept (0 = off, at most 64; see set_solution_pool)."""
         self._lib = load_library()
         opt = COptions(device, nodes_per_round, pool_capacity, max_rounds, verbose)
         h = C.c_void_p()
@@ -241,6 +266,8 @@ class Solver:
                                 "(this backend has no CPU fallback)")
         self._h = h
         self._batch = None
+        if solution_pool:
+            self.set_solution_pool(solution_pool)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -333,6 +360,7 @@ class Solver:
         """One miqp_b200_solve_batch call on host buffers: pack + H2D + device solve + D2H."""
         self._check(self._lib.miqp_b200_solve_batch(self._h, b["arr"], b["n"], b["warm"], b["xptr"], b["infos"]),
                     "miqp_b200_solve_batch")
+        self._batch = (b["n"], [len(x) for x in b["xs"]]); self._shapes = [(p.C, p.N) for p in b["problems"]]
         return b["xs"], b["infos"]
 
     def solve_batch(self, problems, gap_tol=None, time_limit=None, warm=None):
@@ -343,6 +371,7 @@ class Solver:
         xptr = (_dp * n)(*[x.ctypes.data_as(_dp) for x in xs])
         infos = (CSolveInfo * n)()
         self._check(self._lib.miqp_b200_solve_batch(self._h, arr, n, warm_arr, xptr, infos), "miqp_b200_solve_batch")
+        self._batch = (n, ncols); self._shapes = [(p.C, p.N) for p in problems]
         return xs, [self._info(i) for i in infos]
 
     def solve(self, p, gap_tol=None, time_limit=None, warm=None):
@@ -374,6 +403,37 @@ class Solver:
         self._lib.miqp_b200_fetch_vector.argtypes = [C.c_void_p, C.c_int, _dp]
         self._check(self._lib.miqp_b200_fetch_vector(self._h, int(k), x.ctypes.data_as(_dp)), "miqp_b200_fetch_vector")
         return x
+
+    # ---- solution pool ---------------------------------------------------------------
+    def set_solution_pool(self, capacity: int):
+        """keep up to `capacity` (1..64) best distinct integer-feasible plans per problem from the next upload on; 0 = off"""
+        self._check(self._lib.miqp_b200_set_solution_pool(self._h, int(capacity)), "miqp_b200_set_solution_pool")
+
+    def pool_sizes(self) -> np.ndarray:
+        """number of pool entries of every plan of the last run"""
+        out = np.zeros(self._batch[0], dtype=np.int32)
+        self._check(self._lib.miqp_b200_pool_sizes(self._h, out.ctypes.data_as(_ip)), "miqp_b200_pool_sizes")
+        return out
+
+    def pool(self, k: int, vectors: bool = True, max_entries: int = 64) -> list[PoolEntry]:
+        """pool of plan k, best first (entry 0 is the incumbent); vectors: also the full column vectors and trajectories"""
+        n, ncols = self._batch
+        if not 0 <= k < n:
+            raise IndexError(k)
+        m = int(max_entries)
+        ents = (CPoolEntry * max(m, 1))()
+        x = tr = None
+        if vectors:
+            c, nn = self._shapes[k]
+            x = np.zeros((m, ncols[k]))
+            tr = np.zeros((m, c, nn, 8))
+        got = C.c_int()
+        self._check(self._lib.miqp_b200_pool_fetch(self._h, int(k), m, ents, None if x is None else x.ctypes.data_as(_dp),
+                                                   None if tr is None else tr.ctypes.data_as(_dp), C.byref(got)),
+                    "miqp_b200_pool_fetch")
+        return [PoolEntry(e.objective, e.max_violation, e.search_value, bool(e.converged), e.round, e.uid,
+                          None if x is None else x[j].copy(), None if tr is None else tr[j].copy())
+                for j, e in enumerate(ents[:got.value])]
 
     def solve_prepared_compact(self, b):
         """One miqp_b200_solve_batch_compact call on host buffers: pack + H2D + device solve + D2H of trajectories and infos."""

@@ -82,6 +82,7 @@ __global__ void bnb_init_kernel(BnbState st, const DevProb *probs, const unsigne
     st.done[s] = 0; st.done_round[s] = -1; st.lock[s] = 0;
     st.stat_nodes[s] = 0; st.stat_iters[s] = 0; st.stat_rows[s] = 0; st.stat_uncert[s] = 0; st.overflow[s] = 0;
     st.inc_uid[s] = ~0ULL;
+    if (st.pool_cap > 0) st.pool_cnt[s] = 0;
     if (s == 0) { *st.active_prev = 0; *st.work_cnt = 0; *st.work_next = 0; *st.active = 0; *st.err = 0; *st.work_cnt2 = 0; *st.work_next2 = 0; }
   }
 }
@@ -518,6 +519,24 @@ __device__ __forceinline__ void copy_bytes16(unsigned char *dst, const unsigned 
   for (int k = lane; k < nbytes / 16; k += 32) d4[k] = s4[k];
 }
 
+// solution pool: a leaf of bnb_nodes_kernel (warp 0, plan lock held) goes in if it is among the pool's best (pool_slot).  Out of
+// line so that the node kernel keeps its register allocation; it runs only at leaves and only when the pool is on.
+__device__ __noinline__ void pool_insert_warp(PoolRef pr, const unsigned char *dec, const double *V, int N, double val,
+                                              unsigned long long uid, int round, int converged, int lane) {
+  const int slot = pool_slot(pr, dec, val, uid, lane, 32, [](bool p) { return __any_sync(FULL, p) != 0; });
+  __syncwarp();   // every lane has read the pool before it changes
+  if (slot < 0) return;
+  double *z = pr.z + (long)slot * pr.zstride;
+  for (int k = lane; k < N * 8; k += 32) z[k] = V[(k >> 3) * V_STRIDE + V_Z + (k & 7)];
+  copy_bytes16(pr.dec + (long)slot * pr.ndec_stride, dec, pr.ndec_stride, lane);
+  if (lane == 0) {
+    PoolRec r; r.val = val; r.uid = uid; r.round = round; r.converged = converged;
+    pr.rec[slot] = r;
+    const int cnt = __ldcg(pr.cnt);
+    if (slot == cnt) *pr.cnt = cnt + 1;
+  }
+}
+
 __device__ __forceinline__ void effective_regions(const WarpCtx &w) {
   const DevProb &p = *w.p;
   if (w.lane == 0) {
@@ -730,6 +749,7 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
         __syncwarp();
         if (lane == 0) { st.ub[s] = inc; st.inc_uid[s] = nuid; }
       }
+      if (st.pool_cap > 0) pool_insert_warp(pool_ref(st, s), w.dec, w.V, p.N, inc, nuid, round, r.converged ? 1 : 0, lane);
       warp_unlock(&st.lock[s], lane);
       continue;
     }
@@ -931,37 +951,13 @@ void launch_bnb_shift_warm(const DevProb *probs, const int *iblob, int count, co
 // finish: best bound, full column vector of the incumbent (collectRawResults,
 // src/cplex_wrapper.cpp:311-448)
 // ---------------------------------------------------------------------------------------
-__global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob,
-                                  double *xall, double *best_bound) {
-  const int s = blockIdx.x;
+// Full OPL column vector x (zeroed by the caller) of a fully decided node: decisions `dec`, relaxed optimum `z` ([C][N][8], then
+// the pair slacks [P][N][4]; z is overwritten with the exact trajectory).  Called by every thread of the block; jeff_s: shared
+// [8 * 64].  Out of line: the incumbent (bnb_finish_kernel) and the pool entries (pool_expand_kernel) run the same code.
+__device__ __noinline__ void expand_solution(const DevProb &p, const double *D, const int *I, const unsigned char *dec, double *z,
+                                             double *x, int *jeff_s) {
   const int tid = threadIdx.x, nt = blockDim.x;
-  const DevProb &p = probs[s];
-  const double *D = dblob; const int *I = iblob;
-  const long pb = (long)s * st.cap;
-  __shared__ double red[128];
-  __shared__ int jeff_s[8 * 64];
-  // best bound: smallest bound still open or pruned by the gap rule
-  double lb = MQ_INF;
-  const int nopen = st.open_cnt[s];
-  for (int k = tid; k < nopen; k += nt) lb = fmin(lb, st.bound[pb + st.open_idx[pb + k]]);
-  red[tid] = lb;
-  __syncthreads();
-  if (tid == 0) {
-    for (int k = 0; k < nt; ++k) lb = fmin(lb, red[k]);
-    lb = fmin(lb, st.pruned_lb[s]);
-    const double ub = st.ub[s];
-    if (st.done[s] && lb == MQ_INF) lb = ub;  // tree exhausted
-    if (ub < MQ_INF && lb > ub) lb = ub;
-    best_bound[s] = lb;
-  }
-  const double ub = st.ub[s];
-  double *x = xall + p.x_base;
-  for (int k = tid; k < p.ncols; k += nt) x[k] = 0.0;
-  __syncthreads();
-  if (!(ub < MQ_INF) || st.inc_uid[s] == ~0ULL) return;   // no incumbent of its own (ub may come from another rank: frontier sharding)
   const int C = p.C, N = p.N, R = p.R, E = p.E, O = p.O, L = p.L;
-  const unsigned char *dec = st.inc_dec + (long)s * st.ndec_stride;
-  double *z = st.inc_z + (long)s * st.zstride;
   // exact trajectory from the jerks (model_region_constraints.mod:11-19)
   if (tid < C) {
     const int c = tid;
@@ -1071,9 +1067,63 @@ __global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const doubl
   }
 }
 
+__global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob,
+                                  double *xall, double *best_bound) {
+  const int s = blockIdx.x;
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const DevProb &p = probs[s];
+  const double *D = dblob; const int *I = iblob;
+  const long pb = (long)s * st.cap;
+  __shared__ double red[128];
+  __shared__ int jeff_s[8 * 64];
+  // best bound: smallest bound still open or pruned by the gap rule
+  double lb = MQ_INF;
+  const int nopen = st.open_cnt[s];
+  for (int k = tid; k < nopen; k += nt) lb = fmin(lb, st.bound[pb + st.open_idx[pb + k]]);
+  red[tid] = lb;
+  __syncthreads();
+  if (tid == 0) {
+    for (int k = 0; k < nt; ++k) lb = fmin(lb, red[k]);
+    lb = fmin(lb, st.pruned_lb[s]);
+    const double ub = st.ub[s];
+    if (st.done[s] && lb == MQ_INF) lb = ub;  // tree exhausted
+    if (ub < MQ_INF && lb > ub) lb = ub;
+    best_bound[s] = lb;
+  }
+  const double ub = st.ub[s];
+  double *x = xall + p.x_base;
+  for (int k = tid; k < p.ncols; k += nt) x[k] = 0.0;
+  __syncthreads();
+  if (!(ub < MQ_INF) || st.inc_uid[s] == ~0ULL) return;   // no incumbent of its own (ub may come from another rank: frontier sharding)
+  expand_solution(p, D, I, st.inc_dec + (long)s * st.ndec_stride, st.inc_z + (long)s * st.zstride, x, jeff_s);
+}
+
 void launch_bnb_finish(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob,
                        double *xall, double *best_bound, cudaStream_t s) {
   bnb_finish_kernel<<<st.count, 128, 0, s>>>(st, probs, dblob, iblob, xall, best_bound);
+}
+
+// solution pool entries of plan k as full column vectors (miqp_b200_pool_fetch); the trajectory is integrated in a copy of the
+// stored relaxed optimum, so the pool stays as the search left it
+__global__ void pool_expand_kernel(BnbState st, int k, const int *idx, const DevProb *eprobs, const double *dblob, const int *iblob,
+                                   double *zs, double *xall) {
+  const int e = blockIdx.x;
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const DevProb &p = eprobs[e];
+  __shared__ int jeff_s[8 * 64];
+  const long ent = (long)k * st.pool_cap + idx[e];
+  const double *zp = st.pool_z + ent * st.zstride;
+  double *z = zs + (long)e * st.zstride;
+  double *x = xall + p.x_base;
+  for (int q = tid; q < st.zstride; q += nt) z[q] = zp[q];
+  for (int q = tid; q < p.ncols; q += nt) x[q] = 0.0;
+  __syncthreads();
+  expand_solution(p, dblob, iblob, st.pool_dec + ent * st.ndec_stride, z, x, jeff_s);
+}
+
+void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const DevProb *eprobs, const double *dblob, const int *iblob,
+                        double *zs, double *xall, cudaStream_t s) {
+  if (n > 0) pool_expand_kernel<<<n, 128, 0, s>>>(st, k, idx, eprobs, dblob, iblob, zs, xall);
 }
 
 }  // namespace miqp

@@ -14,6 +14,33 @@ namespace miqp {
 
 constexpr int MULTI_MAX_THREADS = 128;
 
+// solution pool: a leaf of bnb_nodes_multi_kernel (whole CTA, plan lock held) goes in if it is among the pool's best (pool_slot).
+// Out of line so that the node kernel keeps its register allocation; it runs only at leaves and only when the pool is on.
+__device__ __noinline__ void pool_insert_cta(PoolRef pr, const unsigned char *dec, const double *Z, int nz, const double *sig, int C, int N,
+                                             int P, double val, unsigned long long uid, int round, int converged) {
+  const int tid = threadIdx.x, nthr = blockDim.x;
+  const int slot = pool_slot(pr, dec, val, uid, tid, nthr, [](bool p) { return __syncthreads_or(p) != 0; });
+  __syncthreads();   // every thread has read the pool before it changes
+  if (slot < 0) return;
+  double *z = pr.z + (long)slot * pr.zstride;   // the layout of inc_z
+  for (int e = tid; e < C * N * 8; e += nthr) {
+    const int c = e / (N * 8), i = (e / 8) % N, t = e % 8;
+    z[e] = Z[(long)i * nz + 8 * c + t];
+  }
+  for (int e = tid; e < P * N * 4; e += nthr) z[(long)C * N * 8 + e] = sig[e * SG_SIZE + SG_VAL];
+  const uint4 *s4 = reinterpret_cast<const uint4 *>(dec);
+  uint4 *d4 = reinterpret_cast<uint4 *>(pr.dec + (long)slot * pr.ndec_stride);
+  for (int e = tid; e < pr.ndec_stride / 16; e += nthr) d4[e] = s4[e];
+  if (tid == 0) {
+    PoolRec r; r.val = val; r.uid = uid; r.round = round; r.converged = converged;
+    pr.rec[slot] = r;
+    const int cnt = __ldcg(pr.cnt);
+    if (slot == cnt) *pr.cnt = cnt + 1;
+  }
+  __threadfence();
+  __syncthreads();
+}
+
 long multi_workspace_bytes(int C, int N, int P, int kmax, int ndec_stride) {
   return (multi_layout(C, N, P, kmax, ndec_stride).total_bytes + 15) & ~15L;
 }
@@ -88,6 +115,7 @@ __global__ void __launch_bounds__(MULTI_MAX_THREADS) bnb_nodes_multi_kernel(BnbS
         __threadfence();
       }
       __syncthreads();
+      if (st.pool_cap > 0) pool_insert_cta(pool_ref(st, s), k.dec, k.Z, k.nz, k.sig, k.C, k.N, k.P, out.fval, nuid, round, out.converged);
       if (tid == 0) {
         if (s_i[1]) { st.ub[s] = out.fval; st.inc_uid[s] = nuid; }
         __threadfence();

@@ -13,6 +13,13 @@ void launch_evaluate(const DevProb *probs, const double *dblob, const int *iblob
                      const double *xall, double *max_viol, double *objective, cudaStream_t st);
 
 // ---- bnb.cu ---------------------------------------------------------------------------
+// entry of the solution pool (BnbState::pool_rec)
+struct PoolRec {
+  double val;               // value the search stored for the leaf (the incumbent's ub when it is the best)
+  unsigned long long uid;   // node uid (tie break, as inc_uid)
+  int round, converged;     // round the leaf was solved in; 1 if its QP was solved to optimality
+};
+
 // Device-resident branch and bound state of a batch of plans.
 struct BnbState {
   int count;            // plans
@@ -67,6 +74,19 @@ struct BnbState {
   // round control
   int2 *work; int *work_cnt; int *work_next; int *active; int *err; int *active_prev;
   int2 *work2; int *work_cnt2; int *work_next2;   // plans with NumCars > 1 (bnb_multi.cu)
+  // solution pool (pool_cap > 0): the pool_cap best distinct leaves of every plan by the incumbent's key (value, uid), unsorted;
+  // records laid out like the incumbent's (inc_z, inc_dec).  Written under the plan's lock by pool_insert_* (bnb.cu).
+  int pool_cap;
+  double *pool_z;           // [count][pool_cap][zstride]
+  unsigned char *pool_dec;  // [count][pool_cap][ndec_stride]
+  PoolRec *pool_rec;        // [count][pool_cap]
+  int *pool_cnt;            // [count]
+};
+
+// one plan's share of the solution pool, handed to the out-of-line insertion (kernel parameters stay in parameter space)
+struct PoolRef {
+  double *z; unsigned char *dec; PoolRec *rec; int *cnt;
+  int cap, zstride, ndec_stride;
 };
 
 void launch_bnb_init(const BnbState &st, const DevProb *probs, const unsigned char *warm_dec /* [count][ndec_stride] or null */,
@@ -90,6 +110,10 @@ void launch_bnb_fingerprint(const BnbState &st, unsigned long long *out, cudaStr
 void launch_bnb_tighten(const BnbState &st, const double *ub, cudaStream_t s);      // st.ub = min(st.ub, ub): incumbents of other ranks
 void launch_bnb_finish(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob,
                        double *xall, double *best_bound, cudaStream_t s);
+// full column vectors of n pool entries of plan k: block e expands entry idx[e] with eprobs[e] (plan k's DevProb, x_base = e * ncols)
+// into xall; the entry's trajectory goes to zs[e * zstride] (pool storage is not modified)
+void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const DevProb *eprobs, const double *dblob, const int *iblob,
+                        double *zs, double *xall, cudaStream_t s);
 int node_kernel_smem_per_warp(int maxN, int kmax, int ndec_stride);
 int node_kernel_narrow_np(int N);                                  // row stride of the (s, lambda) records of a two-warp team
 int node_kernel_smem_narrow(int N, int kmax, int ndec_stride);   // shared memory of a two-warp team (uniform horizon N)

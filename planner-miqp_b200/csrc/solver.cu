@@ -116,6 +116,10 @@ struct MiqpB200Solver {
   std::vector<double> h_z;                                     // compact results: incumbent trajectories
   int single_maxN = 2;
   size_t pool_budget = 0;
+  // solution pool: capacity requested for the next upload, device storage, fetch scratch (pool_* of BnbState)
+  int solution_pool = 0;
+  DevBuf<double> sp_z; DevBuf<unsigned char> sp_dec; DevBuf<PoolRec> sp_rec; DevBuf<int> sp_cnt;
+  DevBuf<DevProb> sp_probs; DevBuf<int> sp_idx; DevBuf<double> sp_x, sp_zs, sp_obj, sp_viol;
 };
 
 namespace {
@@ -419,6 +423,16 @@ void setup_bnb(MiqpB200Solver *s) {
   st.work_cnt2 = s->b_ctrl.p + 4; st.work_next2 = s->b_ctrl.p + 5; st.active_prev = s->b_ctrl.p + 6;
   s->d_x.ensure(std::max<long>(pk.total_cols, 1));
   s->d_viol.ensure(count); s->d_obj.ensure(count); s->d_bb.ensure(count);
+  // solution pool: storage only when it is on (config 2: about 3.2 kB per entry)
+  st.pool_cap = s->solution_pool;
+  st.pool_z = nullptr; st.pool_dec = nullptr; st.pool_rec = nullptr; st.pool_cnt = nullptr;
+  if (st.pool_cap > 0) {
+    const size_t entries = (size_t)count * st.pool_cap;
+    s->sp_z.ensure(entries * st.zstride); st.pool_z = s->sp_z.p;
+    s->sp_dec.ensure(entries * st.ndec_stride); st.pool_dec = s->sp_dec.p;
+    s->sp_rec.ensure(entries); st.pool_rec = s->sp_rec.p;
+    s->sp_cnt.ensure(count); st.pool_cnt = s->sp_cnt.p;
+  }
 }
 
 }  // namespace
@@ -474,6 +488,7 @@ void miqp_b200_destroy(MiqpB200Solver *s) {
   s->b_pruned.release(); s->b_incz.release(); s->b_meta.release(); s->b_work.release();
   s->b_uid.release(); s->b_keybuf.release(); s->b_incuid.release(); s->b_stats.release(); s->b_open.release();
   s->b_opencnt.release(); s->b_free.release(); s->b_freecnt.release(); s->b_sel.release(); s->b_selcnt.release();
+  s->sp_z.release(); s->sp_dec.release(); s->sp_rec.release(); s->sp_cnt.release();
   s->b_zpool.release(); s->b_susp0.release(); s->b_susp1.release(); s->b_suspslot.release(); s->b_suspcnt.release(); s->b_done.release(); s->b_overflow.release(); s->b_lock.release(); s->b_ctrl.release(); s->b_multi_ws.release(); s->b_work2.release();
   if (s->ev0) cudaEventDestroy(s->ev0);
   if (s->ev1) cudaEventDestroy(s->ev1);
@@ -993,6 +1008,87 @@ int miqp_b200_debug_profile(MiqpB200Solver *s, unsigned long long *out256) {
   if (!s || !out256 || !s->b_prof.p) return MIQP_B200_ERR_ARG;
   if (cudaMemcpy(out256, s->b_prof.p, 256 * sizeof(unsigned long long), cudaMemcpyDeviceToHost) != cudaSuccess)
     return fail(s, MIQP_B200_ERR_CUDA, "profile copy failed");
+  return MIQP_B200_OK;
+}
+
+// ---- solution pool --------------------------------------------------------------------------------------------------------
+int miqp_b200_set_solution_pool(MiqpB200Solver *s, int capacity) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (capacity < 0 || capacity > 64) return fail(s, MIQP_B200_ERR_ARG, "solution pool capacity must lie in 0..64");
+  s->solution_pool = capacity;
+  return MIQP_B200_OK;
+}
+
+static const char *pool_unavailable(const MiqpB200Solver *s) {
+  if (!s->uploaded || !s->ran) return "solution pool: no results of a batch_run on this solver";
+  if (s->st.pool_cap <= 0) return "solution pool: the pool was off when this batch was uploaded (miqp_b200_set_solution_pool)";
+  return nullptr;
+}
+
+int miqp_b200_pool_sizes(MiqpB200Solver *s, int *sizes) {
+  if (!s || !sizes) return MIQP_B200_ERR_ARG;
+  if (const char *why = pool_unavailable(s)) return fail(s, MIQP_B200_ERR_ARG, why);
+  if (cudaSetDevice(s->opt.device) != cudaSuccess ||
+      cudaMemcpyAsync(sizes, s->st.pool_cnt, sizeof(int) * s->st.count, cudaMemcpyDeviceToHost, s->stream) != cudaSuccess ||
+      cudaStreamSynchronize(s->stream) != cudaSuccess) return fail(s, MIQP_B200_ERR_CUDA, "copy of the solution pool sizes failed");
+  return MIQP_B200_OK;
+}
+
+// Entries of plan k best first: the records are sorted by (search value, uid) on the host, the chosen entries are expanded into
+// full column vectors on the device (pool_expand_kernel) and evaluated against the big-M model by evaluate_kernel.
+int miqp_b200_pool_fetch(MiqpB200Solver *s, int k, int max_entries, MiqpB200PoolEntry *entries, double *x_out, double *traj_out,
+                         int *n_out) {
+  if (!s || !entries || !n_out || max_entries < 0) return MIQP_B200_ERR_ARG;
+  if (const char *why = pool_unavailable(s)) return fail(s, MIQP_B200_ERR_ARG, why);
+  if (k < 0 || k >= s->st.count) return fail(s, MIQP_B200_ERR_ARG, "pool_fetch: plan index out of range");
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    const BnbState &st = s->st;
+    int cnt = 0;
+    std::vector<PoolRec> rec((size_t)st.pool_cap);
+    CK(cudaMemcpyAsync(&cnt, st.pool_cnt + k, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(rec.data(), st.pool_rec + (size_t)k * st.pool_cap, sizeof(PoolRec) * st.pool_cap, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    std::vector<int> idx(cnt);
+    for (int e = 0; e < cnt; ++e) idx[e] = e;
+    std::sort(idx.begin(), idx.end(), [&](int a, int b) {
+      return rec[a].val < rec[b].val || (rec[a].val == rec[b].val && rec[a].uid < rec[b].uid);
+    });
+    const int n = std::min(cnt, max_entries);
+    idx.resize(n);
+    *n_out = n;
+    if (n == 0) return MIQP_B200_OK;
+    DevProb p;   // the device copy: prepare_tables_kernel completes the plan's record there
+    CK(cudaMemcpyAsync(&p, s->d_probs.p + k, sizeof(DevProb), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    std::vector<DevProb> ep(n, p);
+    for (int e = 0; e < n; ++e) ep[e].x_base = (long)e * p.ncols;
+    s->sp_probs.ensure(n); s->sp_idx.ensure(n); s->sp_obj.ensure(n); s->sp_viol.ensure(n);
+    s->sp_x.ensure((size_t)n * p.ncols); s->sp_zs.ensure((size_t)n * st.zstride);
+    CK(cudaMemcpyAsync(s->sp_probs.p, ep.data(), sizeof(DevProb) * n, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->sp_idx.p, idx.data(), sizeof(int) * n, cudaMemcpyHostToDevice, s->stream));
+    launch_pool_expand(st, k, s->sp_idx.p, n, s->sp_probs.p, s->d_dblob.p, s->d_iblob.p, s->sp_zs.p, s->sp_x.p, s->stream);
+    CK(cudaMemsetAsync(s->sp_viol.p, 0, sizeof(double) * n, s->stream));
+    launch_evaluate(s->sp_probs.p, s->d_dblob.p, s->d_iblob.p, n, s->pk.max_rows, s->sp_x.p, s->sp_viol.p, s->sp_obj.p, s->stream);
+    CK(cudaGetLastError());
+    std::vector<double> obj(n), viol(n);
+    CK(cudaMemcpyAsync(obj.data(), s->sp_obj.p, sizeof(double) * n, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(viol.data(), s->sp_viol.p, sizeof(double) * n, cudaMemcpyDeviceToHost, s->stream));
+    if (x_out) CK(cudaMemcpyAsync(x_out, s->sp_x.p, sizeof(double) * n * p.ncols, cudaMemcpyDeviceToHost, s->stream));
+    const long tsz = (long)p.C * p.N * 8;   // the trajectory part of an entry's zstride doubles
+    if (traj_out)
+      for (int e = 0; e < n; ++e)
+        CK(cudaMemcpyAsync(traj_out + e * tsz, s->sp_zs.p + (size_t)e * st.zstride, sizeof(double) * tsz, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    for (int e = 0; e < n; ++e) {
+      const PoolRec &r = rec[idx[e]];
+      MiqpB200PoolEntry &o = entries[e];
+      o.objective = obj[e]; o.max_violation = viol[e]; o.search_value = r.val;
+      o.converged = r.converged; o.round = r.round; o.uid = r.uid;
+    }
+  } catch (const std::exception &ex) {
+    return fail(s, MIQP_B200_ERR_CUDA, ex.what());
+  }
   return MIQP_B200_OK;
 }
 

@@ -3,6 +3,7 @@
 #include "b200_wrapper.hpp"
 #include "dat_reader.hpp"
 
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -267,7 +268,8 @@ B200Wrapper::B200Wrapper(const B200Wrapper &o)
     : parameters_(o.parameters_), results_(std::make_shared<RawResults>()), precision_(o.precision_), device_(o.device_),
       useSos_(o.useSos_), useBranchingPriorities_(o.useBranchingPriorities_), bufferOutputs_(o.bufferOutputs_),
       debugPrint_(o.debugPrint_), collectSizes_(o.collectSizes_), prioStart_(o.prioStart_), prioExtent_(o.prioExtent_),
-      debugPath_(o.debugPath_), debugPrefix_(o.debugPrefix_), source_(o.source_), modPath_(o.modPath_), datFile_(o.datFile_) {}
+      debugPath_(o.debugPath_), debugPrefix_(o.debugPrefix_), source_(o.source_), modPath_(o.modPath_), datFile_(o.datFile_),
+      poolCapacity_(o.poolCapacity_) {}
 B200Wrapper &B200Wrapper::operator=(const B200Wrapper &o) { debugPath_ = o.debugPath_; return *this; }
 B200Wrapper::~B200Wrapper() { if (solver_) miqp_b200_destroy(solver_); }
 
@@ -455,6 +457,40 @@ bool B200Wrapper::EnsureSolver() {
   return true;
 }
 
+bool B200Wrapper::setSolutionPoolCapacity(int capacity) {
+  if (capacity < 0 || capacity > 64) return false;
+  poolCapacity_ = capacity;
+  return true;
+}
+
+bool B200Wrapper::getSolutionPoolResults(int j, RawResults &out) const {
+  if (j < 0 || j >= (int)pool_.size()) return false;
+  Unpack(poolLayout_, pool_[j].x.data(), out);
+  return true;
+}
+
+// pool of plan k of the last run on `solver` (capacity poolCapacity_), best first; clears the pool when it is off
+bool B200Wrapper::FetchPool(MiqpB200Solver *solver, int k, const MiqpB200Layout &layout) {
+  pool_.clear();
+  if (poolCapacity_ <= 0) return true;
+  std::vector<MiqpB200PoolEntry> e(poolCapacity_);
+  std::vector<double> x((size_t)poolCapacity_ * layout.ncols);
+  int n = 0;
+  if (miqp_b200_pool_fetch(solver, k, poolCapacity_, e.data(), x.data(), nullptr, &n) != MIQP_B200_OK) {
+    const char *m = miqp_b200_last_error(solver);
+    error_ = m ? m : "solution pool fetch failed";
+    return false;
+  }
+  pool_.resize(n);
+  for (int j = 0; j < n; ++j) {
+    SolutionPoolEntry &o = pool_[j];
+    o.objective = e[j].objective; o.max_violation = e[j].max_violation; o.converged = e[j].converged != 0;
+    o.x.assign(x.begin() + (size_t)j * layout.ncols, x.begin() + (size_t)(j + 1) * layout.ncols);
+  }
+  poolLayout_ = layout;
+  return true;
+}
+
 struct B200Wrapper::Prepared {
   FlatProblem flat;
   MiqpB200Layout layout{};
@@ -519,7 +555,7 @@ OptimizationStatus B200Wrapper::Finish(const Prepared &pr, const MiqpB200SolveIn
     // CPLEX status codes callers may look at: 101 optimal, 102 optimal within tolerance, 107 time limit with incumbent
     props_.status = info.proven ? (info.gap == 0.0 ? 101 : 102) : 107;
     props_.objective = info.objective; props_.gap = info.gap; props_.max_violation = info.max_violation;
-    props_.proven_gap = info.proven != 0; props_.NrSolutionPool = 1;
+    props_.proven_gap = info.proven != 0; props_.NrSolutionPool = poolCapacity_ > 0 ? (int)pool_.size() : 1;
     Unpack(pr.layout, x, *results_);
     lastX_.assign(x, x + pr.layout.ncols); lastLayout_ = pr.layout; haveLast_ = true;
     if (useLastSolution_) WriteMst(tmpWarmstartFile_, lastLayout_, lastX_);   // cplex.writeMIPStarts, src/cplex_wrapper.cpp:206-209
@@ -548,6 +584,7 @@ OptimizationStatus B200Wrapper::Finish(const Prepared &pr, const MiqpB200SolveIn
     return SUCCESS;
   }
   props_.objective = NAN; props_.gap = NAN;
+  pool_.clear();
   props_.status = (info.status == MIQP_B200_FAILED_TIMEOUT) ? 108 : 103;   // time limit without incumbent / integer infeasible
   return info.status == MIQP_B200_FAILED_TIMEOUT ? FAILED_TIMEOUT : FAILED_NO_SOLUT;
 }
@@ -571,8 +608,10 @@ OptimizationStatus B200Wrapper::callCplex(double timestamp) {
   const double *warm = pr.have_warm ? pr.warm.data() : nullptr;
   double *xo = x.data();
   MiqpB200SolveInfo info;
+  pool_.clear();
+  miqp_b200_set_solution_pool(solver_, poolCapacity_);   // (0..64: setSolutionPoolCapacity checked it)
   const int rc = miqp_b200_solve_batch(solver_, &pr.flat.p, 1, pr.have_warm ? &warm : nullptr, &xo, &info);
-  if (rc != MIQP_B200_OK) {
+  if (rc != MIQP_B200_OK || (info.status == MIQP_B200_SUCCESS && !FetchPool(solver_, 0, pr.layout))) {
     const char *e = miqp_b200_last_error(solver_);
     error_ = e ? e : "device solve failed";
     props_ = SolutionProperties(); props_.objective = NAN; props_.gap = NAN;
@@ -610,6 +649,10 @@ std::vector<OptimizationStatus> B200Wrapper::callBatch(const std::vector<B200Wra
   std::vector<B200Wrapper *> members(m);
   bool all_warm = true;
   for (int j = 0; j < m; ++j) { members[j] = solvers[idx[j]]; all_warm = all_warm && pr[idx[j]].have_warm; }
+  // solution pool: the batch keeps as many entries as its most demanding member asks for; each member takes its own share
+  int pool_cap = 0;
+  for (B200Wrapper *w : members) pool_cap = std::max(pool_cap, w->poolCapacity_);
+  miqp_b200_set_solution_pool(lead->solver_, pool_cap);   // (0..64: setSolutionPoolCapacity checked it)
   int rc;
   if (lead->deviceWarmstart_ && all_warm && m > 1 && lead->lastBatch_ == members) {
     rc = miqp_b200_batch_upload_replan(lead->solver_, probs.data(), m);
@@ -625,8 +668,16 @@ std::vector<OptimizationStatus> B200Wrapper::callBatch(const std::vector<B200Wra
     for (int k : idx) solvers[k]->error_ = e ? e : "device solve failed";
     return out;
   }
+  for (int j = 0; j < m; ++j) {   // before Finish: its model statistics (collectSizes_) replace the batch on the lead's handle
+    B200Wrapper *w = solvers[idx[j]];
+    if (infos[j].status == MIQP_B200_SUCCESS && !w->FetchPool(lead->solver_, j, pr[idx[j]].layout)) {
+      out[idx[j]] = FAILED_SEG_FAULT;
+      infos[j].status = -1;
+    }
+  }
   for (int j = 0; j < m; ++j) {
     B200Wrapper *w = solvers[idx[j]];
+    if (infos[j].status == -1) continue;
     if (w->collectSizes_ && !w->EnsureSolver()) w->collectSizes_ = false;
     out[idx[j]] = w->Finish(pr[idx[j]], infos[j], xs[j].data(), timestamp);
   }

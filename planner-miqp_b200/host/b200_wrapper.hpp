@@ -49,6 +49,13 @@ std::vector<std::string> ColumnNames(const MiqpB200Layout &l);
 bool WriteMst(const std::string &path, const MiqpB200Layout &l, const std::vector<double> &x);
 bool ReadMst(const std::string &path, int ncols, std::vector<double> &x);
 
+// member of the solution pool (miqp_b200_pool_fetch): objective and violation of its full column vector, device-evaluated
+struct SolutionPoolEntry {
+  double objective = 0.0, max_violation = 0.0;
+  bool converged = false;   // the leaf QP was solved to optimality
+  std::vector<double> x;    // full column vector (decision_variables.mod order): Unpack() gives its RawResults
+};
+
 class B200Wrapper {
  public:
   enum ParameterSource { DATFILE = 0, CPPINPUTS = 1, MIXED = 2 };
@@ -91,6 +98,13 @@ class B200Wrapper {
   bool readMIPStarts(const std::string &mstfile);          // becomes the "last solution" MIP start
   void setCollectModelStatistics(bool in) { collectSizes_ = in; }   // rows / non-zeros cost one more device pass
   void setDevice(int ordinal);
+  // Solution pool: up to `capacity` (0..64, 0 = off) best distinct feasible plans of every solve, entry 0 = the returned solution.
+  // With the pool on, SolutionProperties.NrSolutionPool counts its entries.  Returns false for a capacity outside 0..64.
+  bool setSolutionPoolCapacity(int capacity);
+  int getSolutionPoolCapacity() const { return poolCapacity_; }
+  const std::vector<SolutionPoolEntry> &getSolutionPool() const { return pool_; }
+  // RawResults of pool entry j (false if there is no such entry)
+  bool getSolutionPoolResults(int j, RawResults &out) const;
 
   // one MIQP solve of the bound ModelParameters; `timestamp` only names the debug files
   OptimizationStatus callCplex(double timestamp = 0.0);
@@ -113,6 +127,7 @@ class B200Wrapper {
   bool Prepare(double timestamp, Prepared &out);
   OptimizationStatus Finish(const Prepared &pr, const MiqpB200SolveInfo &info, const double *x, double timestamp);
   bool EnsureSolver();
+  bool FetchPool(MiqpB200Solver *solver, int k, const MiqpB200Layout &layout);
 
   std::shared_ptr<ModelParameters> parameters_;
   std::shared_ptr<RawResults> results_;
@@ -135,6 +150,9 @@ class B200Wrapper {
   std::vector<double> lastX_;           // last solution vector (the ".mst" of the reference)
   MiqpB200Layout lastLayout_{};
   bool haveLast_ = false;
+  int poolCapacity_ = 0;
+  std::vector<SolutionPoolEntry> pool_;   // of the last solve
+  MiqpB200Layout poolLayout_{};
 };
 
 typedef B200Wrapper CplexWrapper;   // reference-side code keeps its spelling

@@ -1,6 +1,7 @@
 // miqp_planner.cpp -- see miqp_planner.hpp.  Reference: src/miqp_planner.cpp.
 #include "miqp_planner.hpp"
 #include "convexified_map.hpp"
+#include "../../include/miqp_planner_c_api.h"   // TRAJECTORY_* row layout
 
 #include <algorithm>
 #include <array>
@@ -501,6 +502,29 @@ std::vector<std::array<double, 5>> MiqpPlanner::GetTrajectory(int c, double star
     out.push_back({start_time + i * dt, r->pos_x(c, i), r->pos_y(c, i), std::atan2(vy, vx), std::sqrt(vx * vx + vy * vy)});
   }
   return out;
+}
+
+void MiqpPlanner::RawTrajectoryRows(const RawResults &r, int carIdx, double start_time, float dt, double *trajectory, int &size) {
+  const int N = r.N;
+  size = N;
+  double time = start_time;
+  for (int i = 0; i < N; ++i) {
+    double *row = trajectory + (long)i * TRAJECTORY_SIZE;
+    row[TRAJECTORY_TIME_IDX] = time;
+    row[TRAJECTORY_X_IDX] = r.pos_x(carIdx, i); row[TRAJECTORY_Y_IDX] = r.pos_y(carIdx, i);
+    row[TRAJECTORY_VX_IDX] = r.vel_x(carIdx, i); row[TRAJECTORY_VY_IDX] = r.vel_y(carIdx, i);
+    row[TRAJECTORY_AX_IDX] = r.acc_x(carIdx, i); row[TRAJECTORY_AY_IDX] = r.acc_y(carIdx, i);
+    row[TRAJECTORY_UX_IDX] = r.u_x(carIdx, i); row[TRAJECTORY_UY_IDX] = r.u_y(carIdx, i);
+    time += dt;
+  }
+}
+
+double MiqpPlanner::GetSolutionPoolTrajectory(int j, int carIdx, double start_time, double *trajectory, int &size) const {
+  RawResults r;
+  size = 0;
+  if (!cplexWrapper_.getSolutionPoolResults(j, r) || carIdx < 0 || carIdx >= r.NrCars) return NAN;
+  RawTrajectoryRows(r, carIdx, start_time, parameters_->ts, trajectory, size);
+  return cplexWrapper_.getSolutionPool()[j].objective;
 }
 
 void MiqpPlanner::CarStateToMiqpState(float x, float y, float theta, float v, float a, double out[6]) {

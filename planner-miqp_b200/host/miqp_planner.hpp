@@ -72,6 +72,12 @@ class MiqpPlanner {
   static std::vector<bool> PlanBatch(const std::vector<MiqpPlanner *> &planners, double timestamp = 0.0);
 
   std::shared_ptr<RawResults> GetSolution() const { return cplexWrapper_.getRawResults(); }
+  // Solution pool of every Plan() / PlanBatch(): up to `capacity` (0..64, 0 = off) best distinct feasible plans, entry 0 = the
+  // solution Plan() returned.  GetSolutionPoolTrajectory fills rows like GetRawCMiqpTrajectoryCMiqpPlanner and returns the
+  // entry's objective (NaN and size 0 if there is no entry j).
+  bool SetSolutionPoolCapacity(int capacity) { return cplexWrapper_.setSolutionPoolCapacity(capacity); }
+  int GetSolutionPoolSize() const { return (int)cplexWrapper_.getSolutionPool().size(); }
+  double GetSolutionPoolTrajectory(int j, int carIdx, double start_time, double *trajectory, int &size) const;
   SolutionProperties GetSolutionProperties() const { return cplexWrapper_.getSolutionProperties(); }
   const cplex::B200Wrapper &GetCplexWrapper() const { return cplexWrapper_; }
   cplex::B200Wrapper &GetCplexWrapper() { return cplexWrapper_; }
@@ -97,6 +103,8 @@ class MiqpPlanner {
   static bool IsVxVyValid(double vx, double vy) { return std::fabs(vx) > 0.7 || std::fabs(vy) > 0.7; }
   // {x, y, theta, v, a} -> {x, vx, ax, y, vy, ay}, in float like the reference (src/miqp_planner.cpp:1189-1199)
   static void CarStateToMiqpState(float x, float y, float theta, float v, float a, double out[6]);
+  // rows {t, x, y, vx, vy, ax, ay, ux, uy} of car carIdx (TRAJECTORY_* of the planner C ABI), N rows from start_time in steps of dt
+  static void RawTrajectoryRows(const RawResults &r, int carIdx, double start_time, float dt, double *trajectory, int &size);
 
  private:
   struct PlanContext { std::vector<std::vector<int>> combos; size_t next = 0; std::vector<char> rollback; bool ready = false; };

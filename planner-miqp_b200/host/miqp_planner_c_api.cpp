@@ -1,6 +1,7 @@
 // miqp_planner_c_api.cpp -- extern "C" shim over MiqpPlanner (include/miqp_planner_c_api.h).
 // Same entry points and behaviour as the reference's src/miqp_planner_c_api.cpp:20-260.
 #include "../../include/miqp_planner_c_api.h"
+#include "../../include/miqp_planner_solution_pool.h"
 
 #include <cassert>
 #include <cmath>
@@ -85,19 +86,7 @@ float GetCollisionRadius(CMiqpPlanner h) { return P(h)->GetCollisionRadius(); }
 void GetRawCMiqpTrajectoryCMiqpPlanner(CMiqpPlanner h, int carIdx, double start_time, double *trajectory, int &size) {
   const std::shared_ptr<RawResults> r = P(h)->GetSolution();
   assert(carIdx < r->NrCars);
-  const int N = r->N;
-  const float dt = P(h)->GetParameters()->ts;
-  size = N;
-  double time = start_time;
-  for (int i = 0; i < N; ++i) {
-    double *row = trajectory + (long)i * TRAJECTORY_SIZE;
-    row[TRAJECTORY_TIME_IDX] = time;
-    row[TRAJECTORY_X_IDX] = r->pos_x(carIdx, i); row[TRAJECTORY_Y_IDX] = r->pos_y(carIdx, i);
-    row[TRAJECTORY_VX_IDX] = r->vel_x(carIdx, i); row[TRAJECTORY_VY_IDX] = r->vel_y(carIdx, i);
-    row[TRAJECTORY_AX_IDX] = r->acc_x(carIdx, i); row[TRAJECTORY_AY_IDX] = r->acc_y(carIdx, i);
-    row[TRAJECTORY_UX_IDX] = r->u_x(carIdx, i); row[TRAJECTORY_UY_IDX] = r->u_y(carIdx, i);
-    time += dt;
-  }
+  MiqpPlanner::RawTrajectoryRows(*r, carIdx, start_time, P(h)->GetParameters()->ts, trajectory, size);
 }
 
 void GetRawCLastReferenceTrajectoryCMiqpPlaner(CMiqpPlanner h, int carIdx, double start_time, double *trajectory, int &size) {
@@ -150,6 +139,12 @@ int PlanBatchCMiqpPlanner(CMiqpPlanner *planners, int count, const double timest
   int n = 0;
   for (int k = 0; k < count; ++k) { if (success) success[k] = ok[k]; n += ok[k]; }
   return n;
+}
+
+bool SetSolutionPoolCapacityCMiqpPlanner(CMiqpPlanner h, int capacity) { return P(h)->SetSolutionPoolCapacity(capacity); }
+int GetSolutionPoolSizeCMiqpPlanner(CMiqpPlanner h) { return P(h)->GetSolutionPoolSize(); }
+double GetSolutionPoolTrajectoryCMiqpPlanner(CMiqpPlanner h, int j, int carIdx, double start_time, double *trajectory, int &size) {
+  return P(h)->GetSolutionPoolTrajectory(j, carIdx, start_time, trajectory, size);
 }
 
 long DeviceWarmstartBatchesCMiqpPlanner() { return miqp::planner::cplex::B200Wrapper::deviceWarmstartBatches(); }

@@ -107,7 +107,7 @@ struct SolutionProperties {
   double gap = 0.0, objective = 0.0, time = 0.0;
   int NrConstraints = 0, NrBinaryVariables = 0, NrFloatVariables = 0, NonZeroCoefficients = 0;
   int NrIterations = 0;     // interior-point iterations summed over all node relaxations
-  int NrSolutionPool = 0;   // 1 if an incumbent exists
+  int NrSolutionPool = 0;   // entries of the solution pool (B200Wrapper::setSolutionPoolCapacity); with the pool off 1 if an incumbent exists
   // additions of the device search
   long NrNodes = 0, NrRounds = 0;
   double best_bound = 0.0, max_violation = 0.0;

@@ -83,7 +83,16 @@ PYBIND11_MODULE(miqp, m) {
       .def("exportModel", &CplexWrapper::exportModel)
       .def("writeMIPStarts", &CplexWrapper::writeMIPStarts)
       .def("readMIPStarts", &CplexWrapper::readMIPStarts)
-      .def("lastError", &CplexWrapper::lastError);
+      .def("lastError", &CplexWrapper::lastError)
+      .def("getSolutionVector", [](const CplexWrapper &w) { const std::vector<double> &x = w.getSolutionVector(); return py::array_t<double>(x.size(), x.data()); })
+      // solution pool: up to `capacity` best distinct feasible plans of every solve, best first (entry 0 = the solution)
+      .def("setSolutionPoolCapacity", &CplexWrapper::setSolutionPoolCapacity)
+      .def("getSolutionPool", [](const CplexWrapper &w) {
+        py::list out;
+        for (const miqp::planner::cplex::SolutionPoolEntry &e : w.getSolutionPool())
+          out.append(py::make_tuple(e.objective, e.max_violation, e.converged, py::array_t<double>(e.x.size(), e.x.data())));
+        return out;
+      }, "list of (objective, max_violation, converged, full column vector)");
 
   // ---- BehaviorMiqpAgent (src/behavior_miqp_agent.cpp:37-335) -------------------------------------------------------------
   using miqp::planner::BehaviorMiqpAgent;
@@ -173,7 +182,8 @@ PYBIND11_MODULE(miqp, m) {
       .def_readwrite("objective", &SolutionProperties::objective)
       .def_readwrite("status", &SolutionProperties::status)
       .def_readwrite("gap", &SolutionProperties::gap)
-      .def_readwrite("time", &SolutionProperties::time);
+      .def_readwrite("time", &SolutionProperties::time)
+      .def_readwrite("NrSolutionPool", &SolutionProperties::NrSolutionPool);
 
   py::enum_<MiqpPlannerWarmstartType>(m, "WarmstartType")
       .value("NO_WARMSTART", NO_WARMSTART)

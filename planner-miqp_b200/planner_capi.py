@@ -20,6 +20,10 @@ C_API_SYMBOLS = [
     # additions of this backend
     "PlanBatchCMiqpPlanner", "GetSolutionPropertiesCMiqpPlanner", "DeviceWarmstartBatchesCMiqpPlanner",
 ]
+# include/miqp_planner_solution_pool.h
+SOLUTION_POOL_SYMBOLS = [
+    "SetSolutionPoolCapacityCMiqpPlanner", "GetSolutionPoolSizeCMiqpPlanner", "GetSolutionPoolTrajectoryCMiqpPlanner",
+]
 
 
 class MiqpPlannerSettings(C.Structure):
@@ -121,6 +125,12 @@ def load_library():
     lib.DebugSetSolutionCMiqpPlanner.restype = b
     lib.DebugWarmstartCMiqpPlanner.argtypes = [vp, _dp, i, b]
     lib.DebugWarmstartCMiqpPlanner.restype = i
+    lib.SetSolutionPoolCapacityCMiqpPlanner.argtypes = [vp, i]
+    lib.SetSolutionPoolCapacityCMiqpPlanner.restype = b
+    lib.GetSolutionPoolSizeCMiqpPlanner.argtypes = [vp]
+    lib.GetSolutionPoolSizeCMiqpPlanner.restype = i
+    lib.GetSolutionPoolTrajectoryCMiqpPlanner.argtypes = [vp, i, i, d, _dp, C.POINTER(i)]
+    lib.GetSolutionPoolTrajectoryCMiqpPlanner.restype = d
     _lib = lib
     return lib
 
@@ -230,6 +240,20 @@ class CMiqpPlanner:
         if n != ncols:
             raise ValueError("column count does not match the planner's model")
         return out
+
+    # ---- solution pool (include/miqp_planner_solution_pool.h) ----
+    def set_solution_pool(self, capacity: int) -> bool:
+        return bool(self.lib.SetSolutionPoolCapacityCMiqpPlanner(self.h, int(capacity)))
+
+    def solution_pool_size(self) -> int:
+        return self.lib.GetSolutionPoolSizeCMiqpPlanner(self.h)
+
+    def solution_pool_trajectory(self, j: int, car=0, t0=0.0):
+        """(objective, rows like trajectory()) of pool entry j"""
+        out = np.zeros((self.N, TRAJECTORY_SIZE))
+        n = C.c_int(0)
+        obj = self.lib.GetSolutionPoolTrajectoryCMiqpPlanner(self.h, int(j), car, t0, out.ctypes.data_as(_dp), C.byref(n))
+        return obj, out[:n.value]
 
     def write_parameters(self, path: str) -> bool:
         return bool(self.lib.DebugWriteParametersCMiqpPlanner(self.h, path.encode(), 0))
