@@ -47,8 +47,6 @@ __device__ __forceinline__ unsigned long long node_key(double bound, int depth, 
   if (newborn) return (r << 47) | (b << 7) | u;
   return (1ULL << 63) | (b << 17) | (d << 7) | u;
 }
-__device__ __forceinline__ int meta_rank(int my) { return (my & 0xff) - 1; }
-__device__ __forceinline__ int meta_birth(int my) { return my >> 8; }
 
 // ---------------------------------------------------------------------------------------
 // init
@@ -69,10 +67,10 @@ __global__ void bnb_init_kernel(BnbState st, const DevProb *probs, const unsigne
   }
   if (tid == 0) {
     st.free_cnt[s] = st.cap - nroot;
-    st.bound[pb] = -MQ_INF; st.meta[pb] = make_int2(0, 1); st.uid[pb] = 1ULL;
+    st.bound[pb] = -MQ_INF; st.meta[pb] = make_int2(0, meta_word(0, 0)); st.uid[pb] = 1ULL;
     st.open_idx[pb] = 0;
     if (nroot == 2) {  // MIP start: the fully decided node is evaluated first (cplex_wrapper.cpp:494-639)
-      st.bound[pb + 1] = -MQ_INF; st.meta[pb + 1] = make_int2(1 << 20, 0); st.uid[pb + 1] = 2ULL;   // rank -1: before the root
+      st.bound[pb + 1] = -MQ_INF; st.meta[pb + 1] = make_int2(DEPTH_MIP_START, meta_word(0, -1)); st.uid[pb + 1] = 2ULL;   // rank -1: before the root
       st.open_idx[pb + 1] = 1;
     }
     if (st.zpool) for (int r = 0; r < nroot; ++r) st.zpool[(pb + r) * (long)st.zp_stride] = __longlong_as_double(0x7ff8000000000000LL);   // no parent: cold start
@@ -513,30 +511,6 @@ __device__ __forceinline__ double alt_delta(const WarpCtx &w, const Branch &br, 
 // ---------------------------------------------------------------------------------------
 // node kernel
 // ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void copy_bytes16(unsigned char *dst, const unsigned char *src, int nbytes, int lane) {
-  const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
-  uint4 *d4 = reinterpret_cast<uint4 *>(dst);
-  for (int k = lane; k < nbytes / 16; k += 32) d4[k] = s4[k];
-}
-
-// solution pool: a leaf of bnb_nodes_kernel (warp 0, plan lock held) goes in if it is among the pool's best (pool_slot).  Out of
-// line so that the node kernel keeps its register allocation; it runs only at leaves and only when the pool is on.
-__device__ __noinline__ void pool_insert_warp(PoolRef pr, const unsigned char *dec, const double *V, int N, double val,
-                                              unsigned long long uid, int round, int converged, int lane) {
-  const int slot = pool_slot(pr, dec, val, uid, lane, 32, [](bool p) { return __any_sync(FULL, p) != 0; });
-  __syncwarp();   // every lane has read the pool before it changes
-  if (slot < 0) return;
-  double *z = pr.z + (long)slot * pr.zstride;
-  for (int k = lane; k < N * 8; k += 32) z[k] = V[(k >> 3) * V_STRIDE + V_Z + (k & 7)];
-  copy_bytes16(pr.dec + (long)slot * pr.ndec_stride, dec, pr.ndec_stride, lane);
-  if (lane == 0) {
-    PoolRec r; r.val = val; r.uid = uid; r.round = round; r.converged = converged;
-    pr.rec[slot] = r;
-    const int cnt = __ldcg(pr.cnt);
-    if (slot == cnt) *pr.cnt = cnt + 1;
-  }
-}
-
 __device__ __forceinline__ void effective_regions(const WarpCtx &w) {
   const DevProb &p = *w.p;
   if (w.lane == 0) {
@@ -591,6 +565,7 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
   const NodeSmem L = node_smem_layout(maxN, st.kmax, st.ndec_stride, row_np);
   WarpCtx w;
   w.D = dblob; w.I = iblob; w.lane = lane; w.wid = wid; w.nw = nw; w.red = s_red;
+  const WarpGroup g{lane};   // warp 0 handles the solved node
   w.dbgrow = nullptr; w.tau_k = st.tau_k;
 #ifdef MQ_PROF
   if (st.dbg && blockIdx.x < 1024) w.dbgrow = st.dbg + (size_t)blockIdx.x * 512;
@@ -624,7 +599,7 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
     w.sgmul = 65536 / w.sg + 1; w.NP = team_row_stride(p.N, w.sg); w.kmax = st.kmax;
     double pen = 0.0;
     if (wid == 0) {
-      copy_bytes16(w.dec, st.dec + (pb + slot) * st.ndec_stride, st.ndec_stride, lane);
+      copy_dec(g, w.dec, st.dec + (pb + slot) * st.ndec_stride, st.ndec_stride);
       __syncwarp();
       effective_regions(w);
       // constant cost of SOFT obstacle decisions
@@ -702,18 +677,9 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
       atomicAdd(&st.prof[137], (unsigned long long)r.c_e); atomicAdd(&st.prof[138], (unsigned long long)r.c_g); atomicAdd(&st.prof[139], (unsigned long long)r.c_atr);
     }
 #endif
-    if (lane == 0) {
-      atomicAdd(&st.stat_nodes[s], 1ULL);
-      atomicAdd(&st.stat_iters[s], (unsigned long long)r.iters);
-      atomicAdd(&st.stat_rows[s], (unsigned long long)r.rows);
-    }
+    if (lane == 0) count_node(st, s, r.iters, r.rows);
     if (r.status == 1) continue;  // proven infeasible (empty box or Farkas certificate): the node dies
-    if (r.status != 0) {
-      // neither solved nor refuted: the node is closed, but its bound stays in the books (the plan cannot be reported as
-      // proven below it) and the event is counted
-      if (lane == 0) { atomic_min_double(&st.pruned_lb[s], nbound); atomicAdd(&st.stat_uncert[s], 1ULL); }
-      continue;
-    }
+    if (r.status != 0) { if (lane == 0) close_uncertified(st, s, nbound); continue; }
     // fval: objective of the point in V_Z (an upper bound of the relaxation); obj: lower bound of the node.  They coincide
     // when the interior-point iteration converged; a stalled iteration yields the Lagrangian bound of its multipliers.
     const double fval = r.obj + pen;
@@ -733,46 +699,15 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
       // is reported as proven only if the incumbent comes within the gap of it.
       if (lane == 0) atomic_min_double(&st.pruned_lb[s], obj);
     }
-    if (br.kind == 0 && und == 0) {
-      // every disjunction decided and satisfied: incumbent candidate
-      if (lane == 0 && !r.converged) atomic_min_double(&st.pruned_lb[s], obj);   // the leaf's optimum may lie below the stalled point, not below obj
-      warp_lock(&st.lock[s], lane);
-      const double cur = *reinterpret_cast<volatile double *>(&st.ub[s]);
-      const unsigned long long cuid = *reinterpret_cast<volatile unsigned long long *>(&st.inc_uid[s]);
-      const double inc = fval > obj ? fval : obj;   // value of the stored point (never below the node's bound)
-      if (inc < cur || (inc == cur && nuid < cuid)) {
-        double *iz = st.inc_z + (long)s * st.zstride;
-        for (int i = lane; i < p.N; i += 32)
-          for (int t = 0; t < 8; ++t) iz[i * 8 + t] = w.V[i * V_STRIDE + V_Z + t];
-        copy_bytes16(st.inc_dec + (long)s * st.ndec_stride, w.dec, st.ndec_stride, lane);
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) { st.ub[s] = inc; st.inc_uid[s] = nuid; }
-      }
-      if (st.pool_cap > 0) pool_insert_warp(pool_ref(st, s), w.dec, w.V, p.N, inc, nuid, round, r.converged ? 1 : 0, lane);
-      warp_unlock(&st.lock[s], lane);
+    const Traj t = {w.V + V_Z, V_STRIDE, 1, p.N, nullptr, 0, 0};
+    if (br.kind == 0 && und == 0) {   // every disjunction decided and satisfied: incumbent candidate
+      offer_leaf(g, st, s, w.dec, t, fval > obj ? fval : obj, obj, r.converged, true, nuid, round);
       continue;
     }
     // children
-    int nalt = 0, soff = 0;
-    const unsigned char *src = w.dec;
-    if (br.kind == 0) { nalt = 1; src = w.imp; soff = -1; }
-    else if (br.kind == 1) {
-      soff = p.off_mode + br.i;
-      const int na = w.I[p.o_nalt];
-      nalt = na + 1;
-      if (lane == 0) { alts[0] = MODE_FROZEN; for (int a = 0; a < na; ++a) alts[1 + a] = (unsigned char)w.I[p.o_alt + a]; }
-    } else if (br.kind == 2) {
-      soff = p.off_env + br.i * 5 + br.pt;
-      nalt = p.E;
-      if (lane == 0) for (int e = 0; e < p.E; ++e) alts[e] = (unsigned char)e;
-    } else {
-      soff = p.off_obs + (br.o * p.N + br.i) * 5 + br.pt;
-      const int ne = w.I[p.o_obs_nedges + br.o * p.N + br.i];
-      nalt = ne;
-      if (lane == 0) { for (int e = 0; e < ne; ++e) alts[e] = (unsigned char)e; }
-      if (w.I[p.o_obs_soft + br.o] == 1) { if (lane == 0) alts[ne] = OBS_SOFT; nalt = ne + 1; }
-    }
+    int nalt = 1, soff = -1;
+    const unsigned char *src = w.imp;
+    if (br.kind != 0) { nalt = branch_alts(p, w.I, br.kind, 0, br.i, br.o, br.pt, 0, 0, soff, lane == 0 ? alts : nullptr); src = w.dec; }
     __syncwarp();
     // child bounds (lane = alternative); the (s, lambda) records are dead after the QP solve and
     // serve as scratch.  Children that reach the cutoff are dropped.
@@ -781,48 +716,17 @@ __global__ void __launch_bounds__(NW * 32, NW == 4 ? NODE_TEAMS_PER_SM : NW == 2
     else for (int a = lane; a < nalt; a += 32) cb[a] = r.converged ? fmax(obj, fval + 0.999 * alt_delta(w, br, alts[a])) : obj;
     __syncwarp();
     {
-      int nk = 0; double pm = MQ_INF;
+      int nk = 0; double pm;
       if (lane == 0) {
-        for (int a = 0; a < nalt; ++a) {
-          if (cb[a] >= cutoff) { pm = fmin(pm, cb[a]); continue; }
-          alts[nk] = alts[a]; cb[nk] = cb[a]; ++nk;
-        }
+        nk = drop_cut_children(alts, cb, nalt, cutoff, pm);
         if (pm < MQ_INF) atomic_min_double(&st.pruned_lb[s], pm);
       }
       nalt = __shfl_sync(FULL, nk, 0);
     }
     __syncwarp();
     if (nalt == 0) continue;
-    int fbase = 0, opos = 0, ok = 1;
-    if (lane == 0) {
-      const int old = atomicSub(&st.free_cnt[s], nalt);
-      if (old < nalt) {   // node pool of this plan exhausted: the children are dropped, their bound stays in the books
-        atomicAdd(&st.free_cnt[s], nalt); atomicExch(&st.overflow[s], 1); atomic_min_double(&st.pruned_lb[s], obj); ok = 0;
-      }
-      else { fbase = old - nalt; opos = atomicAdd(&st.open_cnt[s], nalt); }
-    }
-    ok = __shfl_sync(FULL, ok, 0); fbase = __shfl_sync(FULL, fbase, 0); opos = __shfl_sync(FULL, opos, 0);
-    if (!ok) continue;
-    for (int a = 0; a < nalt; ++a) {
-      const int cs = st.free_stack[pb + fbase + a];
-      unsigned char *dst = st.dec + (pb + cs) * st.ndec_stride;
-      copy_bytes16(dst, src, st.ndec_stride, lane);
-      if (st.zpool) {   // the child starts its interior-point solve from this node's relaxed optimum
-        double *zc = st.zpool + (pb + cs) * (long)st.zp_stride;
-        for (int k = lane; k < p.N * 8; k += 32) zc[k] = w.V[(k >> 3) * V_STRIDE + V_Z + (k & 7)];
-      }
-      __syncwarp();
-      if (lane == 0) {
-        int rank = 0;
-        if (soff >= 0) { dst[soff] = alts[a]; rank = (alts[a] == w.imp[soff]) ? -1 : a; }
-        st.bound[pb + cs] = cb[a];
-        st.meta[pb + cs] = make_int2(nmeta.x >= (1 << 20) ? nmeta.x : nmeta.x + 1, (round << 8) | (rank + 1));
-        st.uid[pb + cs] = mix64(nuid * 0x9e3779b97f4a7c15ULL + (unsigned long long)(a + 1));
-        st.open_idx[pb + opos + a] = cs;
-        if (st.susp_slot) st.susp_slot[pb + cs] = -1;
-      }
-    }
-    __syncwarp();
+    // (the children start their interior-point solves from this node's relaxed optimum)
+    push_children(g, st, s, round, nmeta.x, nuid, obj, nalt, src, 0, nullptr, soff, alts, cb, w.imp, st.zpool ? &t : nullptr);
   }
 }
 

@@ -5,6 +5,7 @@
 // compiles for the host with one thread (MQ_EMULATE) for the CPU tests of the logic.
 #pragma once
 #include "node_qp_multi.cuh"
+#include "bnb_common.cuh"
 
 namespace miqp {
 
@@ -332,39 +333,12 @@ MQ_FN MNodeOut m_process_node(const MCtx &k, MShared *sh, double nbound, double 
   if (br.kind == 0 && und == 0) { out.what = MN_INCUMBENT; return out; }
   out.what = MN_BRANCH;
   if (br.kind == 0) { out.nalt = 1; out.from_imp = true; out.soff = -1; if (k.tid == 0) sh->cb[0] = obj; k.sync(); return out; }
-  out.pruned_min = MQM_INF;
-  if (br.kind == 1) {
-    out.soff = p.off_mode + br.c * k.N + br.i;
-    const int na = k.I[p.o_nalt + br.c];
-    out.nalt = na + 1;
-    if (k.tid == 0) { sh->alts[0] = MODE_FROZEN; for (int a = 0; a < na; ++a) sh->alts[1 + a] = (unsigned char)k.I[p.o_alt + br.c * 4 * p.R + a]; }
-  } else if (br.kind == 2) {
-    out.soff = p.off_env + (br.c * k.N + br.i) * 5 + br.pt;
-    out.nalt = p.E;
-    if (k.tid == 0) for (int e = 0; e < p.E; ++e) sh->alts[e] = (unsigned char)e;
-  } else if (br.kind == 3) {
-    out.soff = p.off_obs + ((br.c * p.O + br.o) * k.N + br.i) * 5 + br.pt;
-    const int ne = k.I[p.o_obs_nedges + br.o * k.N + br.i];
-    out.nalt = ne;
-    if (k.tid == 0) for (int e = 0; e < ne; ++e) sh->alts[e] = (unsigned char)e;
-    if (k.I[p.o_obs_soft + br.o] == 1) { if (k.tid == 0) sh->alts[ne] = OBS_SOFT; out.nalt = ne + 1; }
-  } else {
-    out.soff = p.off_pair + (br.pr * k.N + br.i) * 4 + br.q;
-    out.nalt = 4;
-    if (k.tid == 0) for (int e = 0; e < 4; ++e) sh->alts[e] = (unsigned char)e;
-  }
+  out.nalt = branch_alts(p, k.I, br.kind, br.c, br.i, br.o, br.pt, br.pr, br.q, out.soff, k.tid == 0 ? sh->alts : nullptr);
   k.sync();
   // child bounds; children that reach the cutoff are dropped here
   PFOR(a, out.nalt) sh->cb[a] = r.converged ? fmax(obj, fval + 0.999 * m_alt_delta(k, br, sh->alts[a])) : obj;
   k.sync();
-  if (k.tid == 0) {
-    int n = 0; double pm = MQM_INF;
-    for (int a = 0; a < out.nalt; ++a) {
-      if (sh->cb[a] >= cutoff) { pm = fmin(pm, sh->cb[a]); continue; }
-      sh->alts[n] = sh->alts[a]; sh->cb[n] = sh->cb[a]; ++n;
-    }
-    sh->nkeep = n; sh->pruned_min = pm;
-  }
+  if (k.tid == 0) sh->nkeep = drop_cut_children(sh->alts, sh->cb, out.nalt, cutoff, sh->pruned_min);
   k.sync();
   out.nalt = sh->nkeep; out.pruned_min = sh->pruned_min;
   k.sync();

@@ -75,7 +75,7 @@ struct BnbState {
   int2 *work; int *work_cnt; int *work_next; int *active; int *err; int *active_prev;
   int2 *work2; int *work_cnt2; int *work_next2;   // plans with NumCars > 1 (bnb_multi.cu)
   // solution pool (pool_cap > 0): the pool_cap best distinct leaves of every plan by the incumbent's key (value, uid), unsorted;
-  // records laid out like the incumbent's (inc_z, inc_dec).  Written under the plan's lock by pool_insert_* (bnb.cu).
+  // records laid out like the incumbent's (inc_z, inc_dec).  Written under the plan's lock by pool_insert (bnb_common.cuh).
   int pool_cap;
   double *pool_z;           // [count][pool_cap][zstride]
   unsigned char *pool_dec;  // [count][pool_cap][ndec_stride]
