@@ -24,6 +24,9 @@
  *                                  collectSolutionStatus, src/cplex_wrapper.cpp:158-249,
  *                                  :311-448, :672-678; MIP start :494-639
  * miqp_b200_batch_* (resident)     the same solve with the batch already in HBM
+ * miqp_b200_batch_run_streaming    the same run, each plan's result handed to a callback in
+ *                                  the round its search ends (one result per cplex.solve()
+ *                                  of the reference, instead of one per batch)
  * miqp_b200_set_solution_pool      the solution pool of cplex.solve(); its size is
  *                                  SolutionProperties.NrSolutionPool, collectCplexStatistics,
  *                                  src/cplex_wrapper.cpp:680-690
@@ -167,6 +170,19 @@ int miqp_b200_batch_upload(MiqpB200Solver *s, const MiqpB200Problem *problems, i
 int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *problems, int count);
 int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms);
 int miqp_b200_batch_fetch(MiqpB200Solver *s, double *const *x_out, MiqpB200SolveInfo *infos);
+
+/* Streaming run: the same search as batch_run (after batch_upload or batch_upload_replan; batch_fetch, batch_fetch_compact,
+ * fetch_vector, pool_sizes and pool_fetch return the same afterwards), but every plan is handed to `on_done` as soon as its
+ * search ends instead of when the batch ends.  The device harvests a plan in the round in which it is marked finished (its
+ * result is final then); the callback runs on the calling thread, between rounds, at most one round later, in ascending k
+ * within a round.  Plans still searching when the batch stops (time limit, max_rounds), and plans whose own time limit was over
+ * before the first round, are delivered at the end.  Every plan is delivered exactly once.
+ * `traj` ([C][N][8], the compact layout of batch_fetch_compact) and `info` are valid during the call only.  `info` equals what
+ * batch_fetch_compact returns for plan k after the run, except `rounds`: the rounds the batch had run when the plan finished
+ * (the batch's rounds for the plans delivered at the end).  The callback must not call into this solver.
+ * ERR_ARG: on_done == NULL or no upload. */
+typedef void (*MiqpB200PlanDone)(void *user, int k, const double *traj, const MiqpB200SolveInfo *info);
+int miqp_b200_batch_run_streaming(MiqpB200Solver *s, MiqpB200PlanDone on_done, void *user, float *device_ms);
 
 /* Compact results: per plan the trajectory of every car, [C][N][8] doubles (pos_x, vel_x, acc_x, pos_y, vel_y, acc_y, u_x, u_y per
  * step: what MiqpPlanner::GetTrajectory reads, src/miqp_planner.cpp:1117-1192) instead of the full OPL column vector (config 2:

@@ -9,6 +9,8 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import queue
+import threading
 from dataclasses import dataclass
 
 import numpy as np
@@ -27,6 +29,7 @@ DECLARED_SYMBOLS = [
     "miqp_b200_frontier_tighten", "miqp_b200_frontier_finish", "miqp_b200_frontier_fingerprint", "miqp_b200_frontier_ub_device", "miqp_b200_batch_upload_replan", "miqp_b200_mark", "miqp_b200_elapsed", "miqp_b200_batch_fetch_compact", "miqp_b200_fetch_vector",
     "miqp_b200_solve_batch_compact",
     "miqp_b200_set_solution_pool", "miqp_b200_pool_sizes", "miqp_b200_pool_fetch",
+    "miqp_b200_batch_run_streaming",
 ]
 
 
@@ -81,6 +84,10 @@ class COptions(C.Structure):
 class CPoolEntry(C.Structure):
     _fields_ = [("objective", C.c_double), ("max_violation", C.c_double), ("search_value", C.c_double),
                 ("converged", C.c_int), ("round", C.c_int), ("uid", C.c_ulonglong)]
+
+
+# void (*MiqpB200PlanDone)(void *user, int k, const double *traj, const MiqpB200SolveInfo *info)
+PLAN_DONE = C.CFUNCTYPE(None, C.c_void_p, C.c_int, _dp, C.POINTER(CSolveInfo))
 
 
 class CRunStats(C.Structure):
@@ -159,6 +166,7 @@ def load_library():
     lib.miqp_b200_set_solution_pool.argtypes = [C.c_void_p, C.c_int]
     lib.miqp_b200_pool_sizes.argtypes = [C.c_void_p, _ip]
     lib.miqp_b200_pool_fetch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CPoolEntry), _dp, _dp, _ip]
+    lib.miqp_b200_batch_run_streaming.argtypes = [C.c_void_p, PLAN_DONE, C.c_void_p, C.POINTER(C.c_float)]
     _lib = lib
     return lib
 
@@ -435,8 +443,18 @@ class Solver:
                           None if x is None else x[j].copy(), None if tr is None else tr[j].copy())
                 for j, e in enumerate(ents[:got.value])]
 
-    def solve_prepared_compact(self, b):
-        """One miqp_b200_solve_batch_compact call on host buffers: pack + H2D + device solve + D2H of trajectories and infos."""
+    def solve_prepared_compact(self, b, on_plan=None):
+        """One miqp_b200_solve_batch_compact call on host buffers: pack + H2D + device solve + D2H of trajectories and infos.
+        on_plan(k, traj, info): a streaming run (run_streaming) instead, with the same results."""
+        if on_plan is not None:
+            self.upload_prepared(b)
+            self.run_streaming(on_plan)
+            if "traj" not in b:
+                b["traj"] = [np.zeros((p.C, p.N, 8)) for p in b["problems"]]
+                b["tptr"] = (_dp * b["n"])(*[t.ctypes.data_as(_dp) for t in b["traj"]])
+            self._lib.miqp_b200_batch_fetch_compact.argtypes = [C.c_void_p, C.POINTER(_dp), C.POINTER(CSolveInfo)]
+            self._check(self._lib.miqp_b200_batch_fetch_compact(self._h, b["tptr"], b["infos"]), "miqp_b200_batch_fetch_compact")
+            return b["traj"], b["infos"]
         if "traj" not in b:
             b["traj"] = [np.zeros((p.C, p.N, 8)) for p in b["problems"]]
             b["tptr"] = (_dp * b["n"])(*[t.ctypes.data_as(_dp) for t in b["traj"]])
@@ -467,6 +485,42 @@ class Solver:
         ms = C.c_float()
         self._check(self._lib.miqp_b200_batch_run(self._h, C.byref(ms)), "miqp_b200_batch_run")
         return ms.value
+
+    def run_streaming(self, on_plan) -> float:
+        """miqp_b200_batch_run_streaming: the same run as run(), with on_plan(k, traj, info) called for every plan as soon as its
+        search ends (on this thread, between rounds, ascending k within a round; traj is a copy [C][N][8], info a SolveInfo whose
+        `rounds` is the rounds run when the plan finished).  fetch() and the other results afterwards are those of run().  An
+        exception raised by on_plan stops the calls to it; the run finishes and the exception is raised here.  Returns the
+        device time in ms."""
+        shapes = getattr(self, "_shapes", None)   # (None before an upload: the C call refuses the run)
+        failed = []
+
+        def cb(_user, k, traj, info):
+            if failed:
+                return
+            try:
+                c, nn = shapes[k]
+                t = np.ctypeslib.as_array(traj, shape=(c * nn * 8,)).reshape(c, nn, 8).copy()
+                on_plan(k, t, self._info(info.contents))
+            except BaseException as ex:   # ctypes would print and drop it
+                failed.append(ex)
+
+        return self._run_streaming_raw(PLAN_DONE(cb), failed)
+
+    def _run_streaming_raw(self, cfunc, failed):
+        ms = C.c_float()
+        rc = self._lib.miqp_b200_batch_run_streaming(self._h, cfunc, None, C.byref(ms))
+        if failed:
+            raise failed[0]
+        self._check(rc, "miqp_b200_batch_run_streaming")
+        return ms.value
+
+    def solve_batch_streaming(self, problems, gap_tol=None, time_limit=None, warm=None):
+        """Generator of (k, traj, info) in the order the plans finish: upload + run_streaming on a worker thread (the C call
+        releases the GIL), results through a queue.  Closing the generator early waits for the run to end, so no thread is left
+        behind; the solver is busy until the generator is exhausted or closed.  fetch() etc. afterwards give the whole batch."""
+        self.upload(problems, gap_tol, time_limit, warm)
+        return _stream_results(lambda on_plan: self.run_streaming(on_plan))
 
     def fetch(self):
         n, ncols = self._batch
@@ -610,19 +664,27 @@ class PipelinedSolver:
         Two batches that are in flight together must not share their prepared buffers.  Returns [(xs, infos), ...]."""
         return self._run_threads(list(prepared_batches), lambda s, b: s.solve_prepared(b), stagger_s)
 
-    def solve_stream_compact(self, prepared_batches, stagger_s: float = 0.0):
-        """solve_stream with compact results (trajectories + infos; the full vectors stay on the device)"""
-        return self._run_threads(list(prepared_batches), lambda s, b: s.solve_prepared_compact(b), stagger_s)
+    def solve_stream_compact(self, prepared_batches, stagger_s: float = 0.0, on_plan=None):
+        """solve_stream with compact results (trajectories + infos; the full vectors stay on the device).  on_plan(batch_index,
+        k, traj, info): every plan as soon as its search ends (Solver.run_streaming), called from the instance's worker thread."""
+        jobs = list(enumerate(prepared_batches))
+        if on_plan is None:
+            return self._run_threads(jobs, lambda s, j: s.solve_prepared_compact(j[1]), stagger_s)
+        return self._run_threads(jobs, lambda s, j: s.solve_prepared_compact(
+            j[1], on_plan=lambda k, t, i, bi=j[0]: on_plan(bi, k, t, i)), stagger_s)
 
     def upload_resident(self, prepared_batches):
         """one resident batch per instance (miqp_b200_batch_upload)"""
         for s, b in zip(self.solvers, prepared_batches):
             s.upload_prepared(b)
 
-    def run_resident(self, runs: int, stagger_s: float = 0.0):
+    def run_resident(self, runs: int, stagger_s: float = 0.0, on_plan=None):
         """`runs` searches over the resident batches (miqp_b200_batch_run), run k on instance k mod depth; returns the
-        device time of every run (CUDA events on its own stream; the runs overlap, so their sum exceeds the wall time)."""
-        return self._run_threads(list(range(runs)), lambda s, k: s.run(), stagger_s)
+        device time of every run (CUDA events on its own stream; the runs overlap, so their sum exceeds the wall time).
+        on_plan(run_index, k, traj, info): streaming runs (Solver.run_streaming), called from the instance's worker thread."""
+        if on_plan is None:
+            return self._run_threads(list(range(runs)), lambda s, k: s.run(), stagger_s)
+        return self._run_threads(list(range(runs)), lambda s, r: s.run_streaming(lambda k, t, i: on_plan(r, k, t, i)), stagger_s)
 
     def timed_resident(self, runs: int, stagger_s: float = 0.0):
         """run_resident, timed on the device: CUDA events on the solvers' own streams, from the start of the first run to the
@@ -632,3 +694,38 @@ class PipelinedSolver:
         for s in self.solvers:
             s.mark(1)
         return max(self.solvers[0].elapsed_to(s) for s in self.solvers), per_run
+
+
+_DONE = object()
+
+
+def _stream_results(run):
+    """Generator over the plans a streaming run delivers: run(on_plan) executes on a worker thread and feeds a queue; the
+    run's exception, if any, is raised after the plans delivered before it.  Closing the generator joins the thread."""
+    q = queue.Queue()
+    stop = threading.Event()
+
+    def on_plan(k, traj, info):
+        if not stop.is_set():
+            q.put((k, traj, info))
+
+    def work():
+        try:
+            run(on_plan)
+            q.put(_DONE)
+        except BaseException as ex:
+            q.put(ex)
+
+    th = threading.Thread(target=work, name="miqp_b200-streaming", daemon=True)
+    th.start()
+    try:
+        while True:
+            item = q.get()
+            if item is _DONE:
+                return
+            if isinstance(item, BaseException):
+                raise item
+            yield item
+    finally:
+        stop.set()
+        th.join()

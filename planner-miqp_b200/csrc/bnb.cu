@@ -971,16 +971,14 @@ __device__ __noinline__ void expand_solution(const DevProb &p, const double *D, 
   }
 }
 
-__global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob,
-                                  double *xall, double *best_bound) {
-  const int s = blockIdx.x;
+// Result of one finished (or stopped) plan s: best bound = smallest bound still open or pruned by the gap rule, into best_bound[s];
+// the incumbent's full column vector into xall (zeros without an incumbent) and its exact trajectory in inc_z.  One block of at
+// most 128 threads per plan; red: shared [128], jeff_s: shared [8 * 64].  bnb_finish_kernel (end of a run) and
+// bnb_harvest_finish_kernel (plans of a streaming run, in the round select marks them finished) run the same code.
+__device__ __forceinline__ void finish_plan(const BnbState &st, int s, const DevProb &p, const double *D, const int *I,
+                                            double *xall, double *best_bound, double *red, int *jeff_s) {
   const int tid = threadIdx.x, nt = blockDim.x;
-  const DevProb &p = probs[s];
-  const double *D = dblob; const int *I = iblob;
   const long pb = (long)s * st.cap;
-  __shared__ double red[128];
-  __shared__ int jeff_s[8 * 64];
-  // best bound: smallest bound still open or pruned by the gap rule
   double lb = MQ_INF;
   const int nopen = st.open_cnt[s];
   for (int k = tid; k < nopen; k += nt) lb = fmin(lb, st.bound[pb + st.open_idx[pb + k]]);
@@ -1000,6 +998,16 @@ __global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const doubl
   __syncthreads();
   if (!(ub < MQ_INF) || st.inc_uid[s] == ~0ULL) return;   // no incumbent of its own (ub may come from another rank: frontier sharding)
   expand_solution(p, D, I, st.inc_dec + (long)s * st.ndec_stride, st.inc_z + (long)s * st.zstride, x, jeff_s);
+}
+
+__global__ void bnb_finish_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob,
+                                  double *xall, double *best_bound) {
+  const int s = blockIdx.x;
+  __shared__ double red[128];
+  __shared__ int jeff_s[8 * 64];
+  // streaming run: a plan harvested in an earlier round has its result in place (expand_solution rewrites inc_z: not twice)
+  if (st.delivered && st.delivered[s]) return;
+  finish_plan(st, s, probs[s], dblob, iblob, xall, best_bound, red, jeff_s);
 }
 
 void launch_bnb_finish(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob,
@@ -1028,6 +1036,72 @@ __global__ void pool_expand_kernel(BnbState st, int k, const int *idx, const Dev
 void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const DevProb *eprobs, const double *dblob, const int *iblob,
                         double *zs, double *xall, cudaStream_t s) {
   if (n > 0) pool_expand_kernel<<<n, 128, 0, s>>>(st, k, idx, eprobs, dblob, iblob, zs, xall);
+}
+
+// ---------------------------------------------------------------------------------------
+// streaming runs: harvest of the plans that bnb_select_kernel marked finished, in the same round.  Once select has set done[s],
+// nothing of the search writes plan s again, so its result is final.  The host launches the kernels after select and before the
+// node kernels, sizing the grids by the plans still active in the previous round (an upper bound of the plans select can finish
+// now), at most HARVEST_GRID blocks that stride over the harvested plans: a round that finishes few plans launches few blocks.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(SEL_THREADS) bnb_harvest_kernel(BnbState st, int all, int *list, int *n, double *max_viol) {
+  __shared__ int warp_tot[SEL_THREADS / 32];
+  int base_out = 0;
+  for (int base = 0; base < st.count; base += SEL_THREADS) {
+    const int s = base + threadIdx.x;
+    const int take = (s < st.count && !st.delivered[s] && (all || st.done[s] != 0)) ? 1 : 0;
+    int total; const int rank = block_excl_scan(take, warp_tot, total);   // ascending plan order, no atomics: deterministic
+    if (take) { list[base_out + rank] = s; st.delivered[s] = 1; max_viol[s] = 0.0; }   // (evaluate_list_kernel takes the maximum into it)
+    base_out += total;
+  }
+  if (threadIdx.x == 0) *n = base_out;
+}
+
+__global__ void bnb_harvest_finish_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                                          const int *n, double *xall, double *best_bound) {
+  __shared__ double red[128];
+  __shared__ int jeff_s[8 * 64];
+  const int nh = *n;
+  for (int e = blockIdx.x; e < nh; e += gridDim.x) {
+    const int s = list[e];
+    finish_plan(st, s, probs[s], dblob, iblob, xall, best_bound, red, jeff_s);
+    __syncthreads();   // red / jeff_s are reused by the next plan
+  }
+}
+
+__global__ void bnb_harvest_pack_kernel(BnbState st, const DevProb *probs, const int *list, const int *n, const double *obj,
+                                        const double *viol, const double *best_bound, double *out, long rec_stride) {
+  const int nh = *n;
+  for (int e = blockIdx.x; e < nh; e += gridDim.x) {
+    const int s = list[e];
+    const DevProb &p = probs[s];
+    double *rec = out + (long)e * rec_stride;
+    if (threadIdx.x == 0) {
+      StreamRec r;
+      r.objective = obj[s]; r.max_violation = viol[s]; r.best_bound = best_bound[s]; r.ub = st.ub[s];
+      r.inc_uid = st.inc_uid[s];
+      r.nodes = st.stat_nodes[s]; r.iters = st.stat_iters[s]; r.rows = st.stat_rows[s]; r.uncert = st.stat_uncert[s];
+      r.k = s; r.done = st.done[s]; r.done_round = st.done_round[s]; r.overflow = st.overflow[s];
+      *reinterpret_cast<StreamRec *>(rec) = r;
+    }
+    const double *z = st.inc_z + (long)s * st.zstride;
+    const int nz = p.C * p.N * 8;
+    for (int q = threadIdx.x; q < nz; q += blockDim.x) rec[STREAM_REC_HDR + q] = z[q];
+  }
+}
+
+void launch_bnb_harvest(const BnbState &st, int all, int *list, int *n, double *max_viol, cudaStream_t s) {
+  bnb_harvest_kernel<<<1, SEL_THREADS, 0, s>>>(st, all, list, n, max_viol);
+}
+
+void launch_bnb_harvest_finish(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                               const int *n, int max_n, double *xall, double *best_bound, cudaStream_t s) {
+  if (max_n > 0) bnb_harvest_finish_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, dblob, iblob, list, n, xall, best_bound);
+}
+
+void launch_bnb_harvest_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
+                             const double *viol, const double *best_bound, double *out, long rec_stride, cudaStream_t s) {
+  if (max_n > 0) bnb_harvest_pack_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, list, n, obj, viol, best_bound, out, rec_stride);
 }
 
 }  // namespace miqp

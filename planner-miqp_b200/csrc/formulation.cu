@@ -418,11 +418,11 @@ __device__ __forceinline__ void atomic_max_double(double *addr, double v) {
   atomicMax(reinterpret_cast<unsigned long long *>(addr), (unsigned long long)__double_as_longlong(v));
 }
 
-// max violation of rows, column bounds and integrality; objective (objective_function.mod:7-19)
-__global__ void evaluate_kernel(const DevProb *probs, const double *dblob, const int *iblob, int count,
-                                const double *xall, double *max_viol /* [count], zeroed */, double *objective /* [count] */) {
-  const int s = blockIdx.y;
-  if (s >= count) return;
+// max violation of rows, column bounds and integrality; objective (objective_function.mod:7-19) of plan s: blocks (x, *) of the
+// grid share its rows and columns.  evaluate_kernel (every plan) and evaluate_list_kernel (the plans of a list) run the same code,
+// so both give the same bits.
+__device__ __forceinline__ void evaluate_plan(const DevProb *probs, const double *dblob, const int *iblob, int s,
+                                              const double *xall, double *max_viol, double *objective) {
   const DevProb &p = probs[s];
   const double *x = xall + p.x_base;
   const long nrows = p.fam_row[NUM_FAM];
@@ -479,6 +479,20 @@ __global__ void evaluate_kernel(const DevProb *probs, const double *dblob, const
   }
 }
 
+__global__ void evaluate_kernel(const DevProb *probs, const double *dblob, const int *iblob, int count,
+                                const double *xall, double *max_viol /* [count], zeroed */, double *objective /* [count] */) {
+  const int s = blockIdx.y;
+  if (s >= count) return;
+  evaluate_plan(probs, dblob, iblob, s, xall, max_viol, objective);
+}
+
+// the plans list[0 .. *n) (streaming runs: the plans harvested in this round; *n is only known on the device)
+__global__ void evaluate_list_kernel(const DevProb *probs, const double *dblob, const int *iblob, const int *list, const int *n,
+                                     const double *xall, double *max_viol, double *objective) {
+  const int nh = *n;
+  for (int e = blockIdx.y; e < nh; e += gridDim.y) evaluate_plan(probs, dblob, iblob, list[e], xall, max_viol, objective);
+}
+
 // ------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------
@@ -505,6 +519,16 @@ void launch_evaluate(const DevProb *probs, const double *dblob, const int *iblob
   if (bx > 64) bx = 64;
   dim3 grid(bx, count);
   evaluate_kernel<<<grid, 256, 0, st>>>(probs, dblob, iblob, count, xall, max_viol, objective);
+}
+
+void launch_evaluate_list(const DevProb *probs, const double *dblob, const int *iblob, const int *list, const int *n, int max_n,
+                          long max_rows, const double *xall, double *max_viol, double *objective, cudaStream_t st) {
+  if (max_n <= 0) return;
+  int bx = (int)((max_rows + 255) / 256);
+  if (bx < 1) bx = 1;
+  if (bx > 64) bx = 64;
+  dim3 grid(bx, max_n < HARVEST_GRID / 4 ? max_n : HARVEST_GRID / 4);   // (blocks stride over the plans of the list)
+  evaluate_list_kernel<<<grid, 256, 0, st>>>(probs, dblob, iblob, list, n, xall, max_viol, objective);
 }
 
 }  // namespace miqp

@@ -11,6 +11,10 @@ void launch_assemble_rows(const DevProb *probs, const double *dblob, const int *
                           unsigned long long *nnz_count, cudaStream_t st);
 void launch_evaluate(const DevProb *probs, const double *dblob, const int *iblob, int count, long max_rows,
                      const double *xall, double *max_viol, double *objective, cudaStream_t st);
+// the same for the plans list[0 .. *n) only; *n is read on the device, max_n (>= *n) sizes the grid.  max_viol[list[e]] must be
+// zeroed before (bnb_harvest_kernel does it)
+void launch_evaluate_list(const DevProb *probs, const double *dblob, const int *iblob, const int *list, const int *n, int max_n,
+                          long max_rows, const double *xall, double *max_viol, double *objective, cudaStream_t st);
 
 // ---- bnb.cu ---------------------------------------------------------------------------
 // entry of the solution pool (BnbState::pool_rec)
@@ -81,6 +85,8 @@ struct BnbState {
   unsigned char *pool_dec;  // [count][pool_cap][ndec_stride]
   PoolRec *pool_rec;        // [count][pool_cap]
   int *pool_cnt;            // [count]
+  // streaming runs (miqp_b200_batch_run_streaming): 1 once a finished plan's result has been harvested; null otherwise
+  int *delivered;           // [count]
 };
 
 // one plan's share of the solution pool, handed to the out-of-line insertion (kernel parameters stay in parameter space)
@@ -114,6 +120,25 @@ void launch_bnb_finish(const BnbState &st, const DevProb *probs, const double *d
 // into xall; the entry's trajectory goes to zs[e * zstride] (pool storage is not modified)
 void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const DevProb *eprobs, const double *dblob, const int *iblob,
                         double *zs, double *xall, cudaStream_t s);
+// ---- streaming runs: per-round harvest of the plans that select marked finished -------------------------------------------
+// one record per harvested plan, then its trajectory [C][N][8] (inc_z after expand_solution); records are rec_stride doubles apart
+struct StreamRec {
+  double objective, max_violation, best_bound, ub;                     // evaluate_kernel's values, bnb_finish's best bound, incumbent
+  unsigned long long inc_uid, nodes, iters, rows, uncert;              // incumbent uid and the four stats counters
+  int k, done, done_round, overflow;                                   // plan index and its search state
+};
+constexpr int STREAM_REC_HDR = 12;   // doubles before the trajectory
+constexpr int HARVEST_GRID = 1024;   // most blocks of a harvest kernel (they stride over the harvested plans)
+static_assert(sizeof(StreamRec) <= STREAM_REC_HDR * sizeof(double), "StreamRec outgrew its header");
+// plans to harvest in ascending order into list[0 .. *n): finished (done != 0) and not yet delivered -- or, with all = 1, every
+// plan not yet delivered (end of the run); marks them delivered and zeroes their max_viol for launch_evaluate_list
+void launch_bnb_harvest(const BnbState &st, int all, int *list, int *n, double *max_viol, cudaStream_t s);
+// finishing of the harvested plans (best bound, full column vector into xall, exact trajectory in inc_z)
+void launch_bnb_harvest_finish(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                               const int *n, int max_n, double *xall, double *best_bound, cudaStream_t s);
+// records of the harvested plans into out[e * rec_stride]
+void launch_bnb_harvest_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
+                             const double *viol, const double *best_bound, double *out, long rec_stride, cudaStream_t s);
 int node_kernel_smem_per_warp(int maxN, int kmax, int ndec_stride);
 int node_kernel_narrow_np(int N);                                  // row stride of the (s, lambda) records of a two-warp team
 int node_kernel_smem_narrow(int N, int kmax, int ndec_stride);   // shared memory of a two-warp team (uniform horizon N)

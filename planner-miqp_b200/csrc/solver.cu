@@ -120,6 +120,16 @@ struct MiqpB200Solver {
   int solution_pool = 0;
   DevBuf<double> sp_z; DevBuf<unsigned char> sp_dec; DevBuf<PoolRec> sp_rec; DevBuf<int> sp_cnt;
   DevBuf<DevProb> sp_probs; DevBuf<int> sp_idx; DevBuf<double> sp_x, sp_zs, sp_obj, sp_viol;
+  // streaming runs (miqp_b200_batch_run_streaming): callback (null outside such a run), delivered flags, harvest list, records
+  // (device staging and page-locked host copy), records copied but not yet delivered, records held for the end of the run
+  MiqpB200PlanDone on_done = nullptr; void *on_done_user = nullptr;
+  DevBuf<int> hv_delivered, hv_list; DevBuf<double> hv_rec;
+  DVec h_hvrec;
+  std::vector<double> hv_held;
+  cudaEvent_t ev_hv = nullptr;
+  long hv_stride = 0;
+  int hv_pending = 0, hv_bound = 0, hv_total = 0;
+  bool hv_defer = false;
 };
 
 namespace {
@@ -209,6 +219,100 @@ void pack_batch(MiqpB200Solver *s, const MiqpB200Problem *problems, int count) {
   }
 }
 
+// Solve info of plan k from its device results: batch_fetch and the deliveries of a streaming run build it alike.
+void plan_info(const MiqpB200Solver *s, int k, double ub, unsigned long long incuid, double bb, double obj, double viol, int done,
+               int done_round, int overflow, unsigned long long nodes, unsigned long long iters, unsigned long long uncert,
+               MiqpB200SolveInfo &in) {
+  const DevProb &p = s->pk.probs[k];
+  std::memset(&in, 0, sizeof in);
+  // (a finite bound without an incumbent of its own: the objective came from another rank, frontier sharding)
+  const bool have = std::isfinite(ub) && incuid != ~0ULL;
+  // solve time of THIS plan: the host's clock at the end of the round after which it was finished (the batch's time for a
+  // plan that was still searching when the batch stopped)
+  const int dr = done_round;
+  in.seconds = (done && dr >= 1 && (size_t)(dr - 1) < s->round_elapsed.size() && s->round_elapsed[dr - 1] > 0.0) ? s->round_elapsed[dr - 1] : s->last_seconds;
+  in.nodes = (long)nodes; in.qp_iters = (long)iters; in.rounds = s->stats.rounds;
+  in.best_bound = bb;
+  in.uncertified = (long)uncert;
+  in.pool_exhausted = overflow;
+  if (have) {
+    // every open or pruned node may lie above the incumbent: report min(bound, incumbent) like CPLEX's best bound
+    if (in.best_bound > ub) in.best_bound = ub;
+    in.status = MIQP_B200_SUCCESS;
+    in.objective = obj;  // re-evaluated on the full vector by evaluate_kernel
+    in.max_violation = viol;
+    const double lb = std::min(bb, ub);
+    in.gap = std::fabs(lb - ub) / (1e-10 + std::fabs(ub));
+    in.proven = (in.gap <= p.gap_tol + 1e-15) ? 1 : 0;
+  } else {
+    // no incumbent: the reference reports FAILED_TIMEOUT only for the time-limit status
+    in.status = ((s->timed_out && !done) || done == 2) ? MIQP_B200_FAILED_TIMEOUT : MIQP_B200_FAILED_NO_SOLUT;
+    in.objective = NAN; in.gap = NAN; in.max_violation = NAN;
+  }
+}
+
+// ---- streaming runs -------------------------------------------------------------------------------------------------------
+// Harvest of a round (after select): the plans select has just marked finished are finished like bnb_finish does it, evaluated
+// and packed into records; their number lands in ctrl[7], which the host reads with the round's ctrl copy.  all = 1 (end of the
+// run, after bnb_finish, which skips the delivered plans): every plan not delivered yet is evaluated and packed.
+void launch_harvest(MiqpB200Solver *s, int all, int max_n) {
+  int *list = s->hv_list.p, *n = s->b_ctrl.p + 7;
+  launch_bnb_harvest(s->st, all, list, n, s->d_viol.p, s->stream);
+  if (!all)
+    launch_bnb_harvest_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, s->d_x.p, s->d_bb.p, s->stream);
+  launch_evaluate_list(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
+  launch_bnb_harvest_pack(s->st, s->d_probs.p, list, n, max_n, s->d_obj.p, s->d_viol.p, s->d_bb.p, s->hv_rec.p, s->hv_stride, s->stream);
+}
+
+// copy of n records to the host (stream-ordered before the next harvest overwrites the staging area)
+void copy_records(MiqpB200Solver *s, int n) {
+  CK(cudaMemcpyAsync(s->h_hvrec.data(), s->hv_rec.p, sizeof(double) * (size_t)n * s->hv_stride, cudaMemcpyDeviceToHost, s->stream));
+  CK(cudaEventRecord(s->ev_hv, s->stream));
+  s->hv_pending = n;
+  s->hv_total += n;
+}
+
+void deliver_record(MiqpB200Solver *s, const double *rec, long rounds) {
+  StreamRec r;
+  std::memcpy(&r, rec, sizeof r);
+  MiqpB200SolveInfo in;
+  plan_info(s, r.k, r.ub, r.inc_uid, r.best_bound, r.objective, r.max_violation, r.done, r.done_round, r.overflow, r.nodes, r.iters,
+            r.uncert, in);
+  in.rounds = rounds;
+  s->on_done(s->on_done_user, r.k, rec + STREAM_REC_HDR, &in);
+}
+
+// Callbacks of the copied records, in ascending plan order.  A plan that finished before the first round (its time limit was over
+// when the run started) reports the batch's time as its solve time, known only at the end: it is held and delivered then.
+void deliver_pending(MiqpB200Solver *s) {
+  if (s->hv_pending == 0) return;
+  CK(cudaEventSynchronize(s->ev_hv));
+  for (int e = 0; e < s->hv_pending; ++e) {
+    const double *rec = s->h_hvrec.data() + (size_t)e * s->hv_stride;
+    StreamRec r;
+    std::memcpy(&r, rec, sizeof r);
+    if (r.done_round >= 1) deliver_record(s, rec, r.done_round);
+    else s->hv_held.insert(s->hv_held.end(), rec, rec + s->hv_stride);
+  }
+  s->hv_pending = 0;
+}
+
+// end of the run: the held plans and the plans stopped with the batch, merged in ascending plan order
+void deliver_final(MiqpB200Solver *s) {
+  CK(cudaEventSynchronize(s->ev_hv));
+  std::vector<const double *> recs;
+  for (size_t o = 0; o < s->hv_held.size(); o += (size_t)s->hv_stride) recs.push_back(s->hv_held.data() + o);
+  for (int e = 0; e < s->hv_pending; ++e) recs.push_back(s->h_hvrec.data() + (size_t)e * s->hv_stride);
+  std::sort(recs.begin(), recs.end(), [](const double *a, const double *b) {
+    StreamRec ra, rb;
+    std::memcpy(&ra, a, sizeof ra); std::memcpy(&rb, b, sizeof rb);
+    return ra.k < rb.k;
+  });
+  s->hv_pending = 0;
+  for (const double *rec : recs) deliver_record(s, rec, s->stats.rounds);
+  s->hv_held.clear();
+}
+
 // Select / solve rounds of the uploaded batch, starting from the current device state: until every plan is finished, the time
 // limit or round cap is hit, or `max_rounds_now` rounds have run (< 0: no such cap).  Returns the number of unfinished plans.
 int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launches, long &node_launches, double &node_ms) {
@@ -221,6 +325,7 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launch
     if ((size_t)rounds >= s->round_elapsed.size()) s->round_elapsed.resize(rounds + 64, 0.0);
     launch_bnb_select(s->st, s->d_probs.p, (int)rounds + 1, el0, s->stream);
     launches += 2;
+    if (s->on_done) { launch_harvest(s, 0, rounds == 0 ? s->st.count : s->hv_bound); launches += 4; }
     CK(cudaEventRecord(s->evr0, s->stream));
     if (s->n_single > 0) {
       // fewer single-car nodes than wide teams fit (work count of the last round as the estimate): latency matters, not throughput;
@@ -244,10 +349,16 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launch
       ++launches; ++node_launches;
     }
     CK(cudaEventRecord(s->evr1, s->stream));
+    if (s->on_done && !s->hv_defer) deliver_pending(s);   // the last round's plans, while this round's node kernels run
     ++s->fr_rounds; ++done_now;
     CK(cudaMemcpyAsync(ctrl, s->b_ctrl.p, sizeof ctrl, cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     s->fr_ctrl0 = ctrl[0];
+    if (s->on_done) {
+      deliver_pending(s);   // (deferred delivery: the last round's plans)
+      s->hv_bound = ctrl[2];   // only plans active in this round can finish in the next select
+      if (ctrl[7] > 0) copy_records(s, ctrl[7]);
+    }
     float ms = 0.f;
     CK(cudaEventElapsedTime(&ms, s->evr0, s->evr1));
     node_ms += ms;
@@ -496,6 +607,7 @@ void miqp_b200_destroy(MiqpB200Solver *s) {
   if (s->mark[0]) cudaEventDestroy(s->mark[0]);
   if (s->mark[1]) cudaEventDestroy(s->mark[1]);
   if (s->evr1) cudaEventDestroy(s->evr1);
+  if (s->ev_hv) cudaEventDestroy(s->ev_hv);
   if (s->stream) cudaStreamDestroy(s->stream);
   delete s;
 }
@@ -709,9 +821,14 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
   return MIQP_B200_OK;
 }
 
-int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms) {
-  if (!s) return MIQP_B200_ERR_ARG;
-  if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "batch_run without batch_upload");
+// One search of the uploaded batch; a streaming run (s->on_done set) also harvests every plan in the round select marks it
+// finished and hands it to the callback.  Both compute the same results.
+static int run_batch(MiqpB200Solver *s, float *device_ms) {
+  const bool streaming = s->on_done != nullptr;
+  struct Reset {   // the delivered flags are seen by the kernels of streaming runs only
+    MiqpB200Solver *s;
+    ~Reset() { s->st.delivered = nullptr; s->on_done = nullptr; s->on_done_user = nullptr; s->hv_pending = 0; s->hv_held.clear(); }
+  } reset{s};
   try {
     CK(cudaSetDevice(s->opt.device));
     const int count = s->st.count;
@@ -722,6 +839,17 @@ int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms) {
     double node_ms = 0.0;
     CK(cudaMemsetAsync(s->b_prof.p, 0, 256 * sizeof(unsigned long long), s->stream));
     if (s->st.susp_slot) CK(cudaMemsetAsync(s->st.susp_slot, 0xff, sizeof(int) * (size_t)s->st.count * s->st.cap, s->stream));
+    if (streaming) {
+      s->hv_stride = (STREAM_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
+      s->hv_delivered.ensure(count); s->hv_list.ensure(count); s->hv_rec.ensure((size_t)count * s->hv_stride);
+      s->h_hvrec.resize((size_t)count * s->hv_stride);
+      if (!s->ev_hv) CK(cudaEventCreateWithFlags(&s->ev_hv, cudaEventDisableTiming));
+      CK(cudaMemsetAsync(s->hv_delivered.p, 0, sizeof(int) * count, s->stream));
+      s->st.delivered = s->hv_delivered.p;
+      s->hv_pending = 0; s->hv_total = 0; s->hv_held.clear();
+      const char *e = std::getenv("MIQP_STREAM_DEFER");   // 1: deliver a round's plans after the next round's sync (A/B of the delivery point)
+      s->hv_defer = e && e[0] == '1';
+    }
     CK(cudaEventRecord(s->ev0, s->stream));
     launch_bnb_init(s->st, s->d_probs.p, s->any_warm ? s->d_warm.p : nullptr, s->any_warm ? s->d_haswarm.p : nullptr, s->stream);
     ++launches;
@@ -729,9 +857,17 @@ int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms) {
     s->fr_rounds = 0; s->fr_ctrl0 = 0; s->fr_t0 = t0;
     run_rounds(s, -1, tlim, launches, node_launches, node_ms);
     rounds = s->fr_rounds;
+    if (streaming) deliver_pending(s);   // the plans select finished in the last round
     launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
-    CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
-    launch_evaluate(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, count, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
+    if (!streaming) {
+      CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
+      launch_evaluate(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, count, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
+    } else {   // the plans that were still searching when the batch stopped: exactly the ones not delivered yet (same evaluate code)
+      const int left = count - s->hv_total;
+      launch_harvest(s, 1, left);
+      launches += 2;
+      if (left > 0) copy_records(s, left);
+    }
     launches += 2;
     CK(cudaGetLastError());
     CK(cudaEventRecord(s->ev1, s->stream));
@@ -743,10 +879,25 @@ int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms) {
     s->stats.launches = launches; s->stats.node_kernel_launches = node_launches; s->stats.rounds = rounds;
     s->stats.node_kernel_ms = node_ms; s->stats.total_ms = total_ms;
     s->ran = true;
+    if (streaming) deliver_final(s);
   } catch (const std::exception &ex) {
     return fail(s, MIQP_B200_ERR_CUDA, ex.what());
   }
   return MIQP_B200_OK;
+}
+
+int miqp_b200_batch_run(MiqpB200Solver *s, float *device_ms) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "batch_run without batch_upload");
+  return run_batch(s, device_ms);
+}
+
+int miqp_b200_batch_run_streaming(MiqpB200Solver *s, MiqpB200PlanDone on_done, void *user, float *device_ms) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (!on_done) return fail(s, MIQP_B200_ERR_ARG, "batch_run_streaming without a callback");
+  if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "batch_run_streaming without batch_upload");
+  s->on_done = on_done; s->on_done_user = user;
+  return run_batch(s, device_ms);
 }
 
 static int fetch_results(MiqpB200Solver *s, double *const *x_out, double *const *traj_out, MiqpB200SolveInfo *infos);
@@ -814,35 +965,10 @@ static int fetch_results(MiqpB200Solver *s, double *const *x_out, double *const 
       }
     }
     for (int k = 0; k < count; ++k) {
-      const DevProb &p = s->pk.probs[k];
       nodes += (long)s->h_stats[k]; iters += (long)s->h_stats[count + k]; rows += (long)s->h_stats[2 * count + k];
       if (!infos) continue;
-      MiqpB200SolveInfo &in = infos[k];
-      std::memset(&in, 0, sizeof in);
-      // (a finite bound without an incumbent of its own: the objective came from another rank, frontier sharding)
-      const bool have = std::isfinite(s->h_ub[k]) && s->h_incuid[k] != ~0ULL;
-      // solve time of THIS plan: the host's clock at the end of the round after which it was finished (the batch's time for a
-      // plan that was still searching when the batch stopped)
-      const int dr = s->h_doneround[k];
-      in.seconds = (s->h_done[k] && dr >= 1 && (size_t)(dr - 1) < s->round_elapsed.size() && s->round_elapsed[dr - 1] > 0.0) ? s->round_elapsed[dr - 1] : s->last_seconds;
-      in.nodes = (long)s->h_stats[k]; in.qp_iters = (long)s->h_stats[count + k]; in.rounds = s->stats.rounds;
-      in.best_bound = s->h_bb[k];
-      in.uncertified = (long)s->h_stats[3 * (size_t)count + k];
-      in.pool_exhausted = s->h_overflow[k];
-      if (have) {
-        // every open or pruned node may lie above the incumbent: report min(bound, incumbent) like CPLEX's best bound
-        if (in.best_bound > s->h_ub[k]) in.best_bound = s->h_ub[k];
-        in.status = MIQP_B200_SUCCESS;
-        in.objective = s->h_obj[k];  // re-evaluated on the full vector by evaluate_kernel
-        in.max_violation = s->h_viol[k];
-        const double lb = std::min(s->h_bb[k], s->h_ub[k]);
-        in.gap = std::fabs(lb - s->h_ub[k]) / (1e-10 + std::fabs(s->h_ub[k]));
-        in.proven = (in.gap <= p.gap_tol + 1e-15) ? 1 : 0;
-      } else {
-        // no incumbent: the reference reports FAILED_TIMEOUT only for the time-limit status
-        in.status = ((s->timed_out && !s->h_done[k]) || s->h_done[k] == 2) ? MIQP_B200_FAILED_TIMEOUT : MIQP_B200_FAILED_NO_SOLUT;
-        in.objective = NAN; in.gap = NAN; in.max_violation = NAN;
-      }
+      plan_info(s, k, s->h_ub[k], s->h_incuid[k], s->h_bb[k], s->h_obj[k], s->h_viol[k], s->h_done[k], s->h_doneround[k], s->h_overflow[k],
+                s->h_stats[k], s->h_stats[count + k], s->h_stats[3 * (size_t)count + k], infos[k]);
     }
     s->stats.nodes = nodes; s->stats.qp_iters = iters; s->stats.rows_visited = rows;
     s->stats.fetch_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tf0).count();
