@@ -16,8 +16,6 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-ffp-contract=o
 # formulation.cu is compared bit for bit with the oracle: no FMA contraction there
 if os.environ.get("MIQP_PROF") == "1":      # per-phase cycle counters of the node kernel (miqp_b200_debug_profile)
     COMMON.append("-DMQ_PROF")
-if os.environ.get("MIQP_TEAMS_PER_SM"):
-    COMMON.append("-DMQ_TEAMS_PER_SM=" + os.environ["MIQP_TEAMS_PER_SM"])
 UNITS = [("formulation.cu", ["--fmad=false"]), ("bnb.cu", []), ("bnb_multi.cu", []), ("solver.cu", []), ("peaks.cu", [])]
 
 
@@ -79,30 +77,6 @@ def build_pymodule(force: bool = False) -> str:
     return out
 
 
-def build_variant(tag: str) -> str:
-    """libmiqp_b200_<tag>.so with the build-time switches of the environment (MIQP_TEAMS_PER_SM, MIQP_PROF): for A/B runs,
-    loaded with MIQP_B200_VARIANT=<tag>; the host libraries are not rebuilt."""
-    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    lib = os.path.join(HERE, f"libmiqp_b200_{tag}.so")
-    objs = []
-    for src, extra in UNITS:
-        obj = os.path.join(CSRC, src.replace(".cu", f".{tag}.o"))
-        r = subprocess.run([nvcc] + ARCH + COMMON + extra + ["-c", os.path.join(CSRC, src), "-o", obj], capture_output=True, text=True)
-        if r.returncode != 0:
-            sys.stderr.write(r.stdout + r.stderr)
-            raise RuntimeError(f"nvcc failed on {src}")
-        if src == "bnb.cu":
-            sys.stderr.write("\n".join(l for l in r.stderr.splitlines() if "registers" in l or "spill" in l) + "\n")
-        objs.append(obj)
-    r = subprocess.run([nvcc] + ARCH + ["-shared", "-o", lib] + objs + ["-lcudart", "-lpthread"], capture_output=True, text=True)
-    if r.returncode != 0:
-        sys.stderr.write(r.stdout + r.stderr)
-        raise RuntimeError("link failed")
-    for o in objs:
-        os.remove(o)
-    return lib
-
-
 def build(force: bool = False, verbose: bool = False) -> str:
     if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= _newest_src():
         build_host(force=False)
@@ -135,7 +109,4 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 
 if __name__ == "__main__":
-    if os.environ.get("MIQP_VARIANT"):
-        print(build_variant(os.environ["MIQP_VARIANT"]))
-        sys.exit(0)
     print(build(force="--force" in sys.argv, verbose=True))

@@ -128,9 +128,7 @@ class PoolEntry:
 
 
 def library_path() -> str:
-    # MIQP_B200_VARIANT=<tag>: a build variant made by `MIQP_VARIANT=<tag> python build.py` (A/B runs of build-time switches)
-    tag = os.environ.get("MIQP_B200_VARIANT")
-    return os.path.join(_HERE, f"libmiqp_b200_{tag}.so" if tag else "libmiqp_b200.so")
+    return os.path.join(_HERE, "libmiqp_b200.so")
 
 
 _lib = None

@@ -31,18 +31,11 @@ namespace miqp {
 // newborn node) it restarts from the best bound.  Deepest-first backtracking is deliberately NOT
 // used: it gets trapped below a wrong early decision (seen on 3 of 512 config-2 plans: 20k+ nodes
 // instead of ~40).  With an incumbent: best bound first, then deepest.
-// plunge: multi-car plans with an incumbent, every other round -- the preferred children (least violated alternative) of the last
-// two rounds go first, deepest first, the rest of the round is best-bound as usual (MIQP_MULTI_PLUNGE=1; off by default).  With 8
-// nodes per round (tests/emu, EMU_POLICY=3) alternating with dives improved the incumbents of the hard 1-4 agent scenarios from
-// gaps of 80-97 % to 17-29 % at the same node count, at +30 % nodes on the instances that are proven; on the device, where a plan
-// takes up to 64 nodes per round, the gain shrinks to 3 of 512 plans and 11 fewer are proven within 2 s (profiles/r2_knobs_heldout.md).
-__device__ __forceinline__ unsigned long long node_key(double bound, int depth, int rank, unsigned long long uid, bool have_inc, bool newborn,
-                                                       bool plunge = false, bool recent = false) {
+__device__ __forceinline__ unsigned long long node_key(double bound, int depth, int rank, unsigned long long uid, bool have_inc, bool newborn) {
   unsigned long long d = 1023 - (unsigned long long)(depth > 1023 ? 1023 : depth);  // 10 bits
   unsigned long long r = (unsigned long long)(rank + 1 > 127 ? 127 : rank + 1);      // 7 bits
   unsigned long long b = ordered_bits(bound) >> 24;                                   // 40 bits
   unsigned long long u = uid & 127ULL;                                                // 7 bits
-  if (have_inc && plunge) return (recent && rank <= 0) ? ((d << 47) | (b << 7) | u) : ((1ULL << 63) | (b << 17) | (d << 7) | u);
   if (have_inc) return (b << 24) | (d << 14) | (r << 7) | u;
   if (newborn) return (r << 47) | (b << 7) | u;
   return (1ULL << 63) | (b << 17) | (d << 7) | u;
@@ -135,7 +128,6 @@ __global__ void __launch_bounds__(SEL_THREADS) bnb_select_kernel(BnbState st, co
   const double ub = st.ub[s];
   const bool have_inc = ub < MQ_INF;
   const double cutoff = have_inc ? ub - p.gap_tol * fabs(ub) : MQ_INF;
-  const bool plunge = st.multi_plunge && p.C > 1 && have_inc && (round & 1);
   // nodes taken this round: one dive head per plan until an incumbent exists; afterwards the base
   // count, raised when few plans are still active so that the resident warps stay busy
   int K = st.sel_dive;
@@ -167,7 +159,7 @@ __global__ void __launch_bounds__(SEL_THREADS) bnb_select_kernel(BnbState st, co
       if (parked && keep) { key = 0ULL; atomicAdd(&s_nsusp, 1); }        // continues first: its state is only kept for one round
       else if (keep) {
         int2 m = st.meta[pb + slot];
-        key = node_key(b, m.x, meta_rank(m.y), st.uid[pb + slot], have_inc, meta_birth(m.y) == round - 1, plunge, meta_birth(m.y) >= round - 2);
+        key = node_key(b, m.x, meta_rank(m.y), st.uid[pb + slot], have_inc, meta_birth(m.y) == round - 1);
       }
       else { pruned = fmin(pruned, b); int pos = atomicAdd(&s_free, 1); st.free_stack[pb + pos] = slot; }
     }
@@ -187,10 +179,7 @@ __global__ void __launch_bounds__(SEL_THREADS) bnb_select_kernel(BnbState st, co
     for (int k = 0; k < SEL_THREADS / 32; ++k) pm = fmin(pm, s_pruned[k]);
     st.pruned_lb[s] = pm;
   }
-  // a plan whose frontier stays large after pruning is a hard one: let it run wide even while the easy
-  // plans still fill the machine (its sequential depth, not the node count, is what ends the batch)
   K += s_nsusp; if (K > KS) K = KS;   // parked relaxations do not take the place of new nodes
-  if (have_inc && st.wide_div > 0) { int kw = n1 / st.wide_div; if (kw > KS) kw = KS; if (kw > K) K = kw; }
   // 4. threshold key of the K best
   unsigned long long T = ~0ULL; int remaining = n1;  // take everything
   if (n1 > K) {

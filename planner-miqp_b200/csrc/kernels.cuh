@@ -37,8 +37,6 @@ struct BnbState {
   int sel_base;         // nodes per plan per round once an incumbent exists (raised when few plans are active)
   int sel_dive;         // nodes per plan per round while diving for the first incumbent
   int dive_fill;        // >0: while diving, widen to (resident warps / active plans) / dive_fill heads when few plans are active
-  int wide_div;         // >0: a plan with an incumbent takes at least (open nodes below the cutoff) / wide_div nodes per round
-  int multi_plunge;                 // multi-car plans with an incumbent: dives of the preferred children every other round (1) or best bound only (0)
   int multi_heur;                   // multi-car plans without incumbent: completion heuristic at every multi_heur-th level of the tree (0: off)
   int dive_patience, dive_growth;   // a plan without incumbent after dive_patience rounds widens its dive by dive_growth heads per round
   int work_cap;
@@ -100,10 +98,7 @@ void launch_bnb_init(const BnbState &st, const DevProb *probs, const unsigned ch
 void launch_bnb_select(const BnbState &st, const DevProb *probs, int round, double elapsed_s, cudaStream_t s);
 constexpr int SUSP_REQUEUE = 1 << 30;      // susp_slot mark of a node that is solved again from the cold start (keeps its slot like a parked one)
 constexpr int NODE_TEAM_WARPS = 4;        // warps that share one node relaxation (bnb_nodes_kernel), 2 teams per SM
-#ifndef MQ_TEAMS_PER_SM
-#define MQ_TEAMS_PER_SM 2
-#endif
-constexpr int NODE_TEAMS_PER_SM = MQ_TEAMS_PER_SM;   // 2: 255 registers per thread; 3: 168 registers (spills), A/B in profiles/r1k
+constexpr int NODE_TEAMS_PER_SM = 2;      // 255 registers per thread; 3 (168 registers, spills) gave no gain: profiles/r1k, r2_knobs_heldout
 constexpr int NODE_TEAM_WARPS_NARROW = 2; // throughput variant: two warps per node, four teams per SM (rounds with more nodes than the four-warp teams hold)
 constexpr int NODE_TEAM_WARPS_WIDE = 8;   // the same for rounds with fewer nodes than SMs, 1 team per SM
 // returns 0 or a cudaError

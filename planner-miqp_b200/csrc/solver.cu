@@ -98,8 +98,9 @@ struct MiqpB200Solver {
   DevBuf<double> b_multi_ws;
   DevBuf<int2> b_work2;
   bool uploaded = false, ran = false;
+  // the current run (start_run .. finish_run, batch runs and the stepped frontier search alike)
   long fr_rounds = 0; int fr_ctrl0 = 0;                       // rounds run so far / work items of the last round
-  std::chrono::steady_clock::time_point fr_t0;                // start of the current run (time limit)
+  std::chrono::steady_clock::time_point fr_t0;                // start of the run (time limit)
   long fr_launches = 0, fr_node_launches = 0; double fr_node_ms = 0.0;
   DevBuf<int> b_doneround; DevBuf<double> d_tlimit; std::vector<double> round_elapsed; std::vector<int> h_doneround;   // per-plan solve times and limits
   DevBuf<unsigned char> d_prev_dec; DevBuf<double> d_prev_ub; DevBuf<unsigned long long> d_prev_uid; DevBuf<int> d_same;   // previous cycle (replan)
@@ -129,7 +130,6 @@ struct MiqpB200Solver {
   cudaEvent_t ev_hv = nullptr;
   long hv_stride = 0;
   int hv_pending = 0, hv_bound = 0, hv_total = 0;
-  bool hv_defer = false;
 };
 
 namespace {
@@ -315,7 +315,9 @@ void deliver_final(MiqpB200Solver *s) {
 
 // Select / solve rounds of the uploaded batch, starting from the current device state: until every plan is finished, the time
 // limit or round cap is hit, or `max_rounds_now` rounds have run (< 0: no such cap).  Returns the number of unfinished plans.
-int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launches, long &node_launches, double &node_ms) {
+int run_rounds(MiqpB200Solver *s, long max_rounds_now) {
+  double tlim = 0.0;
+  for (double t : s->time_limits) tlim = std::max(tlim, t);
   int ctrl[8] = {s->fr_ctrl0, 0, 1, 0, 0, 0, 0, 0};
   long done_now = 0;
   for (;;) {
@@ -324,8 +326,8 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launch
     const double el0 = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
     if ((size_t)rounds >= s->round_elapsed.size()) s->round_elapsed.resize(rounds + 64, 0.0);
     launch_bnb_select(s->st, s->d_probs.p, (int)rounds + 1, el0, s->stream);
-    launches += 2;
-    if (s->on_done) { launch_harvest(s, 0, rounds == 0 ? s->st.count : s->hv_bound); launches += 4; }
+    s->fr_launches += 2;
+    if (s->on_done) { launch_harvest(s, 0, rounds == 0 ? s->st.count : s->hv_bound); s->fr_launches += 4; }
     CK(cudaEventRecord(s->evr0, s->stream));
     if (s->n_single > 0) {
       // fewer single-car nodes than wide teams fit (work count of the last round as the estimate): latency matters, not throughput;
@@ -340,28 +342,27 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launch
                                          s->single_maxN + 7, (int)rounds + 1, s->stream);
       if (narrow) ++s->narrow_launches;
       if (rc != 0) throw std::runtime_error(std::string("node kernel launch failed: ") + cudaGetErrorString((cudaError_t)rc));
-      ++launches; ++node_launches;
+      ++s->fr_launches; ++s->fr_node_launches;
     }
     if (s->n_multi > 0) {
       int rc = launch_bnb_nodes_multi(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->b_multi_ws.p, s->multi_ws_bytes,
                                       s->multi_use_smem, s->multi_threads, s->multi_ctas, (int)rounds + 1, s->stream);
       if (rc != 0) throw std::runtime_error(std::string("multi-car node kernel launch failed: ") + cudaGetErrorString((cudaError_t)rc));
-      ++launches; ++node_launches;
+      ++s->fr_launches; ++s->fr_node_launches;
     }
     CK(cudaEventRecord(s->evr1, s->stream));
-    if (s->on_done && !s->hv_defer) deliver_pending(s);   // the last round's plans, while this round's node kernels run
+    if (s->on_done) deliver_pending(s);   // the last round's plans, while this round's node kernels run
     ++s->fr_rounds; ++done_now;
     CK(cudaMemcpyAsync(ctrl, s->b_ctrl.p, sizeof ctrl, cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     s->fr_ctrl0 = ctrl[0];
     if (s->on_done) {
-      deliver_pending(s);   // (deferred delivery: the last round's plans)
       s->hv_bound = ctrl[2];   // only plans active in this round can finish in the next select
       if (ctrl[7] > 0) copy_records(s, ctrl[7]);
     }
     float ms = 0.f;
     CK(cudaEventElapsedTime(&ms, s->evr0, s->evr1));
-    node_ms += ms;
+    s->fr_node_ms += ms;
     if (s->opt.verbose > 1) fprintf(stderr, "[miqp_b200] round %ld: work %d active %d err %d node kernel %.3f ms (narrow launches so far %ld)\n", s->fr_rounds, ctrl[0], ctrl[2], ctrl[3], ms, s->narrow_launches);
     if (ctrl[2] == 0) break;  // every plan finished
     const double el = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
@@ -370,6 +371,59 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now, double tlim, long &launch
     if (s->opt.max_rounds > 0 && s->fr_rounds >= s->opt.max_rounds) { s->timed_out = true; break; }
   }
   return ctrl[2];
+}
+
+// Start of a search of the uploaded batch, for batch runs and the stepped search (miqp_b200_frontier_*) alike: fresh search
+// state, the run's counters and its clocks.  A streaming run also clears its delivered flags.
+void start_run(MiqpB200Solver *s) {
+  const int count = s->st.count;
+  s->fr_t0 = std::chrono::steady_clock::now();
+  CK(cudaMemsetAsync(s->b_prof.p, 0, 256 * sizeof(unsigned long long), s->stream));
+  if (s->st.susp_slot) CK(cudaMemsetAsync(s->st.susp_slot, 0xff, sizeof(int) * (size_t)count * s->st.cap, s->stream));
+  if (s->on_done) {
+    s->hv_stride = (STREAM_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
+    s->hv_delivered.ensure(count); s->hv_list.ensure(count); s->hv_rec.ensure((size_t)count * s->hv_stride);
+    s->h_hvrec.resize((size_t)count * s->hv_stride);
+    if (!s->ev_hv) CK(cudaEventCreateWithFlags(&s->ev_hv, cudaEventDisableTiming));
+    CK(cudaMemsetAsync(s->hv_delivered.p, 0, sizeof(int) * count, s->stream));
+    s->st.delivered = s->hv_delivered.p;
+    s->hv_pending = 0; s->hv_total = 0; s->hv_held.clear();
+  }
+  CK(cudaEventRecord(s->ev0, s->stream));
+  launch_bnb_init(s->st, s->d_probs.p, s->any_warm ? s->d_warm.p : nullptr, s->any_warm ? s->d_haswarm.p : nullptr, s->stream);
+  s->fr_rounds = 0; s->fr_ctrl0 = 0;
+  s->fr_launches = 1; s->fr_node_launches = 0; s->fr_node_ms = 0.0;
+  s->timed_out = false; s->ran = false;
+}
+
+// End of a search: final solution vectors and their evaluation, then the run's device time and statistics.  A streaming run
+// delivers the plans of its last round first, and the plans still searching when the batch stopped last (same evaluate code).
+void finish_run(MiqpB200Solver *s, float *device_ms) {
+  const bool streaming = s->on_done != nullptr;
+  const int count = s->st.count;
+  if (streaming) deliver_pending(s);
+  launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
+  if (!streaming) {
+    CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
+    launch_evaluate(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, count, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
+  } else {   // exactly the plans not delivered yet
+    const int left = count - s->hv_total;
+    launch_harvest(s, 1, left);
+    s->fr_launches += 2;
+    if (left > 0) copy_records(s, left);
+  }
+  s->fr_launches += 2;
+  CK(cudaGetLastError());
+  CK(cudaEventRecord(s->ev1, s->stream));
+  CK(cudaStreamSynchronize(s->stream));
+  float total_ms = 0.f;
+  CK(cudaEventElapsedTime(&total_ms, s->ev0, s->ev1));
+  if (device_ms) *device_ms = total_ms;
+  s->last_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
+  s->stats.launches = s->fr_launches; s->stats.node_kernel_launches = s->fr_node_launches; s->stats.rounds = s->fr_rounds;
+  s->stats.node_kernel_ms = s->fr_node_ms; s->stats.total_ms = total_ms;
+  s->ran = true;
+  if (streaming) deliver_final(s);
 }
 
 void setup_bnb(MiqpB200Solver *s) {
@@ -418,9 +472,7 @@ void setup_bnb(MiqpB200Solver *s) {
       s->narrow_min = 2 * s->ctas;   // between one and two waves of four-warp teams the two variants take the same time; the wider team has the lower latency
       if (const char *e = getenv("MIQP_NARROW_MIN")) s->narrow_min = atoi(e);
     }
-    int fm = 1;
-    if (const char *e = getenv("MIQP_FILL_MULT")) fm = std::max(1, atoi(e));
-    st.nwarps += 2 * s->num_sms * fm;   // the round-width rules are tuned for two teams per SM, whatever the launch uses
+    st.nwarps += 2 * s->num_sms;   // the round-width rules are tuned for two teams per SM, whatever the launch uses
   }
   if (s->n_multi > 0) {
     s->multi_threads = (maxCm <= 2) ? 64 : 128;
@@ -443,15 +495,11 @@ void setup_bnb(MiqpB200Solver *s) {
   st.sel_dive = std::max(1, std::min(8, st.nwarps / std::max(count, 1)));   // several dive heads only when warps would idle
   st.dive_fill = 2;   // A/B on 2048 config-2 plans (profiles/r1i, r1k): one dive head 347 ms / 120 rounds; widened dive 143 ms / 53 rounds
   if (const char *e = getenv("MIQP_DIVE_FILL")) st.dive_fill = atoi(e);
-  st.wide_div = 0;
-  if (const char *e = getenv("MIQP_WIDE_DIV")) st.wide_div = atoi(e);
   st.dive_patience = 14; st.dive_growth = 8;   // profiles/r1k: batch 1024 139 -> 80 ms, batch 2048 unchanged (144 ms, 53 -> 38 rounds)
   if (const char *e = getenv("MIQP_DIVE_PATIENCE")) st.dive_patience = atoi(e);
   if (const char *e = getenv("MIQP_DIVE_GROWTH")) st.dive_growth = atoi(e);
   st.multi_heur = 1;
   if (const char *e = getenv("MIQP_MULTI_HEUR")) st.multi_heur = atoi(e);
-  st.multi_plunge = 0;   // A/B on 512 config-4 plans, 2 s limit (profiles/r2_knobs_heldout.md): 3 hard plans more within 10 %, 11 fewer proven
-  if (const char *e = getenv("MIQP_MULTI_PLUNGE")) st.multi_plunge = atoi(e);
   int kscap = 64;
   // a few multi-car plans alone on the GPU (config 5: ONE joint plan): let a plan take as many nodes per round as CTAs are resident
   if (s->n_single == 0 && s->n_multi > 0) kscap = std::max(64, std::min(1024, st.nwarps / std::max(count, 1)));
@@ -824,62 +872,15 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
 // One search of the uploaded batch; a streaming run (s->on_done set) also harvests every plan in the round select marks it
 // finished and hands it to the callback.  Both compute the same results.
 static int run_batch(MiqpB200Solver *s, float *device_ms) {
-  const bool streaming = s->on_done != nullptr;
   struct Reset {   // the delivered flags are seen by the kernels of streaming runs only
     MiqpB200Solver *s;
     ~Reset() { s->st.delivered = nullptr; s->on_done = nullptr; s->on_done_user = nullptr; s->hv_pending = 0; s->hv_held.clear(); }
   } reset{s};
   try {
     CK(cudaSetDevice(s->opt.device));
-    const int count = s->st.count;
-    const auto t0 = std::chrono::steady_clock::now();
-    double tlim = 0.0;
-    for (double t : s->time_limits) tlim = std::max(tlim, t);
-    long launches = 0, node_launches = 0, rounds = 0;
-    double node_ms = 0.0;
-    CK(cudaMemsetAsync(s->b_prof.p, 0, 256 * sizeof(unsigned long long), s->stream));
-    if (s->st.susp_slot) CK(cudaMemsetAsync(s->st.susp_slot, 0xff, sizeof(int) * (size_t)s->st.count * s->st.cap, s->stream));
-    if (streaming) {
-      s->hv_stride = (STREAM_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
-      s->hv_delivered.ensure(count); s->hv_list.ensure(count); s->hv_rec.ensure((size_t)count * s->hv_stride);
-      s->h_hvrec.resize((size_t)count * s->hv_stride);
-      if (!s->ev_hv) CK(cudaEventCreateWithFlags(&s->ev_hv, cudaEventDisableTiming));
-      CK(cudaMemsetAsync(s->hv_delivered.p, 0, sizeof(int) * count, s->stream));
-      s->st.delivered = s->hv_delivered.p;
-      s->hv_pending = 0; s->hv_total = 0; s->hv_held.clear();
-      const char *e = std::getenv("MIQP_STREAM_DEFER");   // 1: deliver a round's plans after the next round's sync (A/B of the delivery point)
-      s->hv_defer = e && e[0] == '1';
-    }
-    CK(cudaEventRecord(s->ev0, s->stream));
-    launch_bnb_init(s->st, s->d_probs.p, s->any_warm ? s->d_warm.p : nullptr, s->any_warm ? s->d_haswarm.p : nullptr, s->stream);
-    ++launches;
-    s->timed_out = false;
-    s->fr_rounds = 0; s->fr_ctrl0 = 0; s->fr_t0 = t0;
-    run_rounds(s, -1, tlim, launches, node_launches, node_ms);
-    rounds = s->fr_rounds;
-    if (streaming) deliver_pending(s);   // the plans select finished in the last round
-    launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
-    if (!streaming) {
-      CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
-      launch_evaluate(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, count, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
-    } else {   // the plans that were still searching when the batch stopped: exactly the ones not delivered yet (same evaluate code)
-      const int left = count - s->hv_total;
-      launch_harvest(s, 1, left);
-      launches += 2;
-      if (left > 0) copy_records(s, left);
-    }
-    launches += 2;
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(s->ev1, s->stream));
-    CK(cudaStreamSynchronize(s->stream));
-    float total_ms = 0.f;
-    CK(cudaEventElapsedTime(&total_ms, s->ev0, s->ev1));
-    if (device_ms) *device_ms = total_ms;
-    s->last_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-    s->stats.launches = launches; s->stats.node_kernel_launches = node_launches; s->stats.rounds = rounds;
-    s->stats.node_kernel_ms = node_ms; s->stats.total_ms = total_ms;
-    s->ran = true;
-    if (streaming) deliver_final(s);
+    start_run(s);
+    run_rounds(s, -1);
+    finish_run(s, device_ms);
   } catch (const std::exception &ex) {
     return fail(s, MIQP_B200_ERR_CUDA, ex.what());
   }
@@ -1002,13 +1003,7 @@ int miqp_b200_frontier_start(MiqpB200Solver *s) {
   if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "frontier_start without batch_upload");
   try {
     CK(cudaSetDevice(s->opt.device));
-    CK(cudaMemsetAsync(s->b_prof.p, 0, 256 * sizeof(unsigned long long), s->stream));
-    if (s->st.susp_slot) CK(cudaMemsetAsync(s->st.susp_slot, 0xff, sizeof(int) * (size_t)s->st.count * s->st.cap, s->stream));
-    CK(cudaEventRecord(s->ev0, s->stream));
-    launch_bnb_init(s->st, s->d_probs.p, s->any_warm ? s->d_warm.p : nullptr, s->any_warm ? s->d_haswarm.p : nullptr, s->stream);
-    s->fr_rounds = 0; s->fr_ctrl0 = 0; s->fr_t0 = std::chrono::steady_clock::now();
-    s->fr_launches = 1; s->fr_node_launches = 0; s->fr_node_ms = 0.0;
-    s->timed_out = false; s->ran = false;
+    start_run(s);
     CK(cudaStreamSynchronize(s->stream));
   } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
   return MIQP_B200_OK;
@@ -1018,9 +1013,7 @@ int miqp_b200_frontier_rounds(MiqpB200Solver *s, int nrounds, int *unfinished) {
   if (!s || !s->uploaded) return MIQP_B200_ERR_ARG;
   try {
     CK(cudaSetDevice(s->opt.device));
-    double tlim = 0.0;
-    for (double t : s->time_limits) tlim = std::max(tlim, t);
-    const int left = run_rounds(s, nrounds, tlim, s->fr_launches, s->fr_node_launches, s->fr_node_ms);
+    const int left = run_rounds(s, nrounds);
     if (unfinished) *unfinished = s->timed_out ? 0 : left;
   } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
   return MIQP_B200_OK;
@@ -1083,20 +1076,7 @@ int miqp_b200_frontier_finish(MiqpB200Solver *s, float *device_ms) {
   if (!s || !s->uploaded) return MIQP_B200_ERR_ARG;
   try {
     CK(cudaSetDevice(s->opt.device));
-    const int count = s->st.count;
-    launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
-    CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
-    launch_evaluate(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, count, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(s->ev1, s->stream));
-    CK(cudaStreamSynchronize(s->stream));
-    float total_ms = 0.f;
-    CK(cudaEventElapsedTime(&total_ms, s->ev0, s->ev1));
-    if (device_ms) *device_ms = total_ms;
-    s->last_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
-    s->stats.launches = s->fr_launches + 2; s->stats.node_kernel_launches = s->fr_node_launches; s->stats.rounds = s->fr_rounds;
-    s->stats.node_kernel_ms = s->fr_node_ms; s->stats.total_ms = total_ms;
-    s->ran = true;
+    finish_run(s, device_ms);
   } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
   return MIQP_B200_OK;
 }

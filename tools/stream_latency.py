@@ -1,12 +1,11 @@
 """Per-plan delivery latency of streaming runs (Solver.run_streaming) against plain batch runs, on the flagship workload of
 bench.py: config 2 (one car, N = 40, R = 32), 2048 plans per batch, the same seeded shards, gap 1e-4.
 
-On one GPU, the same resident batches are run alternately plain (batch_run), streaming with delivery while the next round's
-node kernels run (the default) and streaming with delivery after the next round's sync (MIQP_STREAM_DEFER=1), --runs times
-each.  Reported: device time per batch (CUDA events) of every mode with its spread, per-plan latency from the start of the
-run to the callback (p50 / p90 / p99 / max) next to the batch time and next to each plan's own `seconds`, rounds per batch,
-the harvest kernels' share of device time (one separate torch.profiler run) and whether every run's outputs are identical.
-The card's name and power limit are read in the same process.
+On one GPU, the same resident batches are run alternately plain (batch_run) and streaming, --runs times each.  Reported:
+device time per batch (CUDA events) of both modes with its spread, per-plan latency from the start of the run to the callback
+(p50 / p90 / p99 / max) next to the batch time and next to each plan's own `seconds`, rounds per batch, the harvest kernels'
+share of device time (one separate torch.profiler run) and whether every run's outputs are identical.  The card's name and
+power limit are read in the same process.
 
     python tools/stream_latency.py --out profiles/stream_latency_batch2048.json
 """
@@ -27,7 +26,7 @@ import planner_miqp_b200 as P                                   # noqa: E402
 from planner_miqp_b200.scenarios import obstacle_scenario        # noqa: E402
 
 GAP = 1e-4
-MODES = ("plain", "stream", "stream_defer")
+MODES = ("plain", "stream")
 
 
 def gpu_info():
@@ -65,10 +64,6 @@ def run_once(s, mode):
         t0 = time.perf_counter()
         ms = s.run()
         return ms, time.perf_counter() - t0, None, None
-    if mode == "stream_defer":
-        os.environ["MIQP_STREAM_DEFER"] = "1"
-    else:
-        os.environ.pop("MIQP_STREAM_DEFER", None)
     n = s._batch[0]
     lat = np.full(n, np.nan)
     infos = [None] * n
@@ -80,7 +75,6 @@ def run_once(s, mode):
 
     ms = s.run_streaming(on_plan)
     wall = time.perf_counter() - t0
-    os.environ.pop("MIQP_STREAM_DEFER", None)
     return ms, wall, lat, infos
 
 
@@ -149,8 +143,7 @@ def main():
                     lat_all[mode].extend((lat * 1e3).tolist())
                     after_seconds[mode].extend(((lat - sec) * 1e3).tolist())
                     lat_over_batch[mode].extend((lat / wall).tolist())
-                    if mode == "stream":
-                        seconds_all.extend((sec * 1e3).tolist())
+                    seconds_all.extend((sec * 1e3).tolist())
     out = {
         "tool": "tools/stream_latency.py",
         "gpu": hw,
