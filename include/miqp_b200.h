@@ -32,9 +32,14 @@
  *                                  src/cplex_wrapper.cpp:680-690
  * miqp_b200_pool_sizes / _fetch    the pool's members (IloCplex::getSolnPoolNsolns /
  *                                  getValues(sol, i)), best first
+ * miqp_b200_pool_export / _merge   (no counterpart) the pool of a plan whose frontier is sharded
+ *                                  over GPUs: every rank's pool packed for an all-gather, and
+ *                                  the pool of the union of the ranks' leaves built from them
  */
 #ifndef MIQP_B200_H
 #define MIQP_B200_H
+
+#include <stddef.h>
 
 #ifdef __cplusplus
 extern "C" {
@@ -227,11 +232,25 @@ typedef struct MiqpB200PoolEntry {
 } MiqpB200PoolEntry;
 /* entries per plan, [count]; ERR_ARG with the pool off or before a run */
 int miqp_b200_pool_sizes(MiqpB200Solver *s, int *sizes /* [count] */);
-/* the first min(size, max_entries) entries of plan k in (search_value, uid) order -- entry 0 is the incumbent --, their full column
+/* the first min(size, max_entries) entries of plan k in (search_value, uid) order -- entry 0 is the incumbent; after pool_merge it
+ * is the best merged entry, which is the combined incumbent of the ranks, not necessarily this rank's own --, their full column
  * vectors (x_out, RawResults order like fetch_vector) and trajectories (traj_out, the compact layout of batch_fetch_compact) */
 int miqp_b200_pool_fetch(MiqpB200Solver *s, int k, int max_entries, MiqpB200PoolEntry *entries,
                          double *x_out /* [max_entries][ncols(k)] or NULL */,
                          double *traj_out /* [max_entries][C][N][8] or NULL */, int *n_out);
+/* Pools of a frontier-sharded search (frontier_*): each rank's pool holds the leaves that rank solved.  After frontier_finish every
+ * rank exports its pool, the exports are all-gathered (NCCL in place on the device buffers, or through the host), and every rank
+ * merges them: the result is the pool of the union of all ranks' leaves, the same on every rank and for any rank order.
+ * export: packs this solver's pool into a solver-owned device buffer (*dev, *bytes; valid until the next export, upload or
+ * destroy).  Layout: a 64-byte header (magic/version, count, capacity, zstride, ndec_stride, hash of every plan's C, N, R, O, L,
+ * E, ncols), then cnt[count], rec[count][cap], dec[count][cap][ndec_stride], z[count][cap][zstride], sections 16-byte aligned.
+ * merge: `gathered` holds `world` exports back to back (world x bytes; host memory or device memory); it replaces this solver's
+ * pool by the capacity best entries by (search_value, uid) with pairwise different decisions over all of them.  pool_sizes and
+ * pool_fetch then return the merged pool; entries are expanded and evaluated on this rank's own copy of the problem data.
+ * ERR_ARG, the pool unchanged: no run, pool off, world < 1, world x capacity > 512, or a header that does not match this
+ * solver's upload (another capacity or batch shape). */
+int miqp_b200_pool_export(MiqpB200Solver *s, void **dev, size_t *bytes);
+int miqp_b200_pool_merge(MiqpB200Solver *s, const void *gathered, int world);
 
 /* counters of the last run: kernel launches, node relaxations, IPM iterations, seconds
  * spent in the node kernel (CUDA events on the solver stream) */

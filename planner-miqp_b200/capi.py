@@ -29,7 +29,7 @@ DECLARED_SYMBOLS = [
     "miqp_b200_frontier_tighten", "miqp_b200_frontier_finish", "miqp_b200_frontier_fingerprint", "miqp_b200_frontier_ub_device", "miqp_b200_batch_upload_replan", "miqp_b200_mark", "miqp_b200_elapsed", "miqp_b200_batch_fetch_compact", "miqp_b200_fetch_vector",
     "miqp_b200_solve_batch_compact",
     "miqp_b200_set_solution_pool", "miqp_b200_pool_sizes", "miqp_b200_pool_fetch",
-    "miqp_b200_batch_run_streaming",
+    "miqp_b200_batch_run_streaming", "miqp_b200_pool_export", "miqp_b200_pool_merge",
 ]
 
 
@@ -127,6 +127,13 @@ class PoolEntry:
     traj: np.ndarray | None = None
 
 
+class _DevView:
+    """device memory of the solver as a __cuda_array_interface__ object (torch.as_tensor wraps it without a copy)"""
+
+    def __init__(self, ptr: int, n: int, typestr: str = "<f8"):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 3, "strides": None}
+
+
 def library_path() -> str:
     return os.path.join(_HERE, "libmiqp_b200.so")
 
@@ -165,6 +172,8 @@ def load_library():
     lib.miqp_b200_pool_sizes.argtypes = [C.c_void_p, _ip]
     lib.miqp_b200_pool_fetch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CPoolEntry), _dp, _dp, _ip]
     lib.miqp_b200_batch_run_streaming.argtypes = [C.c_void_p, PLAN_DONE, C.c_void_p, C.POINTER(C.c_float)]
+    lib.miqp_b200_pool_export.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
+    lib.miqp_b200_pool_merge.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
     _lib = lib
     return lib
 
@@ -271,6 +280,7 @@ class Solver:
             raise MiqpB200Error("miqp_b200_create failed: no usable CUDA device "
                                 "(this backend has no CPU fallback)")
         self._h = h
+        self._device = device
         self._batch = None
         if solution_pool:
             self.set_solution_pool(solution_pool)
@@ -440,6 +450,23 @@ class Solver:
         return [PoolEntry(e.objective, e.max_violation, e.search_value, bool(e.converged), e.round, e.uid,
                           None if x is None else x[j].copy(), None if tr is None else tr[j].copy())
                 for j, e in enumerate(ents[:got.value])]
+
+    def pool_export(self):
+        """this solver's pool packed for an all-gather (miqp_b200_pool_export): a torch.uint8 CUDA tensor that views the
+        solver's export buffer without a copy; valid until the next pool_export, upload or close"""
+        import torch
+        ptr, n = C.c_void_p(), C.c_size_t()
+        self._check(self._lib.miqp_b200_pool_export(self._h, C.byref(ptr), C.byref(n)), "miqp_b200_pool_export")
+        return torch.as_tensor(_DevView(ptr.value, n.value, "|u1"), device=torch.device("cuda", self._device))
+
+    def pool_merge(self, gathered, world: int):
+        """replaces this solver's pool by the merge of `world` exports stored back to back in `gathered` (a CPU or CUDA
+        tensor, miqp_b200_pool_merge): the pool of the union of the ranks' leaves"""
+        import torch
+        g = gathered.contiguous()
+        if g.is_cuda:
+            torch.cuda.synchronize(g.device)      # the C call reads it on the solver's own stream
+        self._check(self._lib.miqp_b200_pool_merge(self._h, C.c_void_p(g.data_ptr()), int(world)), "miqp_b200_pool_merge")
 
     def solve_prepared_compact(self, b, on_plan=None):
         """One miqp_b200_solve_batch_compact call on host buffers: pack + H2D + device solve + D2H of trajectories and infos.

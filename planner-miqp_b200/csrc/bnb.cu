@@ -1028,6 +1028,119 @@ void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const 
 }
 
 // ---------------------------------------------------------------------------------------
+// merge of the solution pools of several ranks (frontier sharding, miqp_b200_pool_merge)
+// ---------------------------------------------------------------------------------------
+// The pool policy (pool_slot) applied to the union of the ranks' leaves: the pool_cap best entries by key with pairwise different
+// decisions.  The ranks' pools suffice: the best leaf of a decision class in the global top pool_cap has fewer than pool_cap
+// distinct classes with a better key on its own rank, so it is in that rank's pool.  A greedy scan in key order over the
+// candidates of all ranks accepts every entry whose decisions differ from those accepted so far.  Leaves of the ramp-up are in
+// every rank's pool (same uid and decisions): the first copy is accepted, the others are duplicates.  Decisions are the plan's
+// own ndec_pad bytes: past them, up to the batch's ndec_stride, a node the multi-car kernel makes from its completion (k.imp)
+// carries bytes nothing wrote, which differ between ranks.
+constexpr int MERGE_THREADS = 256;
+
+__global__ void __launch_bounds__(MERGE_THREADS) pool_merge_kernel(BnbState st, const DevProb *probs, const unsigned char *g, PoolExportLayout lay,
+                                                                   int world) {
+  __shared__ double val[POOL_MERGE_MAX];
+  __shared__ unsigned long long uid[POOL_MERGE_MAX], hsh[POOL_MERGE_MAX];
+  __shared__ int src[POOL_MERGE_MAX];
+  __shared__ int acc[64];
+  __shared__ int nvalid;
+  const int k = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+  const int cap = st.pool_cap, nw = probs[k].ndec_pad / 16;
+  constexpr int NONE = 0x7fffffff;
+  // candidate i = entry i % cap of rank i / cap
+  auto entry = [=](int i) { return (long)k * cap + i % cap; };
+  auto dec_of = [=](int i) {
+    return reinterpret_cast<const uint4 *>(g + (long)(i / cap) * lay.bytes + lay.off_dec + entry(i) * st.ndec_stride);
+  };
+  auto rec_of = [=](int i) { return reinterpret_cast<const PoolRec *>(g + (long)(i / cap) * lay.bytes + lay.off_rec) + entry(i); };
+  const int n = world * cap;
+  int np = 1;
+  while (np < n) np <<= 1;
+  if (tid == 0) nvalid = 0;
+  for (int i = tid; i < np; i += nt) {
+    double v = MQ_INF; unsigned long long u = ~0ULL; int c = NONE;
+    if (i < n) {
+      const int cnt = reinterpret_cast<const int *>(g + (long)(i / cap) * lay.bytes + lay.off_cnt)[k];
+      if (i % cap < min(max(cnt, 0), cap)) { const PoolRec *r = rec_of(i); v = r->val; u = r->uid; c = i; }
+    }
+    val[i] = v; uid[i] = u; src[i] = c;
+  }
+  __syncthreads();
+  // bitonic sort by (value, uid, candidate index); the empty slots (inf, ~0, NONE) go last
+  for (int kk = 2; kk <= np; kk <<= 1)
+    for (int j = kk >> 1; j > 0; j >>= 1) {
+      for (int i = tid; i < np; i += nt) {
+        const int l = i ^ j;
+        if (l <= i) continue;
+        const bool l_first = pool_key_less(val[l], uid[l], val[i], uid[i]) || (val[l] == val[i] && uid[l] == uid[i] && src[l] < src[i]);
+        if (((i & kk) == 0) == l_first) {
+          const double tv = val[i]; val[i] = val[l]; val[l] = tv;
+          const unsigned long long tu = uid[i]; uid[i] = uid[l]; uid[l] = tu;
+          const int tc = src[i]; src[i] = src[l]; src[l] = tc;
+        }
+      }
+      __syncthreads();
+    }
+  for (int i = tid; i < np; i += nt)
+    if (src[i] != NONE && (i + 1 == np || src[i + 1] == NONE)) nvalid = i + 1;
+  __syncthreads();
+  const int nv = nvalid;
+  // 64-bit hash of every candidate's decision bytes (one warp per candidate; a sum, so the order of the lanes does not matter).
+  // Only a filter: candidates with equal hashes are compared byte for byte.
+  const int lane = tid & 31;
+  for (int i = tid >> 5; i < nv; i += nt >> 5) {
+    const uint4 *d = dec_of(src[i]);
+    unsigned long long h = 0;
+    for (int w = lane; w < nw; w += 32) {
+      const uint4 q = d[w];
+      h += mix64((((unsigned long long)q.y << 32) | q.x) ^ mix64((((unsigned long long)q.w << 32) | q.z) + (unsigned long long)w));
+    }
+    for (int o = 16; o > 0; o >>= 1) h += __shfl_xor_sync(FULL, h, o);
+    if (lane == 0) hsh[i] = h;
+  }
+  __syncthreads();
+  // greedy scan in key order (every branch below depends on shared memory only: uniform over the block)
+  int nacc = 0;
+  for (int i = 0; i < nv && nacc < cap; ++i) {
+    bool dup = false;
+    for (int a = 0; a < nacc && !dup; ++a) {
+      if (hsh[acc[a]] != hsh[i]) continue;
+      const uint4 *x = dec_of(src[acc[a]]), *y = dec_of(src[i]);
+      int diff = 0;
+      for (int w = tid; w < nw; w += nt) {
+        const uint4 p = x[w], q = y[w];
+        diff |= (p.x != q.x) || (p.y != q.y) || (p.z != q.z) || (p.w != q.w);
+      }
+      dup = !__syncthreads_or(diff);
+    }
+    if (!dup) {
+      if (tid == 0) acc[nacc] = i;
+      ++nacc;
+    }
+    __syncthreads();
+  }
+  // the accepted entries, in key order, into this solver's pool
+  const PoolRef pr = pool_ref(st, k);
+  for (int a = 0; a < nacc; ++a) {
+    const int c = src[acc[a]];
+    const double *z = reinterpret_cast<const double *>(g + (long)(c / cap) * lay.bytes + lay.off_z) + entry(c) * st.zstride;
+    for (int q = tid; q < st.zstride; q += nt) pr.z[(long)a * st.zstride + q] = z[q];
+    const uint4 *d = dec_of(c);
+    uint4 *dd = reinterpret_cast<uint4 *>(pr.dec + (long)a * st.ndec_stride);
+    for (int w = tid; w < st.ndec_stride / 16; w += nt) dd[w] = d[w];
+    if (tid == 0) pr.rec[a] = *rec_of(c);
+  }
+  if (tid == 0) *pr.cnt = nacc;
+}
+
+void launch_pool_merge(const BnbState &st, const DevProb *probs, const unsigned char *gathered, const PoolExportLayout &lay, int world,
+                       cudaStream_t s) {
+  pool_merge_kernel<<<st.count, MERGE_THREADS, 0, s>>>(st, probs, gathered, lay, world);
+}
+
+// ---------------------------------------------------------------------------------------
 // streaming runs: harvest of the plans that bnb_select_kernel marked finished, in the same round.  Once select has set done[s],
 // nothing of the search writes plan s again, so its result is final.  The host launches the kernels after select and before the
 // node kernels, sizing the grids by the plans still active in the previous round (an upper bound of the plans select can finish

@@ -115,6 +115,15 @@ void launch_bnb_finish(const BnbState &st, const DevProb *probs, const double *d
 // into xall; the entry's trajectory goes to zs[e * zstride] (pool storage is not modified)
 void launch_pool_expand(const BnbState &st, int k, const int *idx, int n, const DevProb *eprobs, const double *dblob, const int *iblob,
                         double *zs, double *xall, cudaStream_t s);
+// byte offsets of the sections of one pool export (miqp_b200_pool_export): header, cnt[count], rec[count][pool_cap],
+// dec[count][pool_cap][ndec_stride], z[count][pool_cap][zstride]; every section and the whole export 16-byte aligned
+struct PoolExportLayout { long off_cnt, off_rec, off_dec, off_z, bytes; };
+constexpr int POOL_MERGE_MAX = 512;   // candidates per plan (world x pool_cap) pool_merge_kernel sorts in shared memory
+// this solver's pool := the pool_cap best entries, by (value, uid), with pairwise different decisions (the plan's ndec_pad bytes)
+// of `world` exports stored back to back at `gathered` (device memory of the solver's GPU, exports lay.bytes apart; the pool
+// storage itself is not read)
+void launch_pool_merge(const BnbState &st, const DevProb *probs, const unsigned char *gathered, const PoolExportLayout &lay, int world,
+                       cudaStream_t s);
 // ---- streaming runs: per-round harvest of the plans that select marked finished -------------------------------------------
 // one record per harvested plan, then its trajectory [C][N][8] (inc_z after expand_solution); records are rec_stride doubles apart
 struct StreamRec {

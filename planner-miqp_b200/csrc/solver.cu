@@ -121,6 +121,7 @@ struct MiqpB200Solver {
   int solution_pool = 0;
   DevBuf<double> sp_z; DevBuf<unsigned char> sp_dec; DevBuf<PoolRec> sp_rec; DevBuf<int> sp_cnt;
   DevBuf<DevProb> sp_probs; DevBuf<int> sp_idx; DevBuf<double> sp_x, sp_zs, sp_obj, sp_viol;
+  DevBuf<unsigned char> sp_export, sp_gathered;   // miqp_b200_pool_export's buffer; device copy of a merge input from elsewhere
   // streaming runs (miqp_b200_batch_run_streaming): callback (null outside such a run), delivered flags, harvest list, records
   // (device staging and page-locked host copy), records copied but not yet delivered, records held for the end of the run
   MiqpB200PlanDone on_done = nullptr; void *on_done_user = nullptr;
@@ -596,6 +597,44 @@ void setup_bnb(MiqpB200Solver *s) {
 
 }  // namespace
 
+// ---- pool export layout (miqp_b200_pool_export / miqp_b200_pool_merge) ----------------------------------------------------
+namespace {
+constexpr unsigned POOL_EXPORT_MAGIC = 0x4c4f4f50u;   // "POOL"
+constexpr unsigned POOL_EXPORT_VERSION = 1;
+struct PoolExportHeader {   // first 64 bytes of an export
+  unsigned magic, version;
+  int count, cap, zstride, ndec_stride;
+  unsigned long long shape_hash;   // FNV-1a over (C, N, R, O, L, E, ncols) of every plan
+  unsigned char pad[32];
+};
+static_assert(sizeof(PoolExportHeader) == 64, "export header size");
+
+long align16(long b) { return (b + 15) & ~15L; }
+
+PoolExportLayout export_layout(const BnbState &st) {
+  PoolExportLayout l;
+  const long entries = (long)st.count * st.pool_cap;
+  l.off_cnt = sizeof(PoolExportHeader);
+  l.off_rec = align16(l.off_cnt + (long)sizeof(int) * st.count);
+  l.off_dec = align16(l.off_rec + (long)sizeof(PoolRec) * entries);
+  l.off_z = align16(l.off_dec + entries * st.ndec_stride);
+  l.bytes = align16(l.off_z + (long)sizeof(double) * entries * st.zstride);
+  return l;
+}
+
+PoolExportHeader export_header(const MiqpB200Solver *s) {
+  PoolExportHeader h;
+  std::memset(&h, 0, sizeof h);
+  h.magic = POOL_EXPORT_MAGIC; h.version = POOL_EXPORT_VERSION;
+  h.count = s->st.count; h.cap = s->st.pool_cap; h.zstride = s->st.zstride; h.ndec_stride = s->st.ndec_stride;
+  unsigned long long f = 0xcbf29ce484222325ULL;
+  for (const DevProb &p : s->pk.probs)
+    for (int v : {p.C, p.N, p.R, p.O, p.L, p.E, p.ncols}) { f ^= (unsigned)v; f *= 0x100000001b3ULL; }
+  h.shape_hash = f;
+  return h;
+}
+}  // namespace
+
 extern "C" {
 
 const char *miqp_b200_version(void) { return "planner-miqp_b200 0.1 (sm_100a)"; }
@@ -647,7 +686,7 @@ void miqp_b200_destroy(MiqpB200Solver *s) {
   s->b_pruned.release(); s->b_incz.release(); s->b_meta.release(); s->b_work.release();
   s->b_uid.release(); s->b_keybuf.release(); s->b_incuid.release(); s->b_stats.release(); s->b_open.release();
   s->b_opencnt.release(); s->b_free.release(); s->b_freecnt.release(); s->b_sel.release(); s->b_selcnt.release();
-  s->sp_z.release(); s->sp_dec.release(); s->sp_rec.release(); s->sp_cnt.release();
+  s->sp_z.release(); s->sp_dec.release(); s->sp_rec.release(); s->sp_cnt.release(); s->sp_export.release(); s->sp_gathered.release();
   s->b_zpool.release(); s->b_susp0.release(); s->b_susp1.release(); s->b_suspslot.release(); s->b_suspcnt.release(); s->b_done.release(); s->b_overflow.release(); s->b_lock.release(); s->b_ctrl.release(); s->b_multi_ws.release(); s->b_work2.release();
   if (s->ev0) cudaEventDestroy(s->ev0);
   if (s->ev1) cudaEventDestroy(s->ev1);
@@ -1192,6 +1231,77 @@ int miqp_b200_pool_fetch(MiqpB200Solver *s, int k, int max_entries, MiqpB200Pool
       o.objective = obj[e]; o.max_violation = viol[e]; o.search_value = r.val;
       o.converged = r.converged; o.round = r.round; o.uid = r.uid;
     }
+  } catch (const std::exception &ex) {
+    return fail(s, MIQP_B200_ERR_CUDA, ex.what());
+  }
+  return MIQP_B200_OK;
+}
+
+// ---- pool export / merge (frontier sharding: the pools of all ranks) ----------------------------------------------------------
+int miqp_b200_pool_export(MiqpB200Solver *s, void **dev, size_t *bytes) {
+  if (!s || !dev || !bytes) return MIQP_B200_ERR_ARG;
+  if (const char *why = pool_unavailable(s)) return fail(s, MIQP_B200_ERR_ARG, why);
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    const BnbState &st = s->st;
+    const PoolExportLayout l = export_layout(st);
+    const PoolExportHeader h = export_header(s);
+    const size_t entries = (size_t)st.count * st.pool_cap;
+    s->sp_export.ensure((size_t)l.bytes);
+    unsigned char *b = s->sp_export.p;
+    CK(cudaMemcpyAsync(b, &h, sizeof h, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(b + l.off_cnt, st.pool_cnt, sizeof(int) * st.count, cudaMemcpyDeviceToDevice, s->stream));
+    CK(cudaMemcpyAsync(b + l.off_rec, st.pool_rec, sizeof(PoolRec) * entries, cudaMemcpyDeviceToDevice, s->stream));
+    CK(cudaMemcpyAsync(b + l.off_dec, st.pool_dec, entries * st.ndec_stride, cudaMemcpyDeviceToDevice, s->stream));
+    CK(cudaMemcpyAsync(b + l.off_z, st.pool_z, sizeof(double) * entries * st.zstride, cudaMemcpyDeviceToDevice, s->stream));
+    CK(cudaStreamSynchronize(s->stream));   // (the header's host copy goes out of scope)
+    *dev = b;
+    *bytes = (size_t)l.bytes;
+  } catch (const std::exception &ex) {
+    return fail(s, MIQP_B200_ERR_CUDA, ex.what());
+  }
+  return MIQP_B200_OK;
+}
+
+int miqp_b200_pool_merge(MiqpB200Solver *s, const void *gathered, int world) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (const char *why = pool_unavailable(s)) return fail(s, MIQP_B200_ERR_ARG, why);
+  if (!gathered || world < 1) return fail(s, MIQP_B200_ERR_ARG, "pool_merge: no input or world < 1");
+  if ((long)world * s->st.pool_cap > POOL_MERGE_MAX)
+    return fail(s, MIQP_B200_ERR_ARG, "pool_merge: world x pool capacity exceeds " + std::to_string(POOL_MERGE_MAX));
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    const PoolExportLayout l = export_layout(s->st);
+    const size_t total = (size_t)l.bytes * world;
+    cudaPointerAttributes attr;
+    const bool here = cudaPointerGetAttributes(&attr, gathered) == cudaSuccess && attr.device == s->opt.device &&
+                      (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged);
+    cudaGetLastError();   // (an older runtime reports a host pointer it does not know as an error)
+    // headers first, every one checked before the pool changes
+    const PoolExportHeader mine = export_header(s);
+    std::vector<PoolExportHeader> hs(world);
+    for (int r = 0; r < world; ++r) {
+      const unsigned char *src = static_cast<const unsigned char *>(gathered) + (size_t)r * l.bytes;
+      CK(cudaMemcpyAsync(&hs[r], src, sizeof(PoolExportHeader), cudaMemcpyDefault, s->stream));
+    }
+    CK(cudaStreamSynchronize(s->stream));
+    for (int r = 0; r < world; ++r) {
+      const PoolExportHeader &h = hs[r];
+      if (h.magic != mine.magic || h.version != mine.version || h.count != mine.count || h.cap != mine.cap ||
+          h.zstride != mine.zstride || h.ndec_stride != mine.ndec_stride || h.shape_hash != mine.shape_hash)
+        return fail(s, MIQP_B200_ERR_ARG, "pool_merge: export " + std::to_string(r) +
+                                              " does not come from a solver with this batch's shapes and pool capacity");
+    }
+    const unsigned char *g = static_cast<const unsigned char *>(gathered);
+    if (!here) {   // host memory or another GPU: a copy on this solver's device
+      s->sp_gathered.ensure(total);
+      CK(cudaMemcpyAsync(s->sp_gathered.p, gathered, total, cudaMemcpyDefault, s->stream));
+      g = s->sp_gathered.p;
+    }
+    launch_pool_merge(s->st, s->d_probs.p, g, l, world, s->stream);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(s->stream));
+    s->stats.launches += 1;
   } catch (const std::exception &ex) {
     return fail(s, MIQP_B200_ERR_CUDA, ex.what());
   }

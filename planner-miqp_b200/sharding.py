@@ -10,7 +10,10 @@ from __future__ import annotations
 
 import dataclasses
 import os
+import time
 from typing import Callable, Sequence
+
+from .capi import MiqpB200Error, _DevView
 
 
 def shard_indices(count: int, rank: int, world: int) -> list[int]:
@@ -54,15 +57,8 @@ def solve_sharded(problems: Sequence, solve_fn: Callable, group=None):
 # ---------------------------------------------------------------------------------------------------------------------
 # Frontier sharding (SURVEY.md section 8(e).2): ONE plan (or a few), its open nodes distributed over the ranks
 # ---------------------------------------------------------------------------------------------------------------------
-class _DevView:
-    """device memory of the solver as a __cuda_array_interface__ object (torch.as_tensor wraps it without a copy)"""
-
-    def __init__(self, ptr: int, n: int):
-        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False), "version": 3, "strides": None}
-
-
 def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=None, warm=None, group=None,
-                           ramp_rounds: int = 6, exchange_every: int = 4, stats: dict | None = None):
+                           ramp_rounds: int = 6, exchange_every: int = 4, stats: dict | None = None, merge_pool: bool = False):
     """Every rank passes the same `problems` and its own solver (one GPU each); returns (xs, infos) of ALL plans on every
     rank.  Each plan's branch-and-bound frontier is sharded over the ranks:
 
@@ -76,6 +72,11 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
 
     Node order depends on the rank count (like CPLEX's opportunistic mode); bounds stay valid: every open node lives on
     exactly one rank and pruned bounds are kept per rank.
+
+    merge_pool (solution pool on at upload, world > 1): after the search every rank exports its pool, the exports are
+    all-gathered (NCCL: straight from the device buffers; gloo: through the host) in rank order and merged, so that
+    solver.pool(k) on every rank returns the same pool, that of the union of all ranks' leaves.  stats gains pool_bytes
+    (one rank's export) and pool_merge_ms.  Nothing else of the result changes.
     """
     import numpy as np
     import torch
@@ -124,6 +125,9 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
     if not sharded:
         return xs, infos
 
+    if merge_pool:
+        _merge_pools(solver, group, world, dev, on_nccl, allreduce, stats)
+
     # -- combine: objective and winner per plan, best bound, node counts
     big = 1e300
     own = np.array([i.objective if i.status == 0 else big for i in infos])
@@ -153,3 +157,34 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
                                 uncertified=int(counts[k, 2]), pool_exhausted=int(counts[k, 3] > 0),
                                 max_violation=float(viol[k]) if have else float("nan")))
     return out_x, out_i
+
+
+def _merge_pools(solver, group, world, dev, on_nccl, allreduce, stats):
+    """every rank's pool export, all-gathered in rank order, merged on every rank (solve_frontier_sharded(merge_pool=True))"""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    try:
+        exp, err = solver.pool_export(), None
+    except MiqpB200Error as ex:            # (pool off at upload) every rank learns of it before any rank raises
+        exp, err = None, ex
+    nbytes = 0 if exp is None else int(exp.numel())
+    hi, neg_lo = allreduce(np.array([nbytes, -nbytes], dtype=np.int64), dist.ReduceOp.MAX)
+    if err is not None:
+        raise err
+    if hi != -neg_lo or hi == 0:
+        raise MiqpB200Error("solve_frontier_sharded(merge_pool=True): the solution pool was off or differs between the ranks "
+                            "(set the same capacity on every rank before the upload)")
+    if on_nccl:
+        gathered = torch.empty(world * nbytes, dtype=torch.uint8, device=dev)
+        dist.all_gather_into_tensor(gathered, exp, group=group)
+        torch.cuda.synchronize()
+    else:
+        mine = exp.cpu()
+        parts = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(parts, mine, group=group)
+        gathered = torch.cat(parts)
+    t0 = time.perf_counter()
+    solver.pool_merge(gathered, world)
+    if stats is not None:
+        stats.update(pool_bytes=nbytes, pool_merge_ms=1e3 * (time.perf_counter() - t0))
