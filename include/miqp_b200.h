@@ -27,6 +27,12 @@
  * miqp_b200_batch_run_streaming    the same run, each plan's result handed to a callback in
  *                                  the round its search ends (one result per cplex.solve()
  *                                  of the reference, instead of one per batch)
+ * miqp_b200_batch_run_anytime      the same run, each plan's improved incumbent handed to a
+ *                                  callback while the search goes on (CPLEX's incumbent
+ *                                  callback); a nonzero return stops the plan
+ * miqp_b200_request_stop           IloCplex::Aborter / abort(): ends the search of one plan or
+ *                                  of all plans, from any thread
+ * miqp_b200_stopped                (no counterpart) the last round each stopped plan was searched
  * miqp_b200_set_solution_pool      the solution pool of cplex.solve(); its size is
  *                                  SolutionProperties.NrSolutionPool, collectCplexStatistics,
  *                                  src/cplex_wrapper.cpp:680-690
@@ -188,6 +194,42 @@ int miqp_b200_batch_fetch(MiqpB200Solver *s, double *const *x_out, MiqpB200Solve
  * ERR_ARG: on_done == NULL or no upload. */
 typedef void (*MiqpB200PlanDone)(void *user, int k, const double *traj, const MiqpB200SolveInfo *info);
 int miqp_b200_batch_run_streaming(MiqpB200Solver *s, MiqpB200PlanDone on_done, void *user, float *device_ms);
+
+/* Anytime run: the same search as batch_run, and every improvement of a plan's incumbent is handed to `on_incumbent` while the
+ * search goes on.  The device lists the plans whose incumbent changed at each round's select, expands and evaluates the incumbent
+ * exactly as at the end of the run, and the callback runs on the calling thread, between rounds: an incumbent found in round r is
+ * listed at the select of round r + 1 and delivered while the node kernels of round r + 2 run.  Several improvements of one plan
+ * within one round are delivered once, as the last of them.  Within a delivery plans come in ascending k; a plan's incumbents come
+ * before its `on_done` (may be NULL; the callback of batch_run_streaming, same contract).  For a plan that ends with an incumbent,
+ * the last record delivered has the trajectory, objective and max_violation batch_fetch_compact returns for it after the run.
+ * `traj` ([C][N][8]) and `inc` are valid during the call only.  The callbacks must not call into this solver, except
+ * miqp_b200_request_stop.  A nonzero return of on_incumbent stops plan k (as miqp_b200_request_stop(s, k)).
+ * batch_fetch, batch_fetch_compact, fetch_vector, pool_sizes / pool_fetch and batch_upload_replan work as after batch_run.
+ * ERR_ARG: on_incumbent == NULL or no upload. */
+typedef struct MiqpB200Incumbent {
+  double objective, max_violation;   /* of the expanded full vector, device-evaluated like MiqpB200SolveInfo */
+  double search_value;               /* value the search stored */
+  double best_bound, gap;            /* the plan's best bound when the round ended, gap as in MiqpB200SolveInfo */
+  double seconds;                    /* host clock at the end of the round that found it, from the start of the run */
+  long round, nodes, qp_iters;       /* round that found it; node relaxations and interior-point iterations of the plan so far */
+  unsigned long long uid;            /* node uid of the incumbent */
+} MiqpB200Incumbent;
+/* return nonzero to stop plan k (same as miqp_b200_request_stop(s, k)) */
+typedef int (*MiqpB200IncumbentFound)(void *user, int k, const double *traj, const MiqpB200Incumbent *inc);
+int miqp_b200_batch_run_anytime(MiqpB200Solver *s, MiqpB200IncumbentFound on_incumbent,
+                                MiqpB200PlanDone on_done /* may be NULL */, void *user, float *device_ms);
+/* Stop plan k (-1: every plan) of the uploaded batch: safe from any thread and from the callbacks.  The request takes effect at
+ * the next select a batch run (batch_run, _streaming, _anytime) launches after it; requests made between an upload and a run
+ * apply from round 1.  A callback runs after the next round's select has been launched, so a stop it returns for a record found
+ * in round r takes effect at the select of round r + 3: the plan is still searched in rounds r + 1 and r + 2.  A stopped plan
+ * ends like one that hit its time limit: SUCCESS with its incumbent (proven from the gap at that point), FAILED_TIMEOUT without
+ * one.  Requests are cleared when a run ends and at every upload.  The frontier path (frontier_*) ignores them.  Stopping plans
+ * changes how many nodes the other plans take per round, so their search order changes; it stays deterministic for the same stop
+ * rounds.  Does not set last_error.  ERR_ARG: no upload or k out of range. */
+int miqp_b200_request_stop(MiqpB200Solver *s, int k /* -1: every plan */);
+/* after a run: the last round each stopped plan was searched in (0: stopped before its first node), -1 = not stopped.
+ * ERR_ARG before a run. */
+int miqp_b200_stopped(MiqpB200Solver *s, int *round /* [count] */);
 
 /* Compact results: per plan the trajectory of every car, [C][N][8] doubles (pos_x, vel_x, acc_x, pos_y, vel_y, acc_y, u_x, u_y per
  * step: what MiqpPlanner::GetTrajectory reads, src/miqp_planner.cpp:1117-1192) instead of the full OPL column vector (config 2:

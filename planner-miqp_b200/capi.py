@@ -30,6 +30,7 @@ DECLARED_SYMBOLS = [
     "miqp_b200_solve_batch_compact",
     "miqp_b200_set_solution_pool", "miqp_b200_pool_sizes", "miqp_b200_pool_fetch",
     "miqp_b200_batch_run_streaming", "miqp_b200_pool_export", "miqp_b200_pool_merge",
+    "miqp_b200_batch_run_anytime", "miqp_b200_request_stop", "miqp_b200_stopped",
 ]
 
 
@@ -90,6 +91,16 @@ class CPoolEntry(C.Structure):
 PLAN_DONE = C.CFUNCTYPE(None, C.c_void_p, C.c_int, _dp, C.POINTER(CSolveInfo))
 
 
+class CIncumbent(C.Structure):
+    _fields_ = [("objective", C.c_double), ("max_violation", C.c_double), ("search_value", C.c_double),
+                ("best_bound", C.c_double), ("gap", C.c_double), ("seconds", C.c_double),
+                ("round", C.c_long), ("nodes", C.c_long), ("qp_iters", C.c_long), ("uid", C.c_ulonglong)]
+
+
+# int (*MiqpB200IncumbentFound)(void *user, int k, const double *traj, const MiqpB200Incumbent *inc)
+INCUMBENT_FOUND = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, _dp, C.POINTER(CIncumbent))
+
+
 class CRunStats(C.Structure):
     _fields_ = [("launches", C.c_long), ("node_kernel_launches", C.c_long), ("nodes", C.c_long),
                 ("qp_iters", C.c_long), ("rounds", C.c_long), ("node_kernel_ms", C.c_double),
@@ -111,6 +122,23 @@ class SolveInfo:
     rounds: int
     uncertified: int = 0
     pool_exhausted: int = 0
+
+
+@dataclass
+class Incumbent:
+    """An improved incumbent of an anytime run (miqp_b200_batch_run_anytime): objective and max violation of its full column
+    vector (device-evaluated), the value the search stored, the plan's best bound and gap when the round that found it ended,
+    the host clock then (seconds from the start of the run), that round, and the plan's node and iteration counters so far."""
+    objective: float
+    max_violation: float
+    search_value: float
+    best_bound: float
+    gap: float
+    seconds: float
+    round: int
+    nodes: int
+    qp_iters: int
+    uid: int
 
 
 @dataclass
@@ -174,6 +202,9 @@ def load_library():
     lib.miqp_b200_batch_run_streaming.argtypes = [C.c_void_p, PLAN_DONE, C.c_void_p, C.POINTER(C.c_float)]
     lib.miqp_b200_pool_export.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
     lib.miqp_b200_pool_merge.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
+    lib.miqp_b200_batch_run_anytime.argtypes = [C.c_void_p, INCUMBENT_FOUND, PLAN_DONE, C.c_void_p, C.POINTER(C.c_float)]
+    lib.miqp_b200_request_stop.argtypes = [C.c_void_p, C.c_int]
+    lib.miqp_b200_stopped.argtypes = [C.c_void_p, _ip]
     _lib = lib
     return lib
 
@@ -539,6 +570,62 @@ class Solver:
             raise failed[0]
         self._check(rc, "miqp_b200_batch_run_streaming")
         return ms.value
+
+    def run_anytime(self, on_incumbent, on_plan=None) -> float:
+        """miqp_b200_batch_run_anytime: the same run as run(), with on_incumbent(k, traj, inc) called for every improvement of a
+        plan's incumbent while the search goes on (on this thread, between rounds, ascending k within a delivery; traj is a copy
+        [C][N][8], inc an Incumbent).  A truthy return stops plan k (request_stop(k)); it takes effect two rounds after the round
+        that found the incumbent.  on_plan(k, traj, info): also the deliveries of run_streaming, each plan's after its incumbents.
+        An exception raised by a callback stops the calls to both (the plan it was raised for is not stopped); the run finishes
+        and the exception is raised here.  Returns the device time in ms."""
+        shapes = getattr(self, "_shapes", None)   # (None before an upload: the C call refuses the run)
+        failed = []
+
+        def copy_traj(k, traj):
+            c, nn = shapes[k]
+            return np.ctypeslib.as_array(traj, shape=(c * nn * 8,)).reshape(c, nn, 8).copy()
+
+        def inc_cb(_user, k, traj, inc):
+            if failed:
+                return 0
+            try:
+                i = inc.contents
+                stop = on_incumbent(k, copy_traj(k, traj), Incumbent(i.objective, i.max_violation, i.search_value, i.best_bound,
+                                                                     i.gap, i.seconds, i.round, i.nodes, i.qp_iters, i.uid))
+                return 1 if stop else 0
+            except BaseException as ex:   # ctypes would print and drop it
+                failed.append(ex)
+                return 0
+
+        def done_cb(_user, k, traj, info):
+            if failed:
+                return
+            try:
+                on_plan(k, copy_traj(k, traj), self._info(info.contents))
+            except BaseException as ex:
+                failed.append(ex)
+
+        ifunc = INCUMBENT_FOUND(inc_cb)
+        dfunc = PLAN_DONE(done_cb) if on_plan is not None else PLAN_DONE()
+        ms = C.c_float()
+        rc = self._lib.miqp_b200_batch_run_anytime(self._h, ifunc, dfunc, None, C.byref(ms))
+        if failed:
+            raise failed[0]
+        self._check(rc, "miqp_b200_batch_run_anytime")
+        return ms.value
+
+    def request_stop(self, k: int = -1):
+        """stop plan k (-1: every plan) of the uploaded batch at the next select of a run; safe from any thread and from the
+        callbacks of run_anytime / run_streaming.  Requests are cleared when a run ends and at every upload."""
+        rc = self._lib.miqp_b200_request_stop(self._h, int(k))
+        if rc != 0:
+            raise MiqpB200Error(f"miqp_b200_request_stop failed ({rc}): no upload, or plan {k} out of range")
+
+    def stopped(self) -> np.ndarray:
+        """after a run: the last round each stopped plan was searched in (0: before its first node), -1 if it was not stopped"""
+        out = np.zeros(self._batch[0], dtype=np.int32)
+        self._check(self._lib.miqp_b200_stopped(self._h, out.ctypes.data_as(_ip)), "miqp_b200_stopped")
+        return out
 
     def solve_batch_streaming(self, problems, gap_tol=None, time_limit=None, warm=None):
         """Generator of (k, traj, info) in the order the plans finish: upload + run_streaming on a worker thread (the C call

@@ -112,6 +112,10 @@ __global__ void __launch_bounds__(SEL_THREADS) bnb_select_kernel(BnbState st, co
     if (tid == 0) { st.done[s] = 2; st.done_round[s] = round - 1; st.sel_cnt[s] = 0; }
     return;
   }
+  if (st.stop && st.stop[s]) {   // the caller's stop request (miqp_b200_request_stop): the same, after the time limit
+    if (tid == 0) { st.done[s] = 3; st.done_round[s] = round - 1; st.sel_cnt[s] = 0; }
+    return;
+  }
   const DevProb &p = probs[s];
   const long pb = (long)s * st.cap;
   const int KS = st.sel_per_plan;   // stride of sel_idx = largest number of nodes a plan may take per round
@@ -960,17 +964,17 @@ __device__ __noinline__ void expand_solution(const DevProb &p, const double *D, 
   }
 }
 
-// Result of one finished (or stopped) plan s: best bound = smallest bound still open or pruned by the gap rule, into best_bound[s];
-// the incumbent's full column vector into xall (zeros without an incumbent) and its exact trajectory in inc_z.  One block of at
-// most 128 threads per plan; red: shared [128], jeff_s: shared [8 * 64].  bnb_finish_kernel (end of a run) and
-// bnb_harvest_finish_kernel (plans of a streaming run, in the round select marks them finished) run the same code.
-__device__ __forceinline__ void finish_plan(const BnbState &st, int s, const DevProb &p, const double *D, const int *I,
-                                            double *xall, double *best_bound, double *red, int *jeff_s) {
+// Best bound of plan s into best_bound[s]: the smallest bound of its open nodes, of the nsel nodes select has handed to this
+// round's node kernels (sel_idx; 0 once the round's nodes are solved) and of the nodes pruned by the gap rule (pruned_lb), at most
+// the incumbent's value.  Called by every thread of a block of at most 128; red: shared [128].  fmin is exact and does not depend
+// on the order, so the result does not depend on the block size either.
+__device__ __forceinline__ void plan_best_bound(const BnbState &st, int s, int nsel, double *best_bound, double *red) {
   const int tid = threadIdx.x, nt = blockDim.x;
   const long pb = (long)s * st.cap;
   double lb = MQ_INF;
   const int nopen = st.open_cnt[s];
   for (int k = tid; k < nopen; k += nt) lb = fmin(lb, st.bound[pb + st.open_idx[pb + k]]);
+  for (int k = tid; k < nsel; k += nt) lb = fmin(lb, st.bound[pb + st.sel_idx[(long)s * st.sel_per_plan + k]]);
   red[tid] = lb;
   __syncthreads();
   if (tid == 0) {
@@ -981,6 +985,16 @@ __device__ __forceinline__ void finish_plan(const BnbState &st, int s, const Dev
     if (ub < MQ_INF && lb > ub) lb = ub;
     best_bound[s] = lb;
   }
+}
+
+// Result of one finished (or stopped) plan s: best bound = smallest bound still open or pruned by the gap rule, into best_bound[s];
+// the incumbent's full column vector into xall (zeros without an incumbent) and its exact trajectory in inc_z.  One block of at
+// most 128 threads per plan; red: shared [128], jeff_s: shared [8 * 64].  bnb_finish_kernel (end of a run) and
+// bnb_harvest_finish_kernel (plans of a streaming run, in the round select marks them finished) run the same code.
+__device__ __forceinline__ void finish_plan(const BnbState &st, int s, const DevProb &p, const double *D, const int *I,
+                                            double *xall, double *best_bound, double *red, int *jeff_s) {
+  const int tid = threadIdx.x, nt = blockDim.x;
+  plan_best_bound(st, s, 0, best_bound, red);
   const double ub = st.ub[s];
   double *x = xall + p.x_base;
   for (int k = tid; k < p.ncols; k += nt) x[k] = 0.0;
@@ -1204,6 +1218,87 @@ void launch_bnb_harvest_finish(const BnbState &st, const DevProb *probs, const d
 void launch_bnb_harvest_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
                              const double *viol, const double *best_bound, double *out, long rec_stride, cudaStream_t s) {
   if (max_n > 0) bnb_harvest_pack_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, list, n, obj, viol, best_bound, out, rec_stride);
+}
+
+// ---------------------------------------------------------------------------------------
+// anytime runs: harvest of the plans whose incumbent changed since the last delivery.  The host launches the kernels after select
+// and before the node kernels (and before the streaming harvest, whose finish_plan rewrites inc_z with the exact trajectory), so
+// the node kernels of the round that found the incumbents have ended and those of the next round have not begun: (inc_dec, inc_z,
+// ub, inc_uid) are those of the end of that round.  Several improvements of a plan within one round are one delivery, the last.
+// The incumbent is expanded by the code finish_plan runs (expand_solution) in a scratch copy of inc_z, and evaluated by
+// evaluate_list_kernel like at the end of the run: the last delivery of a plan carries the result batch_fetch returns for it.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(SEL_THREADS) bnb_inc_list_kernel(BnbState st, unsigned long long *reported_uid, int *list, int *n,
+                                                                     double *max_viol) {
+  __shared__ int warp_tot[SEL_THREADS / 32];
+  int base_out = 0;
+  for (int base = 0; base < st.count; base += SEL_THREADS) {
+    const int s = base + threadIdx.x;
+    const unsigned long long u = s < st.count ? st.inc_uid[s] : ~0ULL;
+    const int take = (u != ~0ULL && u != reported_uid[s]) ? 1 : 0;
+    int total; const int rank = block_excl_scan(take, warp_tot, total);   // ascending plan order, no atomics: deterministic
+    if (take) { list[base_out + rank] = s; reported_uid[s] = u; max_viol[s] = 0.0; }   // (evaluate_list_kernel takes the maximum into it)
+    base_out += total;
+  }
+  if (threadIdx.x == 0) *n = base_out;
+}
+
+// with_sel: the nodes select handed to this round's node kernels are still unsolved (0 after the last round: they are solved)
+__global__ void bnb_inc_expand_kernel(BnbState st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                                      const int *n, int with_sel, double *zs, double *xall, double *best_bound) {
+  __shared__ double red[128];
+  __shared__ int jeff_s[8 * 64];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const int nh = *n;
+  for (int e = blockIdx.x; e < nh; e += gridDim.x) {
+    const int s = list[e];
+    const DevProb &p = probs[s];
+    plan_best_bound(st, s, with_sel ? st.sel_cnt[s] : 0, best_bound, red);
+    const double *zi = st.inc_z + (long)s * st.zstride;
+    double *z = zs + (long)s * st.zstride;
+    double *x = xall + p.x_base;   // rewritten for every plan by bnb_finish / bnb_harvest_finish before anyone reads it
+    for (int q = tid; q < st.zstride; q += nt) z[q] = zi[q];
+    for (int q = tid; q < p.ncols; q += nt) x[q] = 0.0;
+    __syncthreads();
+    expand_solution(p, dblob, iblob, st.inc_dec + (long)s * st.ndec_stride, z, x, jeff_s);
+    __syncthreads();   // red / jeff_s are reused by the next plan
+  }
+}
+
+__global__ void bnb_inc_pack_kernel(BnbState st, const DevProb *probs, const int *list, const int *n, const double *obj,
+                                    const double *viol, const double *best_bound, const double *zs, int round, double *out,
+                                    long rec_stride) {
+  const int nh = *n;
+  for (int e = blockIdx.x; e < nh; e += gridDim.x) {
+    const int s = list[e];
+    const DevProb &p = probs[s];
+    double *rec = out + (long)e * rec_stride;
+    if (threadIdx.x == 0) {
+      IncRec r;
+      r.objective = obj[s]; r.max_violation = viol[s]; r.ub = st.ub[s]; r.best_bound = best_bound[s];
+      r.inc_uid = st.inc_uid[s]; r.nodes = st.stat_nodes[s]; r.iters = st.stat_iters[s];
+      r.k = s; r.round = round - 1;
+      *reinterpret_cast<IncRec *>(rec) = r;
+    }
+    const double *z = zs + (long)s * st.zstride;
+    const int nz = p.C * p.N * 8;
+    for (int q = threadIdx.x; q < nz; q += blockDim.x) rec[INC_REC_HDR + q] = z[q];
+  }
+}
+
+void launch_bnb_inc_list(const BnbState &st, unsigned long long *reported_uid, int *list, int *n, double *max_viol, cudaStream_t s) {
+  bnb_inc_list_kernel<<<1, SEL_THREADS, 0, s>>>(st, reported_uid, list, n, max_viol);
+}
+
+void launch_bnb_inc_expand(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                           const int *n, int max_n, int with_sel, double *zs, double *xall, double *best_bound, cudaStream_t s) {
+  if (max_n > 0) bnb_inc_expand_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, dblob, iblob, list, n, with_sel, zs, xall, best_bound);
+}
+
+void launch_bnb_inc_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
+                         const double *viol, const double *best_bound, const double *zs, int round, double *out, long rec_stride,
+                         cudaStream_t s) {
+  if (max_n > 0) bnb_inc_pack_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, list, n, obj, viol, best_bound, zs, round, out, rec_stride);
 }
 
 }  // namespace miqp

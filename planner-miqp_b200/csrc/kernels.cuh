@@ -61,7 +61,8 @@ struct BnbState {
   double *ub;           // incumbent objective (inf if none)
   double *cutoff;       // snapshot used by the node kernel in the current round
   double *pruned_lb;
-  int *done;               // 0 searching, 1 finished (frontier exhausted within the gap), 2 stopped at its own time limit
+  int *done;               // 0 searching, 1 finished (frontier exhausted within the gap), 2 stopped at its own time limit,
+                           // 3 stopped on the caller's request (stop)
   int *done_round;         // round in which the plan finished (its solve time = the host's clock at that round)
   const double *tlimit;    // per-plan time limits in seconds (device copy)
   int *lock;
@@ -85,6 +86,8 @@ struct BnbState {
   int *pool_cnt;            // [count]
   // streaming runs (miqp_b200_batch_run_streaming): 1 once a finished plan's result has been harvested; null otherwise
   int *delivered;           // [count]
+  // stop requests of the caller (miqp_b200_request_stop): nonzero = select stops the plan; null while the run has none
+  const unsigned char *stop;   // [count]
 };
 
 // one plan's share of the solution pool, handed to the out-of-line insertion (kernel parameters stay in parameter space)
@@ -143,6 +146,27 @@ void launch_bnb_harvest_finish(const BnbState &st, const DevProb *probs, const d
 // records of the harvested plans into out[e * rec_stride]
 void launch_bnb_harvest_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
                              const double *viol, const double *best_bound, double *out, long rec_stride, cudaStream_t s);
+// ---- anytime runs: per-round harvest of the plans whose incumbent changed -----------------------------------------------------
+// one record per plan, then its trajectory [C][N][8] (a scratch copy of inc_z after expand_solution); records rec_stride doubles apart
+struct IncRec {
+  double objective, max_violation, ub, best_bound;   // evaluate_kernel's values of the expanded incumbent, its search value, best bound
+  unsigned long long inc_uid, nodes, iters;          // incumbent uid, node and interior-point iteration counters so far
+  int k, round;                                      // plan index, round the incumbent was found in
+};
+constexpr int INC_REC_HDR = 8;   // doubles before the trajectory
+static_assert(sizeof(IncRec) <= INC_REC_HDR * sizeof(double), "IncRec outgrew its header");
+// plans whose incumbent changed since the last delivery (inc_uid != reported_uid), ascending, into list[0 .. *n); sets
+// reported_uid and zeroes their max_viol for launch_evaluate_list
+void launch_bnb_inc_list(const BnbState &st, unsigned long long *reported_uid, int *list, int *n, double *max_viol, cudaStream_t s);
+// the listed incumbents expanded in a scratch copy of inc_z (zs[s * zstride]; inc_z is not modified) into xall, and every listed
+// plan's best bound (open nodes, the nodes select handed to this round's node kernels if with_sel, pruned_lb, at most ub) into
+// best_bound
+void launch_bnb_inc_expand(const BnbState &st, const DevProb *probs, const double *dblob, const int *iblob, const int *list,
+                           const int *n, int max_n, int with_sel, double *zs, double *xall, double *best_bound, cudaStream_t s);
+// records of the listed plans into out[e * rec_stride]; `round`: the round whose select has just run
+void launch_bnb_inc_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
+                         const double *viol, const double *best_bound, const double *zs, int round, double *out, long rec_stride,
+                         cudaStream_t s);
 int node_kernel_smem_per_warp(int maxN, int kmax, int ndec_stride);
 int node_kernel_narrow_np(int N);                                  // row stride of the (s, lambda) records of a two-warp team
 int node_kernel_smem_narrow(int N, int kmax, int ndec_stride);   // shared memory of a two-warp team (uniform horizon N)

@@ -9,6 +9,7 @@
 //   * MIP start: decisions of a full column vector (src/cplex_wrapper.cpp:494-639);
 //   * the round loop: launch select + node kernels, poll the number of unfinished plans,
 //     enforce the time limit (tilim, cplexmodel.mod:8-10).
+#include <atomic>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -18,6 +19,7 @@
 #include <string>
 #include <thread>
 #include <algorithm>
+#include <mutex>
 #include <vector>
 
 #include "../../include/miqp_b200.h"
@@ -131,6 +133,22 @@ struct MiqpB200Solver {
   cudaEvent_t ev_hv = nullptr;
   long hv_stride = 0;
   int hv_pending = 0, hv_bound = 0, hv_total = 0;
+  // anytime runs (miqp_b200_batch_run_anytime): callback (null outside such a run), uid of every plan's last delivered incumbent,
+  // harvest list, scratch trajectories, records (device staging and page-locked host copy), records copied but not yet delivered
+  MiqpB200IncumbentFound on_inc = nullptr; void *on_inc_user = nullptr;
+  DevBuf<unsigned long long> ai_reported; DevBuf<int> ai_list; DevBuf<double> ai_z, ai_rec;
+  DVec h_airec;
+  cudaEvent_t ev_ai = nullptr;
+  long ai_stride = 0;
+  int ai_pending = 0;
+  // stop requests (miqp_b200_request_stop, any thread): the host mask of the current upload ([count], empty without an upload)
+  // under stop_mu; stop_dirty once it differs from the device copy, which batch runs upload before their next select
+  std::mutex stop_mu;
+  std::vector<unsigned char> stop_req;
+  std::atomic<bool> stop_dirty{false};
+  std::vector<unsigned char, PinnedAllocator<unsigned char>> h_stop;
+  DevBuf<unsigned char> d_stop;
+  bool stops_on = false;   // the rounds of a batch run (the frontier path never uploads the mask)
 };
 
 namespace {
@@ -220,6 +238,12 @@ void pack_batch(MiqpB200Solver *s, const MiqpB200Problem *problems, int count) {
   }
 }
 
+// relative gap of CPLEX, |best bound - incumbent| / (1e-10 + |incumbent|), with the best bound taken as at most the incumbent
+double rel_gap(double bb, double ub) {
+  const double lb = std::min(bb, ub);
+  return std::fabs(lb - ub) / (1e-10 + std::fabs(ub));
+}
+
 // Solve info of plan k from its device results: batch_fetch and the deliveries of a streaming run build it alike.
 void plan_info(const MiqpB200Solver *s, int k, double ub, unsigned long long incuid, double bb, double obj, double viol, int done,
                int done_round, int overflow, unsigned long long nodes, unsigned long long iters, unsigned long long uncert,
@@ -242,12 +266,12 @@ void plan_info(const MiqpB200Solver *s, int k, double ub, unsigned long long inc
     in.status = MIQP_B200_SUCCESS;
     in.objective = obj;  // re-evaluated on the full vector by evaluate_kernel
     in.max_violation = viol;
-    const double lb = std::min(bb, ub);
-    in.gap = std::fabs(lb - ub) / (1e-10 + std::fabs(ub));
+    in.gap = rel_gap(bb, ub);
     in.proven = (in.gap <= p.gap_tol + 1e-15) ? 1 : 0;
   } else {
-    // no incumbent: the reference reports FAILED_TIMEOUT only for the time-limit status
-    in.status = ((s->timed_out && !done) || done == 2) ? MIQP_B200_FAILED_TIMEOUT : MIQP_B200_FAILED_NO_SOLUT;
+    // no incumbent: the reference reports FAILED_TIMEOUT only for the time-limit status; a plan the caller stopped (done == 3) is
+    // reported alike, so that a caller never retries a plan it stopped itself
+    in.status = ((s->timed_out && !done) || done == 2 || done == 3) ? MIQP_B200_FAILED_TIMEOUT : MIQP_B200_FAILED_NO_SOLUT;
     in.objective = NAN; in.gap = NAN; in.max_violation = NAN;
   }
 }
@@ -314,20 +338,83 @@ void deliver_final(MiqpB200Solver *s) {
   s->hv_held.clear();
 }
 
+// ---- anytime runs ---------------------------------------------------------------------------------------------------------
+// Incumbent harvest of a round (after select, before the streaming harvest): the plans whose incumbent changed are listed, their
+// incumbents expanded in scratch and evaluated, and packed into records; their number lands in ctrl[8], read with the round's ctrl
+// copy.  `round`: the round whose select has just run (the incumbents were found in round - 1); with_sel = 0 after the last round.
+void launch_inc_harvest(MiqpB200Solver *s, int round, int max_n, int with_sel) {
+  int *list = s->ai_list.p, *n = s->b_ctrl.p + 8;
+  launch_bnb_inc_list(s->st, s->ai_reported.p, list, n, s->d_viol.p, s->stream);
+  launch_bnb_inc_expand(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, with_sel, s->ai_z.p, s->d_x.p, s->d_bb.p, s->stream);
+  launch_evaluate_list(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
+  launch_bnb_inc_pack(s->st, s->d_probs.p, list, n, max_n, s->d_obj.p, s->d_viol.p, s->d_bb.p, s->ai_z.p, round, s->ai_rec.p, s->ai_stride,
+                      s->stream);
+  s->fr_launches += max_n > 0 ? 4 : 1;
+}
+
+void copy_inc_records(MiqpB200Solver *s, int n) {
+  CK(cudaMemcpyAsync(s->h_airec.data(), s->ai_rec.p, sizeof(double) * (size_t)n * s->ai_stride, cudaMemcpyDeviceToHost, s->stream));
+  CK(cudaEventRecord(s->ev_ai, s->stream));
+  s->ai_pending = n;
+}
+
+// callbacks of the copied incumbent records, in ascending plan order; a nonzero return stops the plan
+void deliver_incumbents(MiqpB200Solver *s) {
+  if (s->ai_pending == 0) return;
+  CK(cudaEventSynchronize(s->ev_ai));
+  for (int e = 0; e < s->ai_pending; ++e) {
+    const double *rec = s->h_airec.data() + (size_t)e * s->ai_stride;
+    IncRec r;
+    std::memcpy(&r, rec, sizeof r);
+    MiqpB200Incumbent in;
+    std::memset(&in, 0, sizeof in);
+    in.objective = r.objective; in.max_violation = r.max_violation; in.search_value = r.ub;
+    in.best_bound = std::min(r.best_bound, r.ub); in.gap = rel_gap(r.best_bound, r.ub);
+    // the host's clock at the end of the round that found it (of the last round: the end of the run)
+    in.seconds = (r.round >= 1 && r.round < s->fr_rounds) ? s->round_elapsed[r.round - 1] : s->last_seconds;
+    in.round = r.round; in.nodes = (long)r.nodes; in.qp_iters = (long)r.iters; in.uid = r.inc_uid;
+    if (s->on_inc(s->on_inc_user, r.k, rec + INC_REC_HDR, &in)) miqp_b200_request_stop(s, r.k);
+  }
+  s->ai_pending = 0;
+}
+
+// stop requests made since the last upload of the mask go to the device before the next select (batch runs only)
+void upload_stops(MiqpB200Solver *s) {
+  if (!s->stops_on || !s->stop_dirty.load()) return;
+  {
+    std::lock_guard<std::mutex> g(s->stop_mu);
+    s->h_stop.assign(s->stop_req.begin(), s->stop_req.end());
+    s->stop_dirty = false;
+  }
+  const int count = s->st.count;
+  s->d_stop.ensure(count);
+  CK(cudaMemcpyAsync(s->d_stop.p, s->h_stop.data(), (size_t)count, cudaMemcpyHostToDevice, s->stream));
+  s->st.stop = s->d_stop.p;
+}
+
+void clear_stops(MiqpB200Solver *s, int count) {
+  std::lock_guard<std::mutex> g(s->stop_mu);
+  s->stop_req.assign(count, 0);
+  s->stop_dirty = false;
+}
+
 // Select / solve rounds of the uploaded batch, starting from the current device state: until every plan is finished, the time
 // limit or round cap is hit, or `max_rounds_now` rounds have run (< 0: no such cap).  Returns the number of unfinished plans.
 int run_rounds(MiqpB200Solver *s, long max_rounds_now) {
   double tlim = 0.0;
   for (double t : s->time_limits) tlim = std::max(tlim, t);
-  int ctrl[8] = {s->fr_ctrl0, 0, 1, 0, 0, 0, 0, 0};
+  int ctrl[9] = {s->fr_ctrl0, 0, 1, 0, 0, 0, 0, 0, 0};
   long done_now = 0;
   for (;;) {
     if (max_rounds_now >= 0 && done_now >= max_rounds_now) break;
     const long rounds = s->fr_rounds;
     const double el0 = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
     if ((size_t)rounds >= s->round_elapsed.size()) s->round_elapsed.resize(rounds + 64, 0.0);
+    upload_stops(s);
     launch_bnb_select(s->st, s->d_probs.p, (int)rounds + 1, el0, s->stream);
     s->fr_launches += 2;
+    // (before the streaming harvest: its finish_plan rewrites inc_z; no incumbent exists before round 1)
+    if (s->on_inc) launch_inc_harvest(s, (int)rounds + 1, rounds == 0 ? 0 : s->hv_bound, 1);
     if (s->on_done) { launch_harvest(s, 0, rounds == 0 ? s->st.count : s->hv_bound); s->fr_launches += 4; }
     CK(cudaEventRecord(s->evr0, s->stream));
     if (s->n_single > 0) {
@@ -352,15 +439,16 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now) {
       ++s->fr_launches; ++s->fr_node_launches;
     }
     CK(cudaEventRecord(s->evr1, s->stream));
-    if (s->on_done) deliver_pending(s);   // the last round's plans, while this round's node kernels run
+    if (s->on_inc) deliver_incumbents(s);   // the last round's incumbents, while this round's node kernels run, ...
+    if (s->on_done) deliver_pending(s);     // ... then the last round's plans
     ++s->fr_rounds; ++done_now;
     CK(cudaMemcpyAsync(ctrl, s->b_ctrl.p, sizeof ctrl, cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     s->fr_ctrl0 = ctrl[0];
-    if (s->on_done) {
-      s->hv_bound = ctrl[2];   // only plans active in this round can finish in the next select
-      if (ctrl[7] > 0) copy_records(s, ctrl[7]);
-    }
+    // only plans active in this round can finish in the next select, or have found a new incumbent
+    if (s->on_done || s->on_inc) s->hv_bound = ctrl[2];
+    if (s->on_inc && ctrl[8] > 0) copy_inc_records(s, ctrl[8]);
+    if (s->on_done && ctrl[7] > 0) copy_records(s, ctrl[7]);
     float ms = 0.f;
     CK(cudaEventElapsedTime(&ms, s->evr0, s->evr1));
     s->fr_node_ms += ms;
@@ -375,7 +463,7 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now) {
 }
 
 // Start of a search of the uploaded batch, for batch runs and the stepped search (miqp_b200_frontier_*) alike: fresh search
-// state, the run's counters and its clocks.  A streaming run also clears its delivered flags.
+// state, the run's counters and its clocks.  A streaming run also clears its delivered flags, an anytime run its delivered uids.
 void start_run(MiqpB200Solver *s) {
   const int count = s->st.count;
   s->fr_t0 = std::chrono::steady_clock::now();
@@ -390,6 +478,15 @@ void start_run(MiqpB200Solver *s) {
     s->st.delivered = s->hv_delivered.p;
     s->hv_pending = 0; s->hv_total = 0; s->hv_held.clear();
   }
+  if (s->on_inc) {
+    s->ai_stride = (INC_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
+    s->ai_reported.ensure(count); s->ai_list.ensure(count); s->ai_rec.ensure((size_t)count * s->ai_stride);
+    s->ai_z.ensure((size_t)count * s->st.zstride);
+    s->h_airec.resize((size_t)count * s->ai_stride);
+    if (!s->ev_ai) CK(cudaEventCreateWithFlags(&s->ev_ai, cudaEventDisableTiming));
+    CK(cudaMemsetAsync(s->ai_reported.p, 0xff, sizeof(unsigned long long) * count, s->stream));
+    s->ai_pending = 0;
+  }
   CK(cudaEventRecord(s->ev0, s->stream));
   launch_bnb_init(s->st, s->d_probs.p, s->any_warm ? s->d_warm.p : nullptr, s->any_warm ? s->d_haswarm.p : nullptr, s->stream);
   s->fr_rounds = 0; s->fr_ctrl0 = 0;
@@ -402,7 +499,10 @@ void start_run(MiqpB200Solver *s) {
 void finish_run(MiqpB200Solver *s, float *device_ms) {
   const bool streaming = s->on_done != nullptr;
   const int count = s->st.count;
+  if (s->on_inc) deliver_incumbents(s);
   if (streaming) deliver_pending(s);
+  // anytime run: the incumbents found in the last round, before bnb_finish rewrites inc_z
+  if (s->on_inc) launch_inc_harvest(s, (int)s->fr_rounds + 1, s->fr_rounds == 0 ? 0 : s->hv_bound, 0);
   launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
   if (!streaming) {
     CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
@@ -415,6 +515,8 @@ void finish_run(MiqpB200Solver *s, float *device_ms) {
   }
   s->fr_launches += 2;
   CK(cudaGetLastError());
+  int n_inc = 0;
+  if (s->on_inc) CK(cudaMemcpyAsync(&n_inc, s->b_ctrl.p + 8, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
   CK(cudaEventRecord(s->ev1, s->stream));
   CK(cudaStreamSynchronize(s->stream));
   float total_ms = 0.f;
@@ -424,6 +526,10 @@ void finish_run(MiqpB200Solver *s, float *device_ms) {
   s->stats.launches = s->fr_launches; s->stats.node_kernel_launches = s->fr_node_launches; s->stats.rounds = s->fr_rounds;
   s->stats.node_kernel_ms = s->fr_node_ms; s->stats.total_ms = total_ms;
   s->ran = true;
+  if (n_inc > 0) {   // (a copy after the run's last event: the run's device time stays that of the search)
+    copy_inc_records(s, n_inc);
+    deliver_incumbents(s);
+  }
   if (streaming) deliver_final(s);
 }
 
@@ -576,7 +682,7 @@ void setup_bnb(MiqpB200Solver *s) {
   s->b_overflow.ensure(count); st.overflow = s->b_overflow.p;
   s->b_work.ensure(st.work_cap); st.work = s->b_work.p;
   s->b_work2.ensure(st.work_cap); st.work2 = s->b_work2.p;
-  s->b_ctrl.ensure(8);
+  s->b_ctrl.ensure(9);
   s->b_prof.ensure(256); st.prof = s->b_prof.p;
   s->b_dbg.ensure((size_t)(1024 + 8) * 512); st.dbg = s->b_dbg.p;
   st.work_cnt = s->b_ctrl.p; st.work_next = s->b_ctrl.p + 1; st.active = s->b_ctrl.p + 2; st.err = s->b_ctrl.p + 3;
@@ -695,6 +801,7 @@ void miqp_b200_destroy(MiqpB200Solver *s) {
   if (s->mark[1]) cudaEventDestroy(s->mark[1]);
   if (s->evr1) cudaEventDestroy(s->evr1);
   if (s->ev_hv) cudaEventDestroy(s->ev_hv);
+  if (s->ev_ai) cudaEventDestroy(s->ev_ai);
   if (s->stream) cudaStreamDestroy(s->stream);
   delete s;
 }
@@ -714,7 +821,7 @@ int miqp_b200_assemble(MiqpB200Solver *s, const MiqpB200Problem *p, long *rowptr
   try {
     CK(cudaSetDevice(s->opt.device));
     pack_batch(s, p, 1);
-    s->uploaded = false;
+    s->uploaded = false; clear_stops(s, 0);
     upload_packed(s);
     const long rows = s->pk.total_rows, nnz = s->pk.total_nnz;
     s->a_rowptr.ensure(rows + 1); s->a_cols.ensure(std::max<long>(nnz, 1)); s->a_vals.ensure(std::max<long>(nnz, 1));
@@ -748,7 +855,7 @@ int miqp_b200_assemble_batch(MiqpB200Solver *s, const MiqpB200Problem *problems,
   try {
     CK(cudaSetDevice(s->opt.device));
     pack_batch(s, problems, count);
-    s->uploaded = false;
+    s->uploaded = false; clear_stops(s, 0);
     upload_packed(s);
     const long rows = s->pk.total_rows, nnz = s->pk.total_nnz;
     // every plan owns nrows + 1 row pointers and its own non-zero counter (formulation.cu:assemble_rows_kernel)
@@ -799,7 +906,7 @@ int miqp_b200_evaluate(MiqpB200Solver *s, const MiqpB200Problem *p, const double
   try {
     CK(cudaSetDevice(s->opt.device));
     pack_batch(s, p, 1);
-    s->uploaded = false;
+    s->uploaded = false; clear_stops(s, 0);
     upload_packed(s);
     s->d_x.ensure(s->pk.total_cols); s->d_viol.ensure(1); s->d_obj.ensure(1);
     CK(cudaMemcpyAsync(s->d_x.p, x, sizeof(double) * s->pk.total_cols, cudaMemcpyHostToDevice, s->stream));
@@ -826,6 +933,7 @@ int miqp_b200_batch_upload(MiqpB200Solver *s, const MiqpB200Problem *problems, i
   try {
     CK(cudaSetDevice(s->opt.device));
     s->uploaded = false; s->ran = false;
+    clear_stops(s, 0);
     const auto tp0 = std::chrono::steady_clock::now();
     pack_batch(s, problems, count);
     const auto tp1 = std::chrono::steady_clock::now();
@@ -852,6 +960,7 @@ int miqp_b200_batch_upload(MiqpB200Solver *s, const MiqpB200Problem *problems, i
     s->stats.pack_ms = std::chrono::duration<double, std::milli>(tp1 - tp0).count();
     s->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp1).count();
     s->uploaded = true;
+    clear_stops(s, count);
   } catch (const std::invalid_argument &ex) {
     return fail(s, MIQP_B200_ERR_ARG, ex.what());
   } catch (const std::exception &ex) {
@@ -879,6 +988,7 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
     for (int k = 0; k < count; ++k) { const DevProb &p = s->pk.probs[k]; prev[k] = Shape{p.C, p.N, p.R, p.O, p.E, p.L}; }
     CK(cudaStreamSynchronize(s->stream));
     s->uploaded = false; s->ran = false;
+    clear_stops(s, 0);
     const auto tp0 = std::chrono::steady_clock::now();
     pack_batch(s, problems, count);
     const auto tp1 = std::chrono::steady_clock::now();
@@ -900,6 +1010,7 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
     s->stats.pack_ms = std::chrono::duration<double, std::milli>(tp1 - tp0).count();
     s->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp1).count();
     s->uploaded = true;
+    clear_stops(s, count);
   } catch (const std::invalid_argument &ex) {
     return fail(s, MIQP_B200_ERR_ARG, ex.what());
   } catch (const std::exception &ex) {
@@ -909,12 +1020,19 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
 }
 
 // One search of the uploaded batch; a streaming run (s->on_done set) also harvests every plan in the round select marks it
-// finished and hands it to the callback.  Both compute the same results.
+// finished and hands it to the callback, an anytime run (s->on_inc set) every new incumbent.  All compute the same results.  Stop
+// requests (miqp_b200_request_stop) apply to every batch run and are cleared when it ends.
 static int run_batch(MiqpB200Solver *s, float *device_ms) {
-  struct Reset {   // the delivered flags are seen by the kernels of streaming runs only
+  struct Reset {   // the delivered flags and the stop mask are seen by the kernels of the runs that use them only
     MiqpB200Solver *s;
-    ~Reset() { s->st.delivered = nullptr; s->on_done = nullptr; s->on_done_user = nullptr; s->hv_pending = 0; s->hv_held.clear(); }
+    ~Reset() {
+      s->st.delivered = nullptr; s->on_done = nullptr; s->on_done_user = nullptr; s->hv_pending = 0; s->hv_held.clear();
+      s->on_inc = nullptr; s->on_inc_user = nullptr; s->ai_pending = 0;
+      s->st.stop = nullptr; s->stops_on = false;
+      clear_stops(s, s->st.count);
+    }
   } reset{s};
+  s->stops_on = true;
   try {
     CK(cudaSetDevice(s->opt.device));
     start_run(s);
@@ -938,6 +1056,45 @@ int miqp_b200_batch_run_streaming(MiqpB200Solver *s, MiqpB200PlanDone on_done, v
   if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "batch_run_streaming without batch_upload");
   s->on_done = on_done; s->on_done_user = user;
   return run_batch(s, device_ms);
+}
+
+int miqp_b200_batch_run_anytime(MiqpB200Solver *s, MiqpB200IncumbentFound on_incumbent, MiqpB200PlanDone on_done, void *user,
+                                float *device_ms) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (!on_incumbent) return fail(s, MIQP_B200_ERR_ARG, "batch_run_anytime without an incumbent callback");
+  if (!s->uploaded) return fail(s, MIQP_B200_ERR_ARG, "batch_run_anytime without batch_upload");
+  s->on_inc = on_incumbent; s->on_inc_user = user;
+  s->on_done = on_done; s->on_done_user = user;
+  return run_batch(s, device_ms);
+}
+
+// Thread-safe: it touches only the host mask under its mutex (and sets no last_error, which belongs to the solver's thread).
+int miqp_b200_request_stop(MiqpB200Solver *s, int k) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  std::lock_guard<std::mutex> g(s->stop_mu);
+  const int count = (int)s->stop_req.size();
+  if (count == 0 || k < -1 || k >= count) return MIQP_B200_ERR_ARG;   // no upload, or no such plan
+  if (k < 0) std::fill(s->stop_req.begin(), s->stop_req.end(), (unsigned char)1);
+  else s->stop_req[k] = 1;
+  s->stop_dirty = true;
+  return MIQP_B200_OK;
+}
+
+int miqp_b200_stopped(MiqpB200Solver *s, int *round) {
+  if (!s || !round) return MIQP_B200_ERR_ARG;
+  if (!s->ran) return fail(s, MIQP_B200_ERR_ARG, "stopped: no results of a batch run on this solver");
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    const int count = s->st.count;
+    s->h_done.resize(count); s->h_doneround.resize(count);
+    CK(cudaMemcpyAsync(s->h_done.data(), s->st.done, sizeof(int) * count, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->h_doneround.data(), s->st.done_round, sizeof(int) * count, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    for (int k = 0; k < count; ++k) round[k] = s->h_done[k] == 3 ? s->h_doneround[k] : -1;
+  } catch (const std::exception &ex) {
+    return fail(s, MIQP_B200_ERR_CUDA, ex.what());
+  }
+  return MIQP_B200_OK;
 }
 
 static int fetch_results(MiqpB200Solver *s, double *const *x_out, double *const *traj_out, MiqpB200SolveInfo *infos);
