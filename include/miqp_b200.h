@@ -41,6 +41,10 @@
  * miqp_b200_pool_export / _merge   (no counterpart) the pool of a plan whose frontier is sharded
  *                                  over GPUs: every rank's pool packed for an all-gather, and
  *                                  the pool of the union of the ranks' leaves built from them
+ * miqp_b200_frontier_inc_export /  CPLEX's incumbent callback and Aborter for a plan whose frontier
+ *   _frontier_inc_merge            is sharded over GPUs: every rank's incumbents and stop requests
+ *                                  packed for an all-gather at each exchange, the best of all ranks
+ *                                  handed to a callback and the stops applied on every rank
  */
 #ifndef MIQP_B200_H
 #define MIQP_B200_H
@@ -223,7 +227,10 @@ int miqp_b200_batch_run_anytime(MiqpB200Solver *s, MiqpB200IncumbentFound on_inc
  * apply from round 1.  A callback runs after the next round's select has been launched, so a stop it returns for a record found
  * in round r takes effect at the select of round r + 3: the plan is still searched in rounds r + 1 and r + 2.  A stopped plan
  * ends like one that hit its time limit: SUCCESS with its incumbent (proven from the gap at that point), FAILED_TIMEOUT without
- * one.  Requests are cleared when a run ends and at every upload.  The frontier path (frontier_*) ignores them.  Stopping plans
+ * one.  Requests are cleared when a run ends (batch runs, frontier_finish) and at every upload.  The frontier path (frontier_*)
+ * applies them only through frontier_inc_export / frontier_inc_merge: a request travels with this rank's next export and stops
+ * the plan on every rank from the frontier_rounds after that exchange's merge; a frontier search without those calls ignores
+ * requests.  Stopping plans
  * changes how many nodes the other plans take per round, so their search order changes; it stays deterministic for the same stop
  * rounds.  Does not set last_error.  ERR_ARG: no upload or k out of range. */
 int miqp_b200_request_stop(MiqpB200Solver *s, int k /* -1: every plan */);
@@ -258,6 +265,35 @@ int miqp_b200_frontier_ub_device(MiqpB200Solver *s, void **ub, int *count);
 int miqp_b200_frontier_get_ub(MiqpB200Solver *s, double *ub /* [count] */);
 int miqp_b200_frontier_tighten(MiqpB200Solver *s, const double *ub /* [count] */);
 int miqp_b200_frontier_finish(MiqpB200Solver *s, float *device_ms);
+
+/* Anytime deliveries and stops on the frontier path (opt-in; a search that does not call these computes what it did without
+ * them).  At each exchange every rank calls, in this order: frontier_rounds, frontier_inc_export, a MAX all-reduce of n_records,
+ * an all-gather of every rank's first summary_bytes + n_max x record_bytes bytes of the export (rank order), frontier_inc_merge,
+ * and then the incumbent-objective exchange (frontier_get_ub / frontier_tighten or the NCCL all-reduce on frontier_ub_device).
+ * The export MUST precede that exchange: only frontier_tighten lowers the incumbent objective other than a find of this rank, so a
+ * record's search value is then this rank's own; the export has synchronised the solver's stream when it returns.  One more
+ * export / gather / merge before frontier_finish delivers the last rounds: the last delivery of a plan with an incumbent is the
+ * combined result (least objective over the ranks, lowest rank among ties).
+ * export: packs into a solver-owned device buffer (*dev; summary_bytes + count x record_bytes bytes, valid until the next export,
+ * upload or destroy): a summary (64-byte header with magic/version, count, record stride, n_records, this rank's rounds and a hash
+ * of every plan's C, N, R, O, L, E, ncols; per plan the best bound of this rank's share, its node and interior-point iteration
+ * counters and this rank's stop request), then *n_records records (the incumbents whose uid changed since the last export of this
+ * run, expanded and evaluated as at the end of a run; the first export of a run reports every incumbent), ascending plan order.
+ * merge: `gathered` holds `world` blocks of summary_bytes + n_max x record_bytes bytes (host or device memory).  Per plan the best
+ * record by (objective, rank) is delivered if its key is below the key last delivered for the plan in this run; the merged stop
+ * requests apply on every rank from the next frontier_rounds.  Every rank computes the same deliveries and stops, with or without
+ * a callback.  `cb` (may be NULL) is called per delivery in ascending k, on the calling thread; `traj` ([C][N][8]) and `inc` are
+ * valid during the call only: objective, max_violation, uid of the winning record, search_value = the winning rank's incumbent
+ * value, best_bound = least over the ranks' bounds and at most the objective, gap from it as in MiqpB200SolveInfo, round = the
+ * winning rank's rounds at its export (the incumbent was found in or before it), nodes / qp_iters summed over the ranks, seconds =
+ * this rank's host clock since frontier_start.  A nonzero return is miqp_b200_request_stop(s, k): it travels with this rank's
+ * next export, so the plan is searched for one more exchange interval on every rank.  *n_new (may be NULL): the deliveries.
+ * ERR_ARG, nothing changed: no frontier_start (or after frontier_finish), world < 1, n_max outside 0..count, a block whose header
+ * does not match this solver's upload, or one that holds more than n_max records. */
+typedef int (*MiqpB200FrontierIncumbentFound)(void *user, int k, int rank, const double *traj, const MiqpB200Incumbent *inc);
+int miqp_b200_frontier_inc_export(MiqpB200Solver *s, void **dev, size_t *summary_bytes, size_t *record_bytes, int *n_records);
+int miqp_b200_frontier_inc_merge(MiqpB200Solver *s, const void *gathered, int world, int n_max,
+                                 MiqpB200FrontierIncumbentFound cb /* may be NULL */, void *user, int *n_new);
 
 /* Solution pool (CPLEX's pool, counted by SolutionProperties.NrSolutionPool): up to `capacity` distinct integer-feasible
  * completions per plan that the search solved, best first.  0 = off (default); 1..64; takes effect at the next upload.

@@ -31,6 +31,7 @@ DECLARED_SYMBOLS = [
     "miqp_b200_set_solution_pool", "miqp_b200_pool_sizes", "miqp_b200_pool_fetch",
     "miqp_b200_batch_run_streaming", "miqp_b200_pool_export", "miqp_b200_pool_merge",
     "miqp_b200_batch_run_anytime", "miqp_b200_request_stop", "miqp_b200_stopped",
+    "miqp_b200_frontier_inc_export", "miqp_b200_frontier_inc_merge",
 ]
 
 
@@ -99,6 +100,8 @@ class CIncumbent(C.Structure):
 
 # int (*MiqpB200IncumbentFound)(void *user, int k, const double *traj, const MiqpB200Incumbent *inc)
 INCUMBENT_FOUND = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, _dp, C.POINTER(CIncumbent))
+# int (*MiqpB200FrontierIncumbentFound)(void *user, int k, int rank, const double *traj, const MiqpB200Incumbent *inc)
+FRONTIER_INCUMBENT_FOUND = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_int, _dp, C.POINTER(CIncumbent))
 
 
 class CRunStats(C.Structure):
@@ -128,7 +131,9 @@ class SolveInfo:
 class Incumbent:
     """An improved incumbent of an anytime run (miqp_b200_batch_run_anytime): objective and max violation of its full column
     vector (device-evaluated), the value the search stored, the plan's best bound and gap when the round that found it ended,
-    the host clock then (seconds from the start of the run), that round, and the plan's node and iteration counters so far."""
+    the host clock then (seconds from the start of the run), that round, and the plan's node and iteration counters so far.
+    A delivery of a frontier-sharded search (Solver.frontier_inc_merge) also names the rank that found it; its bound and
+    counters are those of all ranks (-1: an anytime run of one solver)."""
     objective: float
     max_violation: float
     search_value: float
@@ -139,6 +144,7 @@ class Incumbent:
     nodes: int
     qp_iters: int
     uid: int
+    rank: int = -1
 
 
 @dataclass
@@ -205,6 +211,8 @@ def load_library():
     lib.miqp_b200_batch_run_anytime.argtypes = [C.c_void_p, INCUMBENT_FOUND, PLAN_DONE, C.c_void_p, C.POINTER(C.c_float)]
     lib.miqp_b200_request_stop.argtypes = [C.c_void_p, C.c_int]
     lib.miqp_b200_stopped.argtypes = [C.c_void_p, _ip]
+    lib.miqp_b200_frontier_inc_export.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t), _ip]
+    lib.miqp_b200_frontier_inc_merge.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, FRONTIER_INCUMBENT_FOUND, C.c_void_p, _ip]
     _lib = lib
     return lib
 
@@ -616,7 +624,9 @@ class Solver:
 
     def request_stop(self, k: int = -1):
         """stop plan k (-1: every plan) of the uploaded batch at the next select of a run; safe from any thread and from the
-        callbacks of run_anytime / run_streaming.  Requests are cleared when a run ends and at every upload."""
+        callbacks of run_anytime / run_streaming.  Requests are cleared when a run ends and at every upload.  A frontier search
+        applies them only with incumbent deliveries (solve_frontier_sharded(on_incumbent=...)): on every rank, from the
+        exchange after the request."""
         rc = self._lib.miqp_b200_request_stop(self._h, int(k))
         if rc != 0:
             raise MiqpB200Error(f"miqp_b200_request_stop failed ({rc}): no upload, or plan {k} out of range")
@@ -686,6 +696,54 @@ class Solver:
         self._lib.miqp_b200_frontier_finish.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         self._check(self._lib.miqp_b200_frontier_finish(self._h, C.byref(ms)), "miqp_b200_frontier_finish")
         return ms.value
+
+    def frontier_inc_export(self):
+        """this rank's incumbents and summary packed for the all-gather of an exchange (miqp_b200_frontier_inc_export; after
+        frontier_rounds, before the incumbent-objective exchange): (buffer, summary_bytes, record_bytes, n_records).  The buffer
+        is a torch.uint8 CUDA tensor that views the solver's export buffer without a copy (summary_bytes + count x record_bytes
+        bytes, the first n_records records valid); valid until the next export, upload or close."""
+        import torch
+        ptr, sb, rb, n = C.c_void_p(), C.c_size_t(), C.c_size_t(), C.c_int()
+        self._check(self._lib.miqp_b200_frontier_inc_export(self._h, C.byref(ptr), C.byref(sb), C.byref(rb), C.byref(n)),
+                    "miqp_b200_frontier_inc_export")
+        nbytes = sb.value + self._batch[0] * rb.value
+        buf = torch.as_tensor(_DevView(ptr.value, nbytes, "|u1"), device=torch.device("cuda", self._device))
+        return buf, sb.value, rb.value, n.value
+
+    def frontier_inc_merge(self, gathered, world: int, n_max: int, on_incumbent=None) -> int:
+        """merge of `world` blocks of summary_bytes + n_max x record_bytes bytes, back to back in rank order in `gathered` (a CPU
+        or CUDA tensor; miqp_b200_frontier_inc_merge): on_incumbent(k, traj, inc) for every plan whose best incumbent over the
+        ranks improved (ascending k; traj a copy [C][N][8], inc an Incumbent with its rank), and the stop requests of all ranks
+        applied from the next frontier_rounds.  A truthy return stops plan k on every rank after the next exchange.  An exception
+        raised by on_incumbent stops the calls to it; the merge completes and the exception is raised here.  Returns the
+        number of deliveries (the same on every rank)."""
+        import torch
+        g = gathered.contiguous()
+        if g.is_cuda:
+            torch.cuda.synchronize(g.device)      # the C call reads it on the solver's own stream
+        shapes = self._shapes
+        failed = []
+
+        def cb(_user, k, rank, traj, inc):
+            if failed:
+                return 0
+            try:
+                c, nn = shapes[k]
+                t = np.ctypeslib.as_array(traj, shape=(c * nn * 8,)).reshape(c, nn, 8).copy()
+                i = inc.contents
+                return 1 if on_incumbent(k, t, Incumbent(i.objective, i.max_violation, i.search_value, i.best_bound, i.gap, i.seconds,
+                                                         i.round, i.nodes, i.qp_iters, i.uid, rank)) else 0
+            except BaseException as ex:   # ctypes would print and drop it
+                failed.append(ex)
+                return 0
+
+        func = FRONTIER_INCUMBENT_FOUND(cb) if on_incumbent is not None else FRONTIER_INCUMBENT_FOUND()
+        n = C.c_int()
+        rc = self._lib.miqp_b200_frontier_inc_merge(self._h, C.c_void_p(g.data_ptr()), int(world), int(n_max), func, None, C.byref(n))
+        if failed:
+            raise failed[0]
+        self._check(rc, "miqp_b200_frontier_inc_merge")
+        return n.value
 
     def mark(self, which: int):
         self._lib.miqp_b200_mark.argtypes = [C.c_void_p, C.c_int]

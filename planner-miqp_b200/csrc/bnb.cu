@@ -1301,4 +1301,107 @@ void launch_bnb_inc_pack(const BnbState &st, const DevProb *probs, const int *li
   if (max_n > 0) bnb_inc_pack_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(st, probs, list, n, obj, viol, best_bound, zs, round, out, rec_stride);
 }
 
+// ---------------------------------------------------------------------------------------
+// frontier sharding with incumbent deliveries: every rank exports its summary and the records of its changed incumbents (the
+// anytime harvest above), the exports are all-gathered, and every rank merges the same bytes, so every rank computes the same
+// deliveries, keys and stop mask.  The winner rule is that of the final combine (sharding.py): least objective, lowest rank.
+// ---------------------------------------------------------------------------------------
+__global__ void bnb_frontier_inc_summary_kernel(BnbState st, unsigned char *block, FrontierIncLayout lay) {
+  __shared__ double red[128];
+  const int s = blockIdx.x;
+  // (the export runs between frontier_rounds calls: the nodes select handed out are solved)
+  plan_best_bound(st, s, 0, reinterpret_cast<double *>(block + lay.off_bb), red);
+  if (threadIdx.x == 0) {
+    reinterpret_cast<unsigned long long *>(block + lay.off_nodes)[s] = st.stat_nodes[s];
+    reinterpret_cast<unsigned long long *>(block + lay.off_iters)[s] = st.stat_iters[s];
+  }
+}
+
+void launch_frontier_inc_summary(const BnbState &st, unsigned char *block, const FrontierIncLayout &lay, cudaStream_t s) {
+  bnb_frontier_inc_summary_kernel<<<st.count, 128, 0, s>>>(st, block, lay);
+}
+
+// one block: a thread per plan, every rank's record of it found by bisection (records ascend by plan), the deliveries listed in
+// ascending plan order by block_excl_scan (no atomics: the same on every rank)
+__global__ void __launch_bounds__(SEL_THREADS) bnb_frontier_inc_merge_kernel(BnbState st, const unsigned char *g, FrontierIncLayout lay,
+                                                                             long block_bytes, int world, double *key_obj, int *key_rank,
+                                                                             unsigned char *stop_out, int *list, int2 *src, int *n,
+                                                                             double *out, long out_stride) {
+  __shared__ int warp_tot[SEL_THREADS / 32];
+  int base_out = 0;
+  for (int base = 0; base < st.count; base += SEL_THREADS) {
+    const int s = base + threadIdx.x;
+    int take = 0, best_r = -1, best_e = -1;
+    double best_obj = MQ_INF, bb = MQ_INF;
+    unsigned long long nodes = 0, iters = 0;
+    if (s < st.count) {
+      unsigned char stop = 0;
+      for (int r = 0; r < world; ++r) {
+        const unsigned char *blk = g + (long)r * block_bytes;
+        const FrontierIncHeader *h = reinterpret_cast<const FrontierIncHeader *>(blk);
+        bb = fmin(bb, reinterpret_cast<const double *>(blk + lay.off_bb)[s]);
+        nodes += reinterpret_cast<const unsigned long long *>(blk + lay.off_nodes)[s];
+        iters += reinterpret_cast<const unsigned long long *>(blk + lay.off_iters)[s];
+        stop |= blk[lay.off_stop + s];
+        const double *recs = reinterpret_cast<const double *>(blk + lay.summary_bytes);
+        int lo = 0, hi = h->n_records;
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (reinterpret_cast<const IncRec *>(recs + (long)mid * lay.rec_stride)->k < s) lo = mid + 1; else hi = mid;
+        }
+        if (lo < h->n_records) {
+          const IncRec *rec = reinterpret_cast<const IncRec *>(recs + (long)lo * lay.rec_stride);
+          // ranks ascend: a tie keeps the lower rank
+          if (rec->k == s && (best_r < 0 || rec->objective < best_obj)) { best_obj = rec->objective; best_r = r; best_e = lo; }
+        }
+      }
+      stop_out[s] = stop ? 1 : 0;
+      const int kr = key_rank[s];
+      take = best_r >= 0 && (kr < 0 || best_obj < key_obj[s] || (best_obj == key_obj[s] && best_r < kr)) ? 1 : 0;
+    }
+    int total; const int rank = block_excl_scan(take, warp_tot, total);
+    if (take) {
+      const int e = base_out + rank;
+      list[e] = s; src[e] = make_int2(best_r, best_e);
+      key_obj[s] = best_obj; key_rank[s] = best_r;
+      const double *recs = reinterpret_cast<const double *>(g + (long)best_r * block_bytes + lay.summary_bytes);
+      FrontierIncOut o;
+      o.r = *reinterpret_cast<const IncRec *>(recs + (long)best_e * lay.rec_stride);
+      o.r.best_bound = fmin(bb, o.r.objective);   // the final combine's bound: least over the ranks, at most the incumbent
+      o.r.nodes = nodes; o.r.iters = iters;
+      o.rank = best_r; o.pad_ = 0;
+      *reinterpret_cast<FrontierIncOut *>(out + (long)e * out_stride) = o;
+    }
+    base_out += total;
+  }
+  if (threadIdx.x == 0) *n = base_out;
+}
+
+__global__ void bnb_frontier_inc_pack_kernel(const DevProb *probs, const unsigned char *g, FrontierIncLayout lay, long block_bytes,
+                                             const int *list, const int2 *src, const int *n, double *out, long out_stride) {
+  const int nh = *n;
+  for (int e = blockIdx.x; e < nh; e += gridDim.x) {
+    const DevProb &p = probs[list[e]];
+    const int2 w = src[e];
+    const double *rec = reinterpret_cast<const double *>(g + (long)w.x * block_bytes + lay.summary_bytes) + (long)w.y * lay.rec_stride;
+    const int nz = p.C * p.N * 8;
+    for (int q = threadIdx.x; q < nz; q += blockDim.x) out[(long)e * out_stride + FI_OUT_HDR + q] = rec[INC_REC_HDR + q];
+  }
+}
+
+void launch_frontier_inc_merge(const BnbState &st, const unsigned char *g, const FrontierIncLayout &lay, long block_bytes, int world,
+                               double *key_obj, int *key_rank, unsigned char *stop_out, int *list, int2 *src, int *n, double *out,
+                               long out_stride, cudaStream_t s) {
+  bnb_frontier_inc_merge_kernel<<<1, SEL_THREADS, 0, s>>>(st, g, lay, block_bytes, world, key_obj, key_rank, stop_out, list, src, n, out,
+                                                          out_stride);
+}
+
+void launch_frontier_inc_pack(const DevProb *probs, const unsigned char *g, const FrontierIncLayout &lay,
+                              long block_bytes, const int *list, const int2 *src, const int *n, int max_n, double *out, long out_stride,
+                              cudaStream_t s) {
+  if (max_n > 0)
+    bnb_frontier_inc_pack_kernel<<<(max_n < HARVEST_GRID ? max_n : HARVEST_GRID), 128, 0, s>>>(probs, g, lay, block_bytes, list, src, n, out,
+                                                                                               out_stride);
+}
+
 }  // namespace miqp

@@ -167,6 +167,41 @@ void launch_bnb_inc_expand(const BnbState &st, const DevProb *probs, const doubl
 void launch_bnb_inc_pack(const BnbState &st, const DevProb *probs, const int *list, const int *n, int max_n, const double *obj,
                          const double *viol, const double *best_bound, const double *zs, int round, double *out, long rec_stride,
                          cudaStream_t s);
+// ---- frontier sharding with incumbent deliveries (miqp_b200_frontier_inc_export / _merge) -----------------------------------
+// One rank's export block: a 64-byte header, then per plan its best bound (double), node and interior-point iteration counters
+// (unsigned long long) and stop request (byte), each section 16-byte aligned (together: the summary), then n_records records of
+// rec_stride doubles, IncRec + trajectory [C][N][8] as launch_bnb_inc_pack writes them, in ascending plan order.
+struct FrontierIncHeader {
+  unsigned magic, version;
+  int count, n_records;
+  long rec_stride;                 // doubles per record
+  long rounds;                     // rounds this rank had run at the export
+  unsigned long long shape_hash;   // FNV-1a over (C, N, R, O, L, E, ncols) of every plan, as the pool export
+  unsigned char pad[24];
+};
+static_assert(sizeof(FrontierIncHeader) == 64, "frontier export header size");
+struct FrontierIncLayout { long off_bb, off_nodes, off_iters, off_stop, summary_bytes, rec_stride; };
+// one merged delivery: the winning record with the merged best bound and the counters summed over the ranks, and the winner's
+// rank; then its trajectory.  Records FI_OUT_HDR + C * N * 8 doubles apart (out_stride)
+struct FrontierIncOut {
+  IncRec r;
+  int rank, pad_;
+};
+constexpr int FI_OUT_HDR = 10;   // doubles before the trajectory
+static_assert(sizeof(FrontierIncOut) <= FI_OUT_HDR * sizeof(double), "FrontierIncOut outgrew its header");
+// summary of this rank into block (best bounds with no unsolved selected nodes, counters); the header and stop bytes come from
+// the host
+void launch_frontier_inc_summary(const BnbState &st, unsigned char *block, const FrontierIncLayout &lay, cudaStream_t s);
+// merge of `world` blocks block_bytes apart at g (device memory): per plan the best record by (objective, rank); delivered, in
+// ascending plan order into list / out (headers) / src (rank, record), if its key is below (key_obj, key_rank) (key_rank < 0:
+// nothing delivered yet), which it then becomes.  stop_out = OR of the ranks' stop bytes.  *n = deliveries.
+void launch_frontier_inc_merge(const BnbState &st, const unsigned char *g, const FrontierIncLayout &lay, long block_bytes, int world,
+                               double *key_obj, int *key_rank, unsigned char *stop_out, int *list, int2 *src, int *n, double *out,
+                               long out_stride, cudaStream_t s);
+// trajectories of the deliveries into out[e * out_stride + FI_OUT_HDR]
+void launch_frontier_inc_pack(const DevProb *probs, const unsigned char *g, const FrontierIncLayout &lay,
+                              long block_bytes, const int *list, const int2 *src, const int *n, int max_n, double *out, long out_stride,
+                              cudaStream_t s);
 int node_kernel_smem_per_warp(int maxN, int kmax, int ndec_stride);
 int node_kernel_narrow_np(int N);                                  // row stride of the (s, lambda) records of a two-warp team
 int node_kernel_smem_narrow(int N, int kmax, int ndec_stride);   // shared memory of a two-warp team (uniform horizon N)

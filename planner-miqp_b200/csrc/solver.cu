@@ -12,6 +12,7 @@
 #include <atomic>
 #include <chrono>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -149,6 +150,13 @@ struct MiqpB200Solver {
   std::vector<unsigned char, PinnedAllocator<unsigned char>> h_stop;
   DevBuf<unsigned char> d_stop;
   bool stops_on = false;   // the rounds of a batch run (the frontier path never uploads the mask)
+  // frontier sharding with incumbent deliveries (miqp_b200_frontier_inc_export / _merge): export block, device copy of a merge
+  // input from elsewhere, key (objective, rank) of every plan's last delivery, merge list and records (device, page-locked host)
+  DevBuf<unsigned char> fi_export, fi_gathered;
+  DevBuf<double> fi_key_obj, fi_out; DevBuf<int> fi_key_rank, fi_list, fi_n; DevBuf<int2> fi_src;
+  DVec h_fiout;
+  bool fi_started = false;    // between frontier_start and frontier_finish
+  bool fi_reported = false;   // ai_reported initialised for this run (at its first export)
 };
 
 namespace {
@@ -342,12 +350,20 @@ void deliver_final(MiqpB200Solver *s) {
 // Incumbent harvest of a round (after select, before the streaming harvest): the plans whose incumbent changed are listed, their
 // incumbents expanded in scratch and evaluated, and packed into records; their number lands in ctrl[8], read with the round's ctrl
 // copy.  `round`: the round whose select has just run (the incumbents were found in round - 1); with_sel = 0 after the last round.
-void launch_inc_harvest(MiqpB200Solver *s, int round, int max_n, int with_sel) {
+// buffers of the incumbent harvest (anytime runs and frontier exports)
+void ensure_inc_harvest(MiqpB200Solver *s) {
+  const int count = s->st.count;
+  s->ai_stride = (INC_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
+  s->ai_reported.ensure(count); s->ai_list.ensure(count);
+  s->ai_z.ensure((size_t)count * s->st.zstride);
+}
+
+void launch_inc_harvest(MiqpB200Solver *s, int round, int max_n, int with_sel, double *out) {
   int *list = s->ai_list.p, *n = s->b_ctrl.p + 8;
   launch_bnb_inc_list(s->st, s->ai_reported.p, list, n, s->d_viol.p, s->stream);
   launch_bnb_inc_expand(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, with_sel, s->ai_z.p, s->d_x.p, s->d_bb.p, s->stream);
   launch_evaluate_list(s->d_probs.p, s->d_dblob.p, s->d_iblob.p, list, n, max_n, s->pk.max_rows, s->d_x.p, s->d_viol.p, s->d_obj.p, s->stream);
-  launch_bnb_inc_pack(s->st, s->d_probs.p, list, n, max_n, s->d_obj.p, s->d_viol.p, s->d_bb.p, s->ai_z.p, round, s->ai_rec.p, s->ai_stride,
+  launch_bnb_inc_pack(s->st, s->d_probs.p, list, n, max_n, s->d_obj.p, s->d_viol.p, s->d_bb.p, s->ai_z.p, round, out, s->ai_stride,
                       s->stream);
   s->fr_launches += max_n > 0 ? 4 : 1;
 }
@@ -414,7 +430,7 @@ int run_rounds(MiqpB200Solver *s, long max_rounds_now) {
     launch_bnb_select(s->st, s->d_probs.p, (int)rounds + 1, el0, s->stream);
     s->fr_launches += 2;
     // (before the streaming harvest: its finish_plan rewrites inc_z; no incumbent exists before round 1)
-    if (s->on_inc) launch_inc_harvest(s, (int)rounds + 1, rounds == 0 ? 0 : s->hv_bound, 1);
+    if (s->on_inc) launch_inc_harvest(s, (int)rounds + 1, rounds == 0 ? 0 : s->hv_bound, 1, s->ai_rec.p);
     if (s->on_done) { launch_harvest(s, 0, rounds == 0 ? s->st.count : s->hv_bound); s->fr_launches += 4; }
     CK(cudaEventRecord(s->evr0, s->stream));
     if (s->n_single > 0) {
@@ -478,10 +494,10 @@ void start_run(MiqpB200Solver *s) {
     s->st.delivered = s->hv_delivered.p;
     s->hv_pending = 0; s->hv_total = 0; s->hv_held.clear();
   }
+  s->fi_started = false; s->fi_reported = false;
   if (s->on_inc) {
-    s->ai_stride = (INC_REC_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;   // records 16-byte aligned
-    s->ai_reported.ensure(count); s->ai_list.ensure(count); s->ai_rec.ensure((size_t)count * s->ai_stride);
-    s->ai_z.ensure((size_t)count * s->st.zstride);
+    ensure_inc_harvest(s);
+    s->ai_rec.ensure((size_t)count * s->ai_stride);
     s->h_airec.resize((size_t)count * s->ai_stride);
     if (!s->ev_ai) CK(cudaEventCreateWithFlags(&s->ev_ai, cudaEventDisableTiming));
     CK(cudaMemsetAsync(s->ai_reported.p, 0xff, sizeof(unsigned long long) * count, s->stream));
@@ -502,7 +518,7 @@ void finish_run(MiqpB200Solver *s, float *device_ms) {
   if (s->on_inc) deliver_incumbents(s);
   if (streaming) deliver_pending(s);
   // anytime run: the incumbents found in the last round, before bnb_finish rewrites inc_z
-  if (s->on_inc) launch_inc_harvest(s, (int)s->fr_rounds + 1, s->fr_rounds == 0 ? 0 : s->hv_bound, 0);
+  if (s->on_inc) launch_inc_harvest(s, (int)s->fr_rounds + 1, s->fr_rounds == 0 ? 0 : s->hv_bound, 0, s->ai_rec.p);
   launch_bnb_finish(s->st, s->d_probs.p, s->d_dblob.p, s->d_iblob.p, s->d_x.p, s->d_bb.p, s->stream);
   if (!streaming) {
     CK(cudaMemsetAsync(s->d_viol.p, 0, sizeof(double) * count, s->stream));
@@ -739,6 +755,30 @@ PoolExportHeader export_header(const MiqpB200Solver *s) {
   h.shape_hash = f;
   return h;
 }
+
+constexpr unsigned FRONTIER_INC_MAGIC = 0x434e4946u;   // "FINC"
+constexpr unsigned FRONTIER_INC_VERSION = 1;
+
+FrontierIncLayout frontier_inc_layout(const MiqpB200Solver *s) {
+  FrontierIncLayout l;
+  const long count = s->st.count;
+  l.off_bb = sizeof(FrontierIncHeader);
+  l.off_nodes = align16(l.off_bb + (long)sizeof(double) * count);
+  l.off_iters = align16(l.off_nodes + (long)sizeof(unsigned long long) * count);
+  l.off_stop = align16(l.off_iters + (long)sizeof(unsigned long long) * count);
+  l.summary_bytes = align16(l.off_stop + count);
+  l.rec_stride = s->ai_stride;
+  return l;
+}
+
+FrontierIncHeader frontier_inc_header(const MiqpB200Solver *s) {
+  const PoolExportHeader p = export_header(s);
+  FrontierIncHeader h;
+  std::memset(&h, 0, sizeof h);
+  h.magic = FRONTIER_INC_MAGIC; h.version = FRONTIER_INC_VERSION;
+  h.count = s->st.count; h.rec_stride = s->ai_stride; h.shape_hash = p.shape_hash;
+  return h;
+}
 }  // namespace
 
 extern "C" {
@@ -932,7 +972,7 @@ int miqp_b200_batch_upload(MiqpB200Solver *s, const MiqpB200Problem *problems, i
   if (!s || !problems || count <= 0) return MIQP_B200_ERR_ARG;
   try {
     CK(cudaSetDevice(s->opt.device));
-    s->uploaded = false; s->ran = false;
+    s->uploaded = false; s->ran = false; s->fi_started = false; s->st.stop = nullptr;
     clear_stops(s, 0);
     const auto tp0 = std::chrono::steady_clock::now();
     pack_batch(s, problems, count);
@@ -987,7 +1027,7 @@ int miqp_b200_batch_upload_replan(MiqpB200Solver *s, const MiqpB200Problem *prob
     std::vector<Shape> prev(count);
     for (int k = 0; k < count; ++k) { const DevProb &p = s->pk.probs[k]; prev[k] = Shape{p.C, p.N, p.R, p.O, p.E, p.L}; }
     CK(cudaStreamSynchronize(s->stream));
-    s->uploaded = false; s->ran = false;
+    s->uploaded = false; s->ran = false; s->fi_started = false; s->st.stop = nullptr;
     clear_stops(s, 0);
     const auto tp0 = std::chrono::steady_clock::now();
     pack_batch(s, problems, count);
@@ -1200,7 +1240,12 @@ int miqp_b200_frontier_start(MiqpB200Solver *s) {
   try {
     CK(cudaSetDevice(s->opt.device));
     start_run(s);
+    // the keys of the incumbent deliveries (frontier_inc_merge) start over; no stop mask of an earlier run applies
+    s->fi_key_obj.ensure(s->st.count); s->fi_key_rank.ensure(s->st.count);
+    CK(cudaMemsetAsync(s->fi_key_rank.p, 0xff, sizeof(int) * s->st.count, s->stream));
+    s->st.stop = nullptr;
     CK(cudaStreamSynchronize(s->stream));
+    s->fi_started = true;
   } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
   return MIQP_B200_OK;
 }
@@ -1272,7 +1317,128 @@ int miqp_b200_frontier_finish(MiqpB200Solver *s, float *device_ms) {
   if (!s || !s->uploaded) return MIQP_B200_ERR_ARG;
   try {
     CK(cudaSetDevice(s->opt.device));
+    s->fi_started = false;
     finish_run(s, device_ms);
+    // (done is final: miqp_b200_stopped reads it) the merged stop mask and the requests of this run go, as at the end of a batch run
+    s->st.stop = nullptr;
+    clear_stops(s, s->st.count);
+  } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
+  return MIQP_B200_OK;
+}
+
+// ---- frontier sharding with incumbent deliveries (export of every rank, all-gather by the caller, merge on every rank) -------
+// Ordering: the export runs after frontier_rounds and before that exchange's incumbent-objective exchange.  Only frontier_tighten
+// lowers ub other than a find of this rank, so a plan's inc_uid changes only with a find of its own, and a record's ub is this
+// rank's own incumbent value.  The export synchronises the stream: an in-place NCCL all-reduce on ub may follow at once.
+int miqp_b200_frontier_inc_export(MiqpB200Solver *s, void **dev, size_t *summary_bytes, size_t *record_bytes, int *n_records) {
+  if (!s || !dev || !summary_bytes || !record_bytes || !n_records) return MIQP_B200_ERR_ARG;
+  if (!s->uploaded || !s->fi_started) return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_export without frontier_start");
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    const int count = s->st.count;
+    ensure_inc_harvest(s);
+    const FrontierIncLayout l = frontier_inc_layout(s);
+    s->fi_export.ensure((size_t)(l.summary_bytes + (long)count * l.rec_stride * (long)sizeof(double)));
+    unsigned char *b = s->fi_export.p;
+    if (!s->fi_reported) {   // the first export of the run reports every incumbent that exists, the ramp-up's too
+      CK(cudaMemsetAsync(s->ai_reported.p, 0xff, sizeof(unsigned long long) * count, s->stream));
+      s->fi_reported = true;
+    }
+    FrontierIncHeader h = frontier_inc_header(s);
+    h.rounds = s->fr_rounds;
+    {
+      std::lock_guard<std::mutex> g(s->stop_mu);
+      s->h_stop.assign(s->stop_req.begin(), s->stop_req.end());
+    }
+    CK(cudaMemcpyAsync(b, &h, sizeof h, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(b + l.off_stop, s->h_stop.data(), (size_t)count, cudaMemcpyHostToDevice, s->stream));
+    launch_frontier_inc_summary(s->st, b, l, s->stream);
+    // records: the anytime harvest (round = rounds run + 1: a record names the last round before the export)
+    launch_inc_harvest(s, (int)s->fr_rounds + 1, count, 0, reinterpret_cast<double *>(b + l.summary_bytes));
+    CK(cudaMemcpyAsync(b + offsetof(FrontierIncHeader, n_records), s->b_ctrl.p + 8, sizeof(int), cudaMemcpyDeviceToDevice, s->stream));
+    CK(cudaGetLastError());
+    int n = 0;
+    CK(cudaMemcpyAsync(&n, s->b_ctrl.p + 8, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));   // (also: the header's host copy goes out of scope)
+    s->fr_launches += 1;
+    *dev = b;
+    *summary_bytes = (size_t)l.summary_bytes;
+    *record_bytes = (size_t)l.rec_stride * sizeof(double);
+    *n_records = n;
+  } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
+  return MIQP_B200_OK;
+}
+
+int miqp_b200_frontier_inc_merge(MiqpB200Solver *s, const void *gathered, int world, int n_max, MiqpB200FrontierIncumbentFound cb,
+                                 void *user, int *n_new) {
+  if (!s) return MIQP_B200_ERR_ARG;
+  if (!s->uploaded || !s->fi_started) return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_merge without frontier_start");
+  const int count = s->st.count;
+  if (!gathered || world < 1) return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_merge: no input or world < 1");
+  if (n_max < 0 || n_max > count) return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_merge: n_max must lie in 0..count");
+  try {
+    CK(cudaSetDevice(s->opt.device));
+    ensure_inc_harvest(s);
+    const FrontierIncLayout l = frontier_inc_layout(s);
+    const long block = l.summary_bytes + (long)n_max * l.rec_stride * (long)sizeof(double);
+    const size_t total = (size_t)block * world;
+    cudaPointerAttributes attr;
+    const bool here = cudaPointerGetAttributes(&attr, gathered) == cudaSuccess && attr.device == s->opt.device &&
+                      (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged);
+    cudaGetLastError();   // (an older runtime reports a host pointer it does not know as an error)
+    // headers first, every one checked before anything changes
+    const FrontierIncHeader mine = frontier_inc_header(s);
+    std::vector<FrontierIncHeader> hs(world);
+    for (int r = 0; r < world; ++r)
+      CK(cudaMemcpyAsync(&hs[r], static_cast<const unsigned char *>(gathered) + (size_t)r * block, sizeof(FrontierIncHeader),
+                         cudaMemcpyDefault, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    for (int r = 0; r < world; ++r) {
+      const FrontierIncHeader &h = hs[r];
+      if (h.magic != mine.magic || h.version != mine.version || h.count != mine.count || h.rec_stride != mine.rec_stride ||
+          h.shape_hash != mine.shape_hash)
+        return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_merge: block " + std::to_string(r) +
+                                              " does not come from a solver with this batch's shapes (or n_max is wrong)");
+      if (h.n_records < 0 || h.n_records > n_max)
+        return fail(s, MIQP_B200_ERR_ARG, "frontier_inc_merge: block " + std::to_string(r) + " holds more records than n_max");
+    }
+    const unsigned char *g = static_cast<const unsigned char *>(gathered);
+    if (!here) {   // host memory or another GPU: a copy on this solver's device
+      s->fi_gathered.ensure(total);
+      CK(cudaMemcpyAsync(s->fi_gathered.p, gathered, total, cudaMemcpyDefault, s->stream));
+      g = s->fi_gathered.p;
+    }
+    const long out_stride = (FI_OUT_HDR + (long)s->pk.maxC * s->pk.maxN * 8 + 1) & ~1L;
+    s->fi_list.ensure(count); s->fi_src.ensure(count); s->fi_n.ensure(1); s->fi_out.ensure((size_t)count * out_stride);
+    s->d_stop.ensure(count);
+    launch_frontier_inc_merge(s->st, g, l, block, world, s->fi_key_obj.p, s->fi_key_rank.p, s->d_stop.p, s->fi_list.p, s->fi_src.p, s->fi_n.p,
+                              s->fi_out.p, out_stride, s->stream);
+    launch_frontier_inc_pack(s->d_probs.p, g, l, block, s->fi_list.p, s->fi_src.p, s->fi_n.p, count, s->fi_out.p, out_stride, s->stream);
+    CK(cudaGetLastError());
+    s->fr_launches += 2;
+    // the merged stop mask applies from the next select of this rank, the same select on every rank
+    s->st.stop = s->d_stop.p;
+    int n = 0;
+    CK(cudaMemcpyAsync(&n, s->fi_n.p, sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    if (n_new) *n_new = n;
+    if (!cb || n == 0) return MIQP_B200_OK;
+    s->h_fiout.resize((size_t)n * out_stride);
+    CK(cudaMemcpyAsync(s->h_fiout.data(), s->fi_out.p, sizeof(double) * (size_t)n * out_stride, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    const double seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - s->fr_t0).count();
+    for (int e = 0; e < n; ++e) {   // ascending plan order
+      const double *rec = s->h_fiout.data() + (size_t)e * out_stride;
+      FrontierIncOut o;
+      std::memcpy(&o, rec, sizeof o);
+      MiqpB200Incumbent in;
+      std::memset(&in, 0, sizeof in);
+      in.objective = o.r.objective; in.max_violation = o.r.max_violation; in.search_value = o.r.ub;
+      in.best_bound = o.r.best_bound; in.gap = rel_gap(o.r.best_bound, o.r.objective);
+      in.seconds = seconds;
+      in.round = o.r.round; in.nodes = (long)o.r.nodes; in.qp_iters = (long)o.r.iters; in.uid = o.r.inc_uid;
+      if (cb(user, o.r.k, o.rank, rec + FI_OUT_HDR, &in)) miqp_b200_request_stop(s, o.r.k);
+    }
   } catch (const std::exception &ex) { return fail(s, MIQP_B200_ERR_CUDA, ex.what()); }
   return MIQP_B200_OK;
 }

@@ -58,7 +58,8 @@ def solve_sharded(problems: Sequence, solve_fn: Callable, group=None):
 # Frontier sharding (SURVEY.md section 8(e).2): ONE plan (or a few), its open nodes distributed over the ranks
 # ---------------------------------------------------------------------------------------------------------------------
 def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=None, warm=None, group=None,
-                           ramp_rounds: int = 6, exchange_every: int = 4, stats: dict | None = None, merge_pool: bool = False):
+                           ramp_rounds: int = 6, exchange_every: int = 4, stats: dict | None = None, merge_pool: bool = False,
+                           on_incumbent: Callable | None = None, deliver_rank: int | None = 0):
     """Every rank passes the same `problems` and its own solver (one GPU each); returns (xs, infos) of ALL plans on every
     rank.  Each plan's branch-and-bound frontier is sharded over the ranks:
 
@@ -77,6 +78,17 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
     all-gathered (NCCL: straight from the device buffers; gloo: through the host) in rank order and merged, so that
     solver.pool(k) on every rank returns the same pool, that of the union of all ranks' leaves.  stats gains pool_bytes
     (one rank's export) and pool_merge_ms.  Nothing else of the result changes.
+
+    on_incumbent(k, traj, inc) (anytime deliveries): at every exchange each rank exports the incumbents it found since its last
+    export (before the incumbent-objective exchange), the exports are all-gathered in rank order and merged on every rank, and
+    the best incumbent of all ranks is delivered whenever its (objective, rank) improves -- on rank `deliver_rank` only, or on
+    every rank with deliver_rank=None; every rank computes the same deliveries.  inc is a capi.Incumbent with the finding rank,
+    the merged bound and the counters of all ranks.  One more merge before frontier_finish makes the last delivery of a plan its
+    combined result.  A truthy return, or solver.request_stop(k) from any thread on any rank, stops plan k on every rank from
+    the exchange after it.  With one rank the search runs in steps of `exchange_every` rounds.  An exception raised by the
+    callback stops every plan; the ranks finish together and it is raised on its rank after the combine.  stats gains
+    inc_exchanges, inc_gather_bytes (all exchanges), inc_ms (host time of export, gather and merge) and delivered.  Without
+    on_incumbent the search is the one above and ignores stop requests.
     """
     import numpy as np
     import torch
@@ -94,9 +106,19 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
         return t.cpu().numpy()
 
     n = len(problems)
+    inc = None
+    if on_incumbent is not None:
+        deliver = deliver_rank is None or deliver_rank == rank
+        inc = _IncExchange(solver, on_incumbent if deliver else None, group, world, dev, on_nccl, allreduce)
     solver.upload(problems, gap_tol=gap_tol, time_limit=time_limit, warm=warm)
     solver.frontier_start()
-    left = solver.frontier_rounds(ramp_rounds if sharded else -1)
+    if inc is not None and not sharded:      # one rank with deliveries: the same search in steps
+        left = n
+        while left > 0:
+            left = solver.frontier_rounds(exchange_every)
+            inc.exchange()
+    else:
+        left = solver.frontier_rounds(ramp_rounds if sharded else -1)
     exchanges, split_done = 0, False
     if sharded:
         fp = solver.frontier_fingerprint()
@@ -111,6 +133,8 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
         total_left = int(allreduce(np.array([left], dtype=np.int64), dist.ReduceOp.SUM)[0])
         while total_left > 0:
             left = solver.frontier_rounds(exchange_every) if left > 0 else 0
+            if inc is not None:     # before the incumbent objectives are exchanged: each record's value is its rank's own
+                inc.exchange()
             if on_nccl:     # in place on the solver's incumbent objectives: no host copy
                 dist.all_reduce(ub_t, op=dist.ReduceOp.MIN, group=group)
                 torch.cuda.synchronize()
@@ -118,11 +142,17 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
                 solver.frontier_tighten(allreduce(solver.frontier_get_ub(), dist.ReduceOp.MIN))
             exchanges += 1
             total_left = int(allreduce(np.array([left], dtype=np.int64), dist.ReduceOp.SUM)[0])
+    if inc is not None:
+        inc.exchange()      # the last rounds (and a ramp-up that finished everything)
     ms = solver.frontier_finish()
     xs, infos = solver.fetch()
     if stats is not None:
         stats.update(device_ms=ms, exchanges=exchanges, split=split_done, world=world, nodes_this_rank=sum(i.nodes for i in infos))
+        if inc is not None:
+            stats.update(inc_exchanges=inc.exchanges, inc_gather_bytes=inc.gather_bytes, inc_ms=inc.ms, delivered=inc.delivered)
     if not sharded:
+        if inc is not None and inc.error:
+            raise inc.error[0]
         return xs, infos
 
     if merge_pool:
@@ -156,7 +186,58 @@ def solve_frontier_sharded(solver, problems: Sequence, gap_tol=None, time_limit=
                                 proven=bool(have and gap <= gtol + 1e-15), nodes=int(counts[k, 0]), qp_iters=int(counts[k, 1]),
                                 uncertified=int(counts[k, 2]), pool_exhausted=int(counts[k, 3] > 0),
                                 max_violation=float(viol[k]) if have else float("nan")))
+    if inc is not None and inc.error:
+        raise inc.error[0]
     return out_x, out_i
+
+
+class _IncExchange:
+    """the incumbent deliveries of solve_frontier_sharded(on_incumbent=...): export, MAX all-reduce of the record counts,
+    all-gather of the blocks in rank order (NCCL straight from the device buffer, gloo through the host), merge on every rank"""
+
+    def __init__(self, solver, on_incumbent, group, world, dev, on_nccl, allreduce):
+        self.solver, self.group, self.world, self.dev, self.on_nccl, self.allreduce = solver, group, world, dev, on_nccl, allreduce
+        self.user = on_incumbent
+        self.error = []
+        self.exchanges = self.gather_bytes = self.delivered = 0
+        self.ms = 0.0
+
+    def _deliver(self, k, traj, inc):
+        if self.error:
+            return False
+        try:
+            return self.user(k, traj, inc)
+        except BaseException as ex:     # every plan stops on every rank at the next exchange; raised after the combine
+            self.error.append(ex)
+            self.solver.request_stop(-1)
+            return False
+
+    def exchange(self):
+        import numpy as np
+        import torch
+        import torch.distributed as dist
+        t0 = time.perf_counter()
+        buf, summary, record, n_rec = self.solver.frontier_inc_export()
+        if self.world > 1:
+            n_max = int(self.allreduce(np.array([n_rec], dtype=np.int64), dist.ReduceOp.MAX)[0])
+            block = summary + n_max * record
+            if self.on_nccl:
+                gathered = torch.empty(self.world * block, dtype=torch.uint8, device=self.dev)
+                dist.all_gather_into_tensor(gathered, buf[:block], group=self.group)
+                torch.cuda.synchronize()
+            else:
+                mine = buf[:block].cpu()
+                parts = [torch.empty_like(mine) for _ in range(self.world)]
+                dist.all_gather(parts, mine, group=self.group)
+                gathered = torch.cat(parts)
+        else:
+            n_max = n_rec
+            block = summary + n_max * record
+            gathered = buf[:block]
+        self.delivered += self.solver.frontier_inc_merge(gathered, self.world, n_max, self._deliver if self.user is not None else None)
+        self.exchanges += 1
+        self.gather_bytes += self.world * block
+        self.ms += 1e3 * (time.perf_counter() - t0)
 
 
 def _merge_pools(solver, group, world, dev, on_nccl, allreduce, stats):
